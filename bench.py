@@ -3,6 +3,7 @@
 
   python bench.py --gpus 1 --steps K --warmup W          (N>1: launched by torch.distributed.run)
   python bench.py --impl reference ...                    CPU arm: the restated IPOPT path on host cores
+  python bench.py ... --dump-outputs DIR                  also write the last timed step's outputs as DIR/<name>.npy
 
 A step = one cold-start solve (X_k = start, U = 0; centralized_six_robots_implementation.py:398-400)
 of a batch of synthetic start/goal instances (SURVEY.md 8d recipe).  Instances are independent, so
@@ -25,6 +26,22 @@ PER_GPU = 8192
 ALG_BYTES_PER_SOLVE = 15728       # SURVEY.md 8d: p + w0 in, x + f + g out
 F_FACT, F_SOLVE, F_EVAL = 1100160, 92160, 14700   # SURVEY.md 8d dense-stage FP64 flop counts @ Nr=6, N=20
 F_ITER = F_FACT + F_SOLVE + F_EVAL                # 1.207 MFLOP per interior-point iteration (SURVEY.md 8d's unit of work)
+DUMP_BYTES = 64_000_000           # --dump-outputs: bytes written, all files together
+
+
+def dump_outputs(out, path):
+    """Write the arrays one solve returned to its caller (x, f, g, stats, status, iters) as float64 DIR/<name>.npy, row b
+    of every file being the same instance.  When the whole batch would exceed DUMP_BYTES, a default_rng(0) sample of
+    instances is written instead (the same one for every run at a given batch size); instance.npy holds their indices."""
+    arrs = {k: v.cpu().numpy().astype(np.float64) for k, v in out.items()}
+    B = len(arrs["x"])
+    row_bytes = 8 * (1 + sum(a[0].size for a in arrs.values()))      # 1: the instance index
+    keep = min(B, (DUMP_BYTES - 4096) // row_bytes)                    # 4096: room for the .npy headers
+    idx = np.arange(B) if keep == B else np.sort(np.random.default_rng(0).choice(B, keep, replace=False))
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "instance.npy"), idx.astype(np.float64))
+    for k, a in arrs.items():
+        np.save(os.path.join(path, k + ".npy"), a[idx])
 
 
 def measured_traffic():
@@ -139,7 +156,11 @@ def main():
     ap.add_argument("--e2e-steps", type=int, default=2)
     ap.add_argument("--swarm", type=int, default=148, help="N=1 only: also time this many 64-robot swarm instances (BASELINE.json configs[4]) on the dense-block path; 0 = skip")
     ap.add_argument("--clone", type=int, default=-1, help="diagnostic: replicate one instance B times (all warps run in lockstep)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned (rank 0's shard) as DIR/<name>.npy, "
+                                                          "at most 64 MB (a fixed sample of instances when the batch is larger)")
     a = ap.parse_args()
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs records the CUDA path; the reference arm solves a time-bounded, run-dependent sample")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -211,6 +232,8 @@ def main():
         e0.record(); step(); e1.record()
         evs.append((e0, e1))
     torch.cuda.synchronize()
+    if a.dump_outputs and rank == 0:
+        dump_outputs(out, a.dump_outputs)
     if world > 1:
         dist.barrier()
     ms = [e0.elapsed_time(e1) for e0, e1 in evs]
@@ -299,7 +322,7 @@ def main():
             with torch.cuda.stream(streams[i]):
                 pp[i].solve(d_x0, d_p, d_lbx, d_ubx, d_lbg, d_ubg, want=("stats",), out=pouts[i])
         torch.cuda.synchronize()
-        k2 = max(4, a.steps)
+        k2 = a.steps
         flush.fill_(1)
         p0 = torch.cuda.Event(enable_timing=True)
         p0.record()
