@@ -97,7 +97,7 @@ void nmpc_destroy(nmpc_handle *h);
  *   ctas_per_sm       > 0: cap on resident CTAs per SM (occupancy experiments); 0 = as many as fit
  *   force_block_path  != 0: run any Nr on the CTA-per-instance dense-block solver (test hook)
  *   thread_min_batch  > 0: batches at least this large of the one-robot static-obstacle family use the thread-per-instance
- *                     solver; 0 = never */
+ *                     solver; 0 = never.  Ignored by nmpc_create_moving_obstacles (that solver takes one static table) */
 typedef struct nmpc_tuning { int convoy, ctas_per_sm, force_block_path, thread_min_batch; } nmpc_tuning;
 void nmpc_default_tuning(nmpc_tuning *t);
 /* nmpc_create / nmpc_create_obstacles (n_obs > 0) with explicit tuning; t == NULL means the defaults. */
@@ -105,7 +105,7 @@ int nmpc_create_tuned(const nmpc_desc *d, const nmpc_opts *o, const nmpc_tuning 
 
 int nmpc_n(const nmpc_handle *h);        /* decision variables                         */
 int nmpc_mg(const nmpc_handle *h);       /* constraint rows                            */
-int nmpc_np(const nmpc_handle *h);       /* parameters (6 Nr)                          */
+int nmpc_np(const nmpc_handle *h);       /* parameters (6 Nr; + 3 N n_obs with obstacles in p) */
 int nmpc_nnz_jac(const nmpc_handle *h);  /* 3Nr + N(11Nr+4M)   CasADi's CCS of dg/dw   */
 int nmpc_nnz_hess(const nmpc_handle *h); /* N(6Nr+2M)          lower triangle          */
 
@@ -135,6 +135,18 @@ int nmpc_solve(nmpc_handle *h, int B, const double *x0, const double *p,
  * (one robot with up to 32 obstacles; the reference's scripts have one robot and 1, 4 or 6), else on the CTA-per-instance
  * dense-block path; nmpc_eval and the CCS patterns are not available for this family. */
 int nmpc_create_obstacles(const nmpc_desc *d, const nmpc_opts *o, int n_obs, const double *obs, nmpc_handle **out);
+
+/* Static-obstacle family with the obstacle geometry in p (per instance, per stage): scenario sweeps over obstacle layouts in one
+ * batch, and obstacles that move along known or predicted trajectories over the horizon.
+ *     p = [x0bar (3 Nr); xs (3 Nr); O],  O = [N][n_obs][3] = (ox, oy, clearance) of obstacle o at stage k = 0..N-1,
+ *     nmpc_np = 6 Nr + 3 N n_obs.
+ * Row (k, i, o), on X_k, is sqrt((x_{k,i} - ox_{k,o})^2 + (y_{k,i} - oy_{k,o})^2) - c_{k,o}.  Variables, g row layout, mg, bounds,
+ * status and stats are those of nmpc_create_obstacles, and so is the path (warp-per-instance for 1..4 robots while
+ * M + Nr n_obs <= 32, else the dense-block path; t->force_block_path is honoured, t->thread_min_batch is ignored).  A block O that
+ * repeats one table at every stage gives bit for bit what nmpc_create_obstacles with that table gives.  The clearances are device
+ * data and are NOT validated (a negative one is the caller's responsibility).  1 <= n_obs <= 32, else NMPC_EINVAL; t == NULL
+ * means the default tuning.  nmpc_eval and the CCS patterns return NMPC_ENOTSUP; nmpc_shift and nmpc_plant work. */
+int nmpc_create_moving_obstacles(const nmpc_desc *d, const nmpc_opts *o, const nmpc_tuning *t, int n_obs, nmpc_handle **out);
 
 /* Small generic optimal-control problems, one GPU thread per instance.  model NMPC_OCP_VAN_DER_POL is the direct-multiple-shooting
  * demo of mpc_pose_control_casadi.py:22-114: 2 states, 1 control, N intervals over the horizon T, each integrated by rk_steps RK4

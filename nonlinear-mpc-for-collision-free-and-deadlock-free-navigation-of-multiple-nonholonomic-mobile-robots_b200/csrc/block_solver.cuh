@@ -42,7 +42,7 @@ __device__ long long g_block_prof[16];
                  *const DU = wp::global_ptr(this->DU), *const pp = wp::global_ptr(this->pp);                            \
     const int *const pairs = wp::global_ptr(this->pairs);                                                              \
     const double *const obs = wp::global_ptr(this->obs);                                                               \
-    const int Mp = this->Mp, nobs = this->nobs;                                                                        \
+    const int Mp = this->Mp, nobs = this->nobs, ostr = this->ostr;                                                     \
     double *const Pall = wp::global_ptr(this->Pall), *const Yall = wp::global_ptr(this->Yall),                          \
                  *const Lall = wp::global_ptr(this->Lall),                                                             \
                  *const Wg = wp::global_ptr(this->Wg);                                                                 \
@@ -51,7 +51,7 @@ __device__ long long g_block_prof[16];
     auto row = [=](int r, int k) -> double * { return ws + ((long long)r * S + k) * W; };                              \
     (void)sm; (void)ws; (void)BL; (void)BU; (void)CE; (void)DL; (void)DU; (void)pp; (void)pairs; (void)Pall;            \
     (void)Yall; (void)Lall; (void)Wg; (void)S; (void)W; (void)N; (void)Nr; (void)ns; (void)nc; (void)nz; (void)M;       \
-    (void)tid; (void)nt; (void)row; (void)obs; (void)Mp; (void)nobs;
+    (void)tid; (void)nt; (void)row; (void)obs; (void)Mp; (void)nobs; (void)ostr;
 
 struct BlockSolver {
     enum Row {
@@ -67,8 +67,9 @@ struct BlockSolver {
     const NmpcSolveParams &P;
     double *sm, *ws;
     int Nr, N, S, ns, nc, nz, M, W, tid, nt, inst, fn;   // M: inequality rows per block = pair rows + obstacle rows
-    int Mp, nobs, family;                                 // pair rows, static obstacles per robot, row layout (0 centralized, 1 obstacles)
-    const double *obs;                                    // [nobs][3]: centre x, y, clearance radius
+    int Mp, nobs, family;                                 // pair rows, obstacles per robot, row layout (0 centralized, 1 obstacles)
+    const double *obs;                                    // [nobs][3] of stage 0: centre x, y, clearance radius
+    int ostr;                                             // doubles from one stage's obstacle table to the next (0: static obstacles)
     const double *BL, *BU, *CE, *DL, *DU, *pp;
     const int *pairs;
     double *Pall, *Yall, *Lall, *Wg;   // Wg: Linv_II L_IJ blocks of the stage being factored (see factor, step D)
@@ -156,13 +157,15 @@ struct BlockSolver {
     __device__ void setup(int instance)
     {
         inst = instance; Nr = P.Nr; N = P.N; S = N + 1; ns = 3 * Nr; nc = 2 * Nr; nz = 5 * Nr;
-        Mp = Nr * (Nr - 1) / 2; nobs = P.nobs; family = P.family; obs = P.obs; M = Mp + Nr * nobs;
+        Mp = Nr * (Nr - 1) / 2; nobs = P.nobs; family = P.family; M = Mp + Nr * nobs;
         W = row_width(Nr, nobs); T = P.T; tid = threadIdx.x; nt = blockDim.x;
         const double *br = P.brows + (long long)inst * P.bstride;
         BL = br + (long long)NMPC_BR_BL * S * W; BU = br + (long long)NMPC_BR_BU * S * W;
         CE = br + (long long)NMPC_BR_CE * S * W; DL = br + (long long)NMPC_BR_DL * S * W;
         DU = br + (long long)NMPC_BR_DU * S * W;
-        pp = P.p + (long long)inst * 2 * ns;
+        pp = P.p + (long long)inst * P.np;
+        // obstacles in p: [N][nobs][3] after x0bar and xs, one table per stage; else the handle's table at every stage
+        obs = P.obs_in_p ? pp + 2 * ns : P.obs; ostr = P.obs_in_p ? 3 * nobs : 0;
         pairs = P.pairs;
         Pall = ws + (long long)R_COUNT * S * W;
         ldy = ((ns + 4) & ~7) + 4; ncp = (nc + 31) & ~31;
@@ -235,7 +238,7 @@ struct BlockSolver {
             const double lo = DL[b * W + q], hi = DU[b * W + q];
             const bool hl = lo > -NMPC_INF, hu = hi < NMPC_INF;
             double dv = NMPC_DUMMY_ROW_VALUE;
-            if (b > 0) dv = rowgeom(row(R_Z, b - 1), q, Mp, nobs, pairs, obs).dv;
+            if (b > 0) dv = rowgeom(row(R_Z, b - 1), q, Mp, nobs, pairs, obs + (b - 1) * ostr).dv;
             row(R_S, b)[q] = (hl || hu) ? WS::push_in(dv, lo, hi, o.bound_push, o.bound_frac) : dv;
             row(R_VL, b)[q] = hl ? o.bound_mult_init_val : 0.0;
             row(R_VU, b)[q] = hu ? o.bound_mult_init_val : 0.0;
@@ -258,7 +261,8 @@ struct BlockSolver {
 
     // Inequality row q of a block evaluated on the stage vector zr.  Rows q < Mp are the pairwise squared distances
     // (centralized_six_robots_implementation.py:288-306); rows q >= Mp are the static circular obstacles of family F,
-    // sqrt((x - ox)^2 + (y - oy)^2) - r_rob - r_obs (first_scenario_mpc_obstacle_avoidance.py:125), nobs per robot.
+    // sqrt((x - ox)^2 + (y - oy)^2) - r_rob - r_obs (first_scenario_mpc_obstacle_avoidance.py:125), nobs per robot;
+    // obs: the obstacle table [nobs][3] of the stage zr belongs to.
     // i, j: robots (j = -1 for an obstacle row); (gx, gy): gradient w.r.t. (x_i, y_i) (negated for robot j);
     // (hxx, hyy, hxy): second derivatives w.r.t. (x_i, y_i).
     struct RowG { double dv, gx, gy, hxx, hyy, hxy; int i, j; };
@@ -320,7 +324,7 @@ struct BlockSolver {
             const double yd_ = full ? row(R_YD, b)[q] : 0.0, vl_ = full ? row(R_VL, b)[q] : 0.0, vu_ = full ? row(R_VU, b)[q] : 0.0;
             const double dsoc_ = socacc ? row(R_DSOC, b)[q] : 0.0;
             double dv = NMPC_DUMMY_ROW_VALUE;
-            if (b > 0) dv = rowgeom(row(rz, b - 1), q, Mp, nobs, pairs, obs).dv;
+            if (b > 0) dv = rowgeom(row(rz, b - 1), q, Mp, nobs, pairs, obs + (b - 1) * ostr).dv;
             const bool hl = lo > -NMPC_INF, hu = hi < NMPC_INF;
             if (!(hl || hu)) continue;
             const double dms = dv - s;
@@ -379,7 +383,7 @@ struct BlockSolver {
                             }
                             for (int o = 0; o < nobs; o++) {   // static obstacles of this robot
                                 const int q = Mp + rob * nobs + o;
-                                const RowG rg = rowgeom(zr, q, Mp, nobs, pairs, obs);
+                                const RowG rg = rowgeom(zr, q, Mp, nobs, pairs, obs + k * ostr);
                                 r += (comp == 0 ? rg.gx : rg.gy) * ydn[q];
                             }
                         }
@@ -471,7 +475,7 @@ struct BlockSolver {
             const double dsoc_ = (soc && mode != 1) ? row(R_DSOC, b)[q] : 0.0, yd_ = mode == 0 ? row(R_YD, b)[q] : 0.0;
             RowG rg;
             rg.gx = rg.gy = rg.hxx = rg.hyy = rg.hxy = 0.0; rg.dv = NMPC_DUMMY_ROW_VALUE;
-            if (b > 0) rg = rowgeom(row(R_Z, b - 1), q, Mp, nobs, pairs, obs);
+            if (b > 0) rg = rowgeom(row(R_Z, b - 1), q, Mp, nobs, pairs, obs + (b - 1) * ostr);
             if (lo > -NMPC_INF || hi < NMPC_INF) {
                 const double dv = rg.dv, hxx = rg.hxx, hyy = rg.hyy, hxy = rg.hxy;
                 gxq = rg.gx; gyq = rg.gy;
@@ -1148,7 +1152,7 @@ struct BlockSolver {
                     const int b = pass == 0 ? 0 : k + 1;
                     const double lo = DL[b * W + q], hi = DU[b * W + q];
                     double dv = NMPC_DUMMY_ROW_VALUE;
-                    if (pass == 1) dv = rowgeom(zt, q, Mp, nobs, pairs, obs).dv;
+                    if (pass == 1) dv = rowgeom(zt, q, Mp, nobs, pairs, obs + k * ostr).dv;
                     const bool act = lo > -NMPC_INF || hi < NMPC_INF;
                     row(R_DS, b)[q] = act ? WS::push_in(dv, lo, hi, o.bound_push, o.bound_frac) - row(R_S, b)[q] : 0.0;
                 }
@@ -1262,7 +1266,7 @@ struct BlockSolver {
             const int b = idx / M, q = idx - b * M;
             if (family && b == 0) continue;   // family 1: block 0 holds the initial condition only
             double dv = NMPC_DUMMY_ROW_VALUE;
-            if (b > 0) dv = rowgeom(row(R_Z, b - 1), q, Mp, nobs, pairs, obs).dv;
+            if (b > 0) dv = rowgeom(row(R_Z, b - 1), q, Mp, nobs, pairs, obs + (b - 1) * ostr).dv;
             if (g) g[goff(b) + ns + q] = dv;
             if (lg) lg[goff(b) + ns + q] = row(R_YD, b)[q] / df;
         }

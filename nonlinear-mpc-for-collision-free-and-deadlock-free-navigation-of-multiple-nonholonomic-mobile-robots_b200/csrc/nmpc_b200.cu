@@ -111,6 +111,7 @@ struct nmpc_handle {
     nmpc_tuning tune;
     int nobs, family, rk_steps;               // static obstacles per robot; family: 0 centralized, 1 obstacles, 2 small OCP (thread per instance)
     double *d_obs;                            // [nobs][3] on the device
+    bool obs_in_p;                            // obstacle family with the geometry in p (per instance and stage): no d_obs
     bool thread_ok;                           // a thread-per-instance kernel exists for this problem (small-OCP family; one robot with
                                               // static obstacles): used for the small-OCP family always, else from thread_min_batch on
     size_t t_ws_doubles;                      // its scratch per instance
@@ -193,7 +194,7 @@ template <int NR, bool OBS = false> static cudaError_t config_solve(nmpc_handle 
     return e;
 }
 
-static int create_impl(const nmpc_desc *d, const nmpc_opts *o, const nmpc_tuning *t, int nobs, const double *obs, nmpc_handle **out);
+static int create_impl(const nmpc_desc *d, const nmpc_opts *o, const nmpc_tuning *t, int nobs, const double *obs, bool obs_in_p, nmpc_handle **out);
 
 extern "C" void nmpc_default_tuning(nmpc_tuning *t)
 {
@@ -201,7 +202,7 @@ extern "C" void nmpc_default_tuning(nmpc_tuning *t)
     t->ctas_per_sm = 0; t->force_block_path = 0; t->thread_min_batch = 0;
 }
 
-extern "C" int nmpc_create(const nmpc_desc *d, const nmpc_opts *o, nmpc_handle **out) { return create_impl(d, o, nullptr, 0, nullptr, out); }
+extern "C" int nmpc_create(const nmpc_desc *d, const nmpc_opts *o, nmpc_handle **out) { return create_impl(d, o, nullptr, 0, nullptr, false, out); }
 
 static int check_obstacles(int n_obs, const double *obs)
 {
@@ -215,14 +216,21 @@ static int check_obstacles(int n_obs, const double *obs)
 extern "C" int nmpc_create_tuned(const nmpc_desc *d, const nmpc_opts *o, const nmpc_tuning *t, int n_obs, const double *obs, nmpc_handle **out)
 {
     if (n_obs != 0) { int rc = check_obstacles(n_obs, obs); if (rc) return rc; }
-    return create_impl(d, o, t, n_obs, n_obs ? obs : nullptr, out);
+    return create_impl(d, o, t, n_obs, n_obs ? obs : nullptr, false, out);
 }
 
 extern "C" int nmpc_create_obstacles(const nmpc_desc *d, const nmpc_opts *o, int n_obs, const double *obs, nmpc_handle **out)
 {
     int rc = check_obstacles(n_obs, obs);
     if (rc) return rc;
-    return create_impl(d, o, nullptr, n_obs, obs, out);
+    return create_impl(d, o, nullptr, n_obs, obs, false, out);
+}
+
+extern "C" int nmpc_create_moving_obstacles(const nmpc_desc *d, const nmpc_opts *o, const nmpc_tuning *t, int n_obs, nmpc_handle **out)
+{
+    if (n_obs < 1 || n_obs > NMPC_MAX_OBSTACLES)
+        return fail(NMPC_EINVAL, "nmpc_create_moving_obstacles: need 1..%d obstacles, got %d", NMPC_MAX_OBSTACLES, n_obs);
+    return create_impl(d, o, t, n_obs, nullptr, true, out);
 }
 
 // Small generic OCP family (thread per instance): currently the Van der Pol demo of mpc_pose_control_casadi.py
@@ -252,7 +260,7 @@ extern "C" int nmpc_create_ocp(int model, int N, double T, int rk_steps, const n
     return 0;
 }
 
-static int create_impl(const nmpc_desc *d, const nmpc_opts *o, const nmpc_tuning *t, int nobs, const double *obs, nmpc_handle **out)
+static int create_impl(const nmpc_desc *d, const nmpc_opts *o, const nmpc_tuning *t, int nobs, const double *obs, bool obs_in_p, nmpc_handle **out)
 {
     if (!d || !out) return fail(NMPC_EINVAL, "nmpc_create: NULL argument");
     if (d->N < 1 || !(d->T > 0)) return fail(NMPC_EINVAL, "nmpc_create: need N >= 1 and T > 0");
@@ -266,8 +274,9 @@ static int create_impl(const nmpc_desc *d, const nmpc_opts *o, const nmpc_tuning
     if (o) h->o = *o; else nmpc_default_opts(&h->o);
     if (t) h->tune = *t; else nmpc_default_tuning(&h->tune);
     h->ns = 3 * d->Nr; h->nc = 2 * d->Nr; h->M = d->Nr * (d->Nr - 1) / 2; h->S = d->N + 1;
-    h->nobs = nobs; h->family = nobs > 0 ? 1 : 0; h->d_obs = nullptr;
-    h->n = h->ns * h->S + h->nc * d->N; h->np = 2 * h->ns;
+    h->nobs = nobs; h->family = nobs > 0 ? 1 : 0; h->d_obs = nullptr; h->obs_in_p = obs_in_p;
+    // p = [x0bar; xs], then with the obstacles in p one [nobs][3] table per stage k = 0..N-1
+    h->n = h->ns * h->S + h->nc * d->N; h->np = 2 * h->ns + (obs_in_p ? 3 * d->N * nobs : 0);
     // row layout: family 0 = (N+1) blocks of [ns equality rows ; M pair rows]; family 1 (static obstacles) = ns rows, then N
     // blocks of [ns ; M + Nr n_obs]   (first_scenario_mpc_obstacle_avoidance.py:109-125)
     h->mg = h->family ? h->ns + d->N * (h->ns + h->M + d->Nr * nobs) : h->S * (h->ns + h->M);
@@ -284,7 +293,8 @@ static int create_impl(const nmpc_desc *d, const nmpc_opts *o, const nmpc_tuning
     // solver (UnicycleObstacles model), parity-tested, but measured slower than the CTA-per-instance path both alone (88 ms
     // against 49 ms per solve at N = 100) and in batches (9.2 k against 23.0 k solves/s, B = 8192, N = 20: its per-thread
     // scratch is not coalesced across instances), so it is off unless nmpc_tuning.thread_min_batch sets a switch-over batch size.
-    h->thread_ok = h->family == 1 && d->Nr == 1;
+    // (the thread-per-instance solver takes one static table: never for obstacles in p)
+    h->thread_ok = h->family == 1 && d->Nr == 1 && !obs_in_p;
     h->t_ws_doubles = h->thread_ok ? (size_t)ThreadSolver<UnicycleObstacles>::ws_doubles(d->N) : 0;
     h->thread_min_batch = h->tune.thread_min_batch > 0 ? h->tune.thread_min_batch : 0x7fffffff;
     h->convoy = h->tune.convoy;   // 0 off, 1 barrier per iteration, 2 also before the forward pass
@@ -346,7 +356,7 @@ static int create_impl(const nmpc_desc *d, const nmpc_opts *o, const nmpc_tuning
             break;
         }
     }
-    if (e == cudaSuccess && h->nobs > 0) {
+    if (e == cudaSuccess && h->nobs > 0 && !obs_in_p) {
         e = cudaMalloc(&h->d_obs, (size_t)3 * h->nobs * sizeof(double));
         if (e == cudaSuccess) e = cudaMemcpy(h->d_obs, obs, (size_t)3 * h->nobs * sizeof(double), cudaMemcpyHostToDevice);
     }
@@ -459,7 +469,7 @@ static int solve_impl(nmpc_handle *h, int B, const double *x0, const double *p, 
     // convoy: one-warp teams only (measured -5..-8 % for the two-warp teams of 7..10 robots, whose groups are two instances),
     // and pointless while every CTA has at most one working team
     P.convoy = (!h->block_path && !thr && h->lw == 32 && h->teams_per_cta > 1 && B > solve_grid(h, B)) ? h->convoy : 0;
-    P.lbx = lbx; P.ubx = ubx; P.lbg = lbg; P.ubg = ubg; P.bounds_batched = bounds_batched; P.rk_steps = h->rk_steps; P.np = h->np;
+    P.lbx = lbx; P.ubx = ubx; P.lbg = lbg; P.ubg = ubg; P.bounds_batched = bounds_batched; P.rk_steps = h->rk_steps; P.np = h->np; P.obs_in_p = h->obs_in_p;
     const int grid = thr ? (B + 63) / 64 : solve_grid(h, B);
     if (thr && h->family == 2) solve_kernel_small_ocp<VanDerPol><<<grid, 64, 0, st>>>(P);
     else if (thr) solve_kernel_small_ocp<UnicycleObstacles><<<grid, 64, 0, st>>>(P);

@@ -40,6 +40,7 @@ typedef struct NmpcSolveParams {
     const double *obs;               /* [nobs][3] centre x, y, clearance radius (device) */
     const double *lbx, *ubx, *lbg, *ubg;  /* flat bounds (small-OCP family reads them directly) */
     int bounds_batched, rk_steps, np;
+    int obs_in_p;                    /* obstacle family: geometry from p ([N][nobs][3] after x0bar, xs), not from obs */
 } NmpcSolveParams;
 
 #endif

@@ -38,8 +38,9 @@
     const double T = this->T, df = this->df, xs_l = this->xs_l, qw = this->qw, x0bar_l = this->x0bar_l; \
     const int nobs = OBS ? this->nobs : 0, family = OBS ? this->family : 0;                              \
     const bool isobs = OBS && this->isobs;                                                              \
-    const double qox = this->qox, qoy = this->qoy, qoc = this->qoc;                                     \
-    (void)nobs; (void)family; (void)isobs; (void)qox; (void)qoy; (void)qoc;                              \
+    const double *const qob = OBS ? wp::global_ptr(this->qob) : nullptr;                                \
+    const long long qos = OBS ? this->qos : 0;                                                          \
+    (void)nobs; (void)family; (void)isobs; (void)qob; (void)qos;                                         \
     (void)sm; (void)ws; (void)br; (void)N; (void)S; (void)l;                                            \
     (void)rob; (void)comp; (void)pi; (void)pj; (void)isx; (void)isu; (void)isz; (void)isq; (void)T;    \
     (void)df; (void)xs_l; (void)qw; (void)x0bar_l;                                                     \
@@ -158,11 +159,14 @@ struct WarpSolver {
     bool trig_valid;
     double t2_alpha;
     bool isx, isu, isz, isq;
-    // inequality rows of a block: lanes < M are the pair rows (pi, pj); lanes M .. M + Nr nobs - 1 the static-obstacle rows, robot-major
-    // (row M + i nobs + o: robot pi = i against obstacle o = (qox, qoy, clearance qoc)); family 1 = the obstacle scripts' g layout
+    // inequality rows of a block: lanes < M are the pair rows (pi, pj); lanes M .. M + Nr nobs - 1 the obstacle rows, robot-major
+    // (row M + i nobs + o: robot pi = i against obstacle o); family 1 = the obstacle scripts' g layout.  The obstacle table of stage k
+    // ([nobs][3] = centre x, y, clearance) is qtab + k qos: the handle's static table (qos = 0) or the instance's block of p;
+    // qob = qtab + 3 o: this lane's obstacle at stage 0
     int nobs, family;
     bool isobs;
-    double qox, qoy, qoc;
+    const double *qtab, *qob;
+    long long qos;
     double T, df, xs_l, qw, x0bar_l, ny_nzb, nzb_cnt;
     int n_reg, n_resto, n_soc, n_fact, n_ls;
 
@@ -195,15 +199,16 @@ struct WarpSolver {
     static NMPC_DEV bool fin(double v) { return v > -NMPC_INF && v < NMPC_INF; }
     // One inequality row evaluated on a stage vector zr: value, gradient w.r.t. (x_pi, y_pi) (negated for robot pj of a pair row)
     // and its own second derivatives.  Pair rows: squared distance (centralized_six_robots_implementation.py:288-306); obstacle
-    // rows: sqrt((x - ox)^2 + (y - oy)^2) - clearance (first_scenario_mpc_obstacle_avoidance.py:96-99,125).
+    // rows: sqrt((x - ox)^2 + (y - oy)^2) - clearance (first_scenario_mpc_obstacle_avoidance.py:96-99,125), ob = (ox, oy, clearance)
+    // of the row's obstacle at the stage of zr.
     struct RowG { double dv, gx, gy, hxx, hyy, hxy; };
-    static NMPC_DEV RowG rowg(const double *zr, int pi, int pj, bool isobs, double ox, double oy, double oc)
+    static NMPC_DEV RowG rowg(const double *zr, int pi, int pj, bool isobs, const double *ob)
     {
         RowG r;
         if (isobs) {
-            const double dx = zr[3 * pi] - ox, dy = zr[3 * pi + 1] - oy;
+            const double dx = zr[3 * pi] - ob[0], dy = zr[3 * pi + 1] - ob[1];
             const double rho = sqrt(dx * dx + dy * dy), ir = 1.0 / rho;
-            r.gx = dx * ir; r.gy = dy * ir; r.dv = rho - oc;
+            r.gx = dx * ir; r.gy = dy * ir; r.dv = rho - ob[2];
             r.hxx = (1.0 - r.gx * r.gx) * ir; r.hyy = (1.0 - r.gy * r.gy) * ir; r.hxy = -r.gx * r.gy * ir;
         } else {
             const double dx = zr[3 * pi] - zr[3 * pj], dy = zr[3 * pi + 1] - zr[3 * pj + 1];
@@ -218,21 +223,23 @@ struct WarpSolver {
         inst = instance; N = P.N; S = N + 1; T = P.T; l = wp::team_lane(LW);
         nobs = OBS ? P.nobs : 0; family = OBS ? P.family : 0;
         isx = l < NS; isu = l >= NS && l < NZ; isz = l < NZ; isq = l < M + NR * nobs; isobs = isq && l >= M;
-        qox = qoy = qoc = 0.0;
+        qos = 0; qtab = qob = nullptr;
         rob = isx ? l / 3 : (isu ? (l - NS) / 2 : 0);
         comp = isx ? l % 3 : (isu ? (l - NS) % 2 : 0);
         pi = 0; pj = 0;
         if (isobs) {
-            const int e = l - M, o = e % nobs;
-            pi = e / nobs; pj = pi;   // pj = pi: the "other robot" terms of a pair row cancel for an obstacle row
-            qox = P.obs[3 * o]; qoy = P.obs[3 * o + 1]; qoc = P.obs[3 * o + 2];
+            pi = (l - M) / nobs; pj = pi;   // pj = pi: the "other robot" terms of a pair row cancel for an obstacle row
         } else if (isq) {
             int q = 0;
             for (int a = 0; a < NR; a++)
                 for (int b = a + 1; b < NR; b++) { if (q == l) { pi = a; pj = b; } q++; }
         }
         br = P.brows + (long long)inst * P.bstride;
-        const double *pp = P.p + (long long)inst * 2 * NS;
+        const double *pp = P.p + (long long)inst * (OBS ? P.np : 2 * NS);
+        if (OBS) {   // obstacles in p: [N][nobs][3] after x0bar and xs, one table per stage; else the handle's table at every stage
+            qtab = P.obs_in_p ? pp + 2 * NS : P.obs; qos = P.obs_in_p ? 3 * nobs : 0;
+            if (isobs) qob = qtab + 3 * ((l - M) % nobs);
+        }
         x0bar_l = isx ? pp[l] : 0.0;
         xs_l = isx ? pp[NS + l] : 0.0;
         qw = isx ? 2.0 * P.Q[comp] : (isu ? 2.0 * P.R[comp] : 0.0);
@@ -290,7 +297,7 @@ struct WarpSolver {
                 double lo = brow(NMPC_BR_DL, b)[l], hi = brow(NMPC_BR_DU, b)[l];
                 bool hl = lo > -NMPC_INF, hu = hi < NMPC_INF;
                 double dv = NMPC_DUMMY_ROW_VALUE;
-                if (b > 0) dv = rowg(row(R_Z, b - 1), pi, pj, isobs, qox, qoy, qoc).dv;
+                if (b > 0) dv = rowg(row(R_Z, b - 1), pi, pj, isobs, qob + (b - 1) * qos).dv;
                 s = (hl || hu) ? push_in(dv, lo, hi, o.bound_push, o.bound_frac) : dv;
                 vl = hl ? o.bound_mult_init_val : 0.0; vu = hu ? o.bound_mult_init_val : 0.0;
                 cnt_z += (hl ? 1.0 : 0.0) + (hu ? 1.0 : 0.0);
@@ -425,7 +432,7 @@ struct WarpSolver {
                 if (FULL) ysum += fabs(zc.yc);
             }
             // ---- inequality block k+1 (distances on X_k) ----
-            if (isq && k < N) ineq_row(k + 1, qn, rowg(zb, pi, pj, isobs, qox, qoy, qoc).dv);
+            if (isq && k < N) ineq_row(k + 1, qn, rowg(zb, pi, pj, isobs, qob + k * qos).dv);
             // ---- variable bounds, objective, stationarity of stage k ----
             if (zv) {
                 const double lo = zc.lo, hi = zc.hi;
@@ -459,8 +466,8 @@ struct WarpSolver {
                                     }
                                 }
                                 NMPC_NOUNROLL
-                                for (int o = 0; o < nobs; o++) {   // this robot's static obstacles: gradient (dx, dy) / rho
-                                    const double *ob = wp::global_ptr(P.obs) + 3 * o;
+                                for (int o = 0; o < nobs; o++) {   // this robot's obstacles: gradient (dx, dy) / rho
+                                    const double *ob = wp::global_ptr(this->qtab) + k * qos + 3 * o;
                                     const double dx = zb[3 * rob] - ob[0], dy = zb[3 * rob + 1] - ob[1];
                                     r += (comp == 0 ? dx : dy) / sqrt(dx * dx + dy * dy) * ydn[M + rob * nobs + o];
                                 }
@@ -509,7 +516,7 @@ struct WarpSolver {
     // block's inputs (from the staging buffer inside the sweep, from global memory for block 0).
     struct QIn { double lo, hi, s, vl, vu, yd, dsoc; };
     template <int MODE, class RowFn>
-    static NMPC_DEV void ineq_block(RowFn row, const QIn &in, int l, int pi, int pj, bool isobs, double ox, double oy, double oc, double kd,
+    static NMPC_DEV void ineq_block(RowFn row, const QIn &in, int l, int pi, int pj, bool isobs, const double *ob, double kd,
                                     int b, double mu, double delta, bool soc, const double *zb, double &pxx, double &pyy, double &pxy,
                                     double &phx, double &phy)
     {
@@ -519,7 +526,7 @@ struct WarpSolver {
         if (lo > -NMPC_INF || hi < NMPC_INF) {
             double dv = NMPC_DUMMY_ROW_VALUE, hxx = 0, hyy = 0, hxy = 0;
             if (b > 0) {
-                const RowG g = rowg(zb, pi, pj, isobs, ox, oy, oc);
+                const RowG g = rowg(zb, pi, pj, isobs, ob);
                 gxq = g.gx; gyq = g.gy; dv = g.dv; hxx = g.hxx; hyy = g.hyy; hxy = g.hxy;
             }
             double s = in.s, sigs;
@@ -678,7 +685,7 @@ struct WarpSolver {
                 QIn in;
                 in.lo = stg[FS_DL * LW + l]; in.hi = stg[FS_DU * LW + l]; in.s = stg[FS_S * LW + l]; in.vl = stg[FS_VL * LW + l];
                 in.vu = stg[FS_VU * LW + l]; in.yd = stg[FS_YD * LW + l]; in.dsoc = stg[FS_DSOC * LW + l];
-                ineq_block<MODE>(row, in, l, pi, pj, isobs, qox, qoy, qoc, kd, k + 1, mu, delta, soc, zb, a0, a1, a2, a3, a4);
+                ineq_block<MODE>(row, in, l, pi, pj, isobs, qob + k * qos, kd, k + 1, mu, delta, soc, zb, a0, a1, a2, a3, a4);
                 // pair row: entries (pi, pj) and (pj, pi); obstacle row: column NR + o of robot pi (it only feeds the row sum)
                 const int e1 = isobs ? pi * TCOLS + NR + (l - M) % nobs : pi * TCOLS + pj, e2 = isobs ? e1 : pj * TCOLS + pi;
                 tt[e2] = -a0; tt[TSZ + e2] = -a2; tt[2 * TSZ + e2] = -a1; tt[3 * TSZ + e2] = -a3; tt[4 * TSZ + e2] = -a4;
@@ -843,7 +850,7 @@ struct WarpSolver {
             QIn in;
             in.lo = brow(NMPC_BR_DL, 0)[l]; in.hi = brow(NMPC_BR_DU, 0)[l]; in.s = row(R_S, 0)[l]; in.vl = row(R_VL, 0)[l]; in.vu = row(R_VU, 0)[l];
             in.yd = MODE == 0 ? row(R_YD, 0)[l] : 0.0; in.dsoc = soc ? row(R_DSOC, 0)[l] : 0.0;
-            ineq_block<MODE>(row, in, l, pi, pj, isobs, qox, qoy, qoc, kd, 0, mu, delta, soc, zb, a0, a1, a2, a3, a4);
+            ineq_block<MODE>(row, in, l, pi, pj, isobs, qob, kd, 0, mu, delta, soc, zb, a0, a1, a2, a3, a4);
         }
         tsync();
         return true;
@@ -1069,7 +1076,7 @@ struct WarpSolver {
                     if (pass == 1 && k == N) break;
                     const int b = pass == 0 ? 0 : k + 1;
                     double lo = brow(NMPC_BR_DL, b)[l], hi = brow(NMPC_BR_DU, b)[l], dv = NMPC_DUMMY_ROW_VALUE;
-                    if (pass == 1) dv = rowg(zb, pi, pj, isobs, qox, qoy, qoc).dv;
+                    if (pass == 1) dv = rowg(zb, pi, pj, isobs, qob + k * qos).dv;
                     bool act = lo > -NMPC_INF || hi < NMPC_INF;
                     row(R_DS, b)[l] = act ? push_in(dv, lo, hi, o.bound_push, o.bound_frac) - row(R_S, b)[l] : 0.0;
                 }
@@ -1178,7 +1185,7 @@ struct WarpSolver {
                     if (lg) lg[NS + l] = row(R_YD, 0)[l] / df;
                 }
                 if (k < N) {
-                    if (g) g[goff(k + 1) + NS + l] = rowg(zb, pi, pj, isobs, qox, qoy, qoc).dv;
+                    if (g) g[goff(k + 1) + NS + l] = rowg(zb, pi, pj, isobs, qob + k * qos).dv;
                     if (lg) lg[goff(k + 1) + NS + l] = row(R_YD, k + 1)[l] / df;
                 }
             }

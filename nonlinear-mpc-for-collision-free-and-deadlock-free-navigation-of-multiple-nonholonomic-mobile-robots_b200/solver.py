@@ -97,10 +97,14 @@ def _flat(a, size, name):
 class Problem:
     """Handle on the CUDA library for one (Nr, N, T, Q, R) problem family."""
 
-    def __init__(self, Nr, N, T, Q=(1.0, 5.0, 0.1), R=(0.5, 0.05), obstacles=None, tuning=None, **opts):
+    def __init__(self, Nr, N, T, Q=(1.0, 5.0, 0.1), R=(0.5, 0.05), obstacles=None, tuning=None, moving_obstacles=None, **opts):
         """obstacles: optional [n_obs, 3] array of static circular obstacles (centre x, y, clearance = rob_dim + r_obs): the
         reference's obstacle-avoidance family (first_scenario_mpc_obstacle_avoidance.py:96-152), see nmpc_create_obstacles.
+        moving_obstacles: n_obs instead of `obstacles` -> the same family with the obstacles in p, one [n_obs, 3] table per
+        instance and stage (p = [x0bar; xs; O[N][n_obs][3]], see nmpc_create_moving_obstacles and params()).
         tuning: optional dict of nmpc_tuning fields (convoy, ctas_per_sm, force_block_path, thread_min_batch)."""
+        if obstacles is not None and moving_obstacles is not None:
+            raise ValueError("obstacles= and moving_obstacles= are mutually exclusive")
         self.L = lib()
         self.desc = Desc(int(Nr), int(N), float(T), (C.c_double * 3)(*[float(q) for q in Q]),
                          (C.c_double * 2)(*[float(r) for r in R]))
@@ -108,10 +112,16 @@ class Problem:
         self.h = C.c_void_p()
         self.obstacles = None if obstacles is None else np.ascontiguousarray(np.asarray(obstacles, dtype=np.float64).reshape(-1, 3))
         self.tuning = default_tuning(**(tuning or {}))
-        check(self.L.nmpc_create_tuned(C.byref(self.desc), C.byref(self.opts), C.byref(self.tuning),
-                                       0 if self.obstacles is None else int(self.obstacles.shape[0]),
-                                       None if self.obstacles is None else self.obstacles.ctypes.data, C.byref(self.h)))
-        self.nobs = 0 if self.obstacles is None else int(self.obstacles.shape[0])
+        self.moving = moving_obstacles is not None
+        if self.moving:
+            check(self.L.nmpc_create_moving_obstacles(C.byref(self.desc), C.byref(self.opts), C.byref(self.tuning),
+                                                      int(moving_obstacles), C.byref(self.h)))
+            self.nobs = int(moving_obstacles)
+        else:
+            check(self.L.nmpc_create_tuned(C.byref(self.desc), C.byref(self.opts), C.byref(self.tuning),
+                                           0 if self.obstacles is None else int(self.obstacles.shape[0]),
+                                           None if self.obstacles is None else self.obstacles.ctypes.data, C.byref(self.h)))
+            self.nobs = 0 if self.obstacles is None else int(self.obstacles.shape[0])
         self.Nr, self.N, self.T = int(Nr), int(N), float(T)
         self.ns, self.nc = 3 * self.Nr, 2 * self.Nr
         self.M = self.Nr * (self.Nr - 1) // 2
@@ -156,6 +166,24 @@ class Problem:
         if x0.ndim == 1:
             return np.concatenate([np.tile(x0, self.N + 1), np.zeros(self.nc * self.N)])
         return np.concatenate([np.tile(x0, (1, self.N + 1)), np.zeros((x0.shape[0], self.nc * self.N))], axis=1)
+
+    def params(self, x0bar, xs, obstacles=None):
+        """p [B, np] from x0bar [B, 3Nr], xs [B, 3Nr] and, for moving_obstacles, obstacles [B, N, n_obs, 3] (ox, oy, clearance of
+        every obstacle at every stage).  NumPy arrays give a NumPy array, CUDA tensors a contiguous float64 tensor on their device."""
+        B = x0bar.shape[0]
+        if tuple(x0bar.shape) != (B, self.ns) or tuple(xs.shape) != (B, self.ns):
+            raise ValueError("x0bar and xs must be [B, %d]" % self.ns)
+        parts = [x0bar, xs]
+        if self.moving:
+            if obstacles is None or tuple(obstacles.shape) != (B, self.N, self.nobs, 3):
+                raise ValueError("obstacles must be [B, N, n_obs, 3] = [%d, %d, %d, 3]" % (B, self.N, self.nobs))
+            parts.append(obstacles.reshape(B, -1))
+        elif obstacles is not None:
+            raise ValueError("obstacles go into p only for Problem(moving_obstacles=n_obs)")
+        if isinstance(x0bar, np.ndarray):
+            return np.ascontiguousarray(np.concatenate([np.asarray(a, np.float64) for a in parts], axis=1))
+        torch = self._torch()
+        return torch.cat([a.to(torch.float64) for a in parts], dim=1).contiguous()
 
     def launch_count(self):
         return int(self.L.nmpc_launch_count(self.h))
@@ -229,6 +257,8 @@ class Problem:
         dev = x0.device
         if any(t.device != dev for t in (p, lbx, ubx, lbg, ubg)):
             raise ValueError("all inputs must live on the same CUDA device")
+        if self.np_ > 0 and tuple(p.shape) != (B, self.np_):
+            raise ValueError("p must be [B, %d], got %s" % (self.np_, tuple(p.shape)))
         ws = self.workspace(B, bool(batched), dev)
         o = out if out is not None else {}
         o.setdefault("x", torch.empty((B, self.n), dtype=torch.float64, device=dev))
@@ -290,15 +320,27 @@ class Problem:
         return o
 
 
-def closed_loop(prob, P, lbx, ubx, lbg, ubg, steps, tol=1e-1, dmin=None):
+def closed_loop(prob, P, lbx, ubx, lbg, ubg, steps, tol=1e-1, dmin=None, obstacles=None):
     """Batched closed-loop driver, device resident (SURVEY.md 8f-1): the reference's loop body
     (centralized_six_robots_implementation.py:416-465 with the Euler plant of casadi_test.py:17-26) for B
     independent instances at once.  Per step: solve -> apply u_0 through the plant -> reference shift as the next
     guess; instances whose ||x - xs|| <= tol stop moving (the loop guard at :416).  Returns a dict of CUDA tensors:
-    traj [steps+1,B,3Nr], u [steps,B,2Nr], status [steps,B], iters [steps,B], active [steps,B], min_dist [B]."""
+    traj [steps+1,B,3Nr], u [steps,B,2Nr], status [steps,B], iters [steps,B], active [steps,B], min_dist [B].
+    obstacles (Problem(moving_obstacles=n_obs) only): CUDA float64 [steps+N, B, n_obs, 3], the obstacles' positions and
+    clearances over time; step t solves with the window t..t+N-1 in p (P then needs only its first 6Nr columns), and the
+    result gains min_clearance [B] = min over time, robots and obstacles of rho - clearance between the plant state and the
+    obstacles at the same time."""
     torch = prob._torch()
     B, ns, nc, N = P.shape[0], prob.ns, prob.nc, prob.N
-    p = P.clone()
+    if obstacles is not None:
+        if not getattr(prob, "moving", False):
+            raise ValueError("obstacles= needs a Problem(moving_obstacles=n_obs)")
+        if not (obstacles.is_cuda and obstacles.dtype == torch.float64) or tuple(obstacles.shape) != (steps + N, B, prob.nobs, 3):
+            raise ValueError("obstacles must be a float64 CUDA tensor [steps + N, B, n_obs, 3] = [%d, %d, %d, 3]"
+                             % (steps + N, B, prob.nobs))
+        p = torch.cat([P[:, :2 * ns], torch.empty((B, 3 * N * prob.nobs), dtype=torch.float64, device=P.device)], dim=1)
+    else:
+        p = P.clone()
     x0 = torch.cat([p[:, :ns].repeat(1, N + 1), torch.zeros((B, nc * N), dtype=torch.float64, device=P.device)], dim=1).contiguous()
     traj = torch.empty((steps + 1, B, ns), dtype=torch.float64, device=P.device)
     us = torch.zeros((steps, B, nc), dtype=torch.float64, device=P.device)
@@ -310,7 +352,9 @@ def closed_loop(prob, P, lbx, ubx, lbg, ubg, steps, tol=1e-1, dmin=None):
     for t in range(steps):
         if t == 0:
             prob.set_order(None)
-        active = (p[:, :ns] - p[:, ns:]).norm(dim=1) > tol
+        if obstacles is not None:
+            p[:, 2 * ns:] = obstacles[t:t + N].permute(1, 0, 2, 3).reshape(B, -1)
+        active = (p[:, :ns] - p[:, ns:2 * ns]).norm(dim=1) > tol
         act[t] = active
         prob.solve(x0, p, lbx, ubx, lbg, ubg, want=(), out=out)
         u0 = out["x"][:, ns * (N + 1):ns * (N + 1) + nc]
@@ -328,6 +372,11 @@ def closed_loop(prob, P, lbx, ubx, lbg, ubg, steps, tol=1e-1, dmin=None):
         d = (pos[:, :, :, None, :] - pos[:, :, None, :, :]).norm(dim=-1)
         d = d + torch.eye(prob.Nr, device=P.device, dtype=torch.float64)[None, None] * 1e9
         res["min_dist"] = d.amin(dim=(0, 2, 3))
+    if obstacles is not None:
+        pos = traj.reshape(steps + 1, B, prob.Nr, 3)[..., :2]
+        ob = obstacles[:steps + 1]
+        rho = (pos[:, :, :, None, :] - ob[:, :, None, :, :2]).norm(dim=-1)
+        res["min_clearance"] = (rho - ob[:, :, None, :, 2]).amin(dim=(0, 2, 3))
     return res
 
 
@@ -388,7 +437,19 @@ class NlpSolver:
             lam_p[:P.ns] = -o["lam_g"][0, :P.ns]
             Xk = o["x"][0, :P.ns * (P.N + 1)].reshape(P.N + 1, P.ns)[:P.N]
             Qd = np.tile(np.asarray(list(P.desc.Q), float), P.Nr)
-            lam_p[P.ns:] = -2.0 * Qd * (Xk - np.asarray(_flat(p, P.np_, "p"))[P.ns:][None]).sum(axis=0)
+            pv = np.asarray(_flat(p, P.np_, "p"))
+            lam_p[P.ns:2 * P.ns] = -2.0 * Qd * (Xk - pv[P.ns:2 * P.ns][None]).sum(axis=0)
+            if getattr(P, "moving", False):
+                # obstacle block O[k][o] = (ox, oy, c): row (k, i, o) = rho - c with rho = |pos_{k,i} - (ox, oy)|, so
+                # dL/d(ox, oy) = -sum_i lam (pos - o) / rho and dL/dc = -sum_i lam
+                O = pv[2 * P.ns:].reshape(P.N, P.nobs, 3)
+                lam = o["lam_g"][0, P.ns:].reshape(P.N, P.ns + P.M + P.Nr * P.nobs)[:, P.ns + P.M:].reshape(P.N, P.Nr, P.nobs)
+                d = Xk.reshape(P.N, P.Nr, 3)[:, :, None, :2] - O[:, None, :, :2]
+                gxy = d / np.linalg.norm(d, axis=-1, keepdims=True)
+                lam_o = np.empty((P.N, P.nobs, 3))
+                lam_o[..., :2] = -(lam[..., None] * gxy).sum(axis=1)
+                lam_o[..., 2] = -lam.sum(axis=1)
+                lam_p[2 * P.ns:] = lam_o.ravel()
         return {"x": DM(o["x"][0]), "f": DM(o["f"][:1]), "g": DM(o["g"][0]), "lam_x": DM(o["lam_x"][0]),
                 "lam_g": DM(o["lam_g"][0]), "lam_p": DM(lam_p)}
 
@@ -404,6 +465,8 @@ def nlpsol(name, plugin, nlp, opts=None):
 
     `nlp` is a problem descriptor instead of CasADi's symbolic dict:
         {'family': 'unicycle_centralized', 'Nr', 'N', 'T', 'Q': (3,), 'R': (2,)}
+        {'family': 'unicycle_obstacles', ..., 'obstacles': [[x, y, clearance], ...]}
+        {'family': 'unicycle_moving_obstacles', ..., 'n_obs'}: the obstacles in p = [x0bar; xs; O[N][n_obs][3]]
     `opts` uses the reference's layout: {'print_time': 0, 'ipopt': {'max_iter': 2000, ...}}.
     """
     if plugin not in ("ipopt", "b200ipm"):
@@ -412,13 +475,18 @@ def nlpsol(name, plugin, nlp, opts=None):
         ip = dict((opts or {}).get("ipopt", {}))
         kw = {k: v for k, v in ip.items() if k in _IPOPT_KEYS}
         return NlpSolver(name, SmallOcp("van_der_pol", nlp.get("N", 20), nlp.get("T", 10.0), nlp.get("rk_steps", 4), **kw))
-    if not isinstance(nlp, dict) or nlp.get("family", "unicycle_centralized") not in ("unicycle_centralized", "unicycle_obstacles"):
-        raise ValueError("nlp must be a descriptor {'family':'unicycle_centralized'|'unicycle_obstacles','Nr','N','T',...}")
+    if not isinstance(nlp, dict) or nlp.get("family", "unicycle_centralized") not in ("unicycle_centralized", "unicycle_obstacles",
+                                                                                   "unicycle_moving_obstacles"):
+        raise ValueError("nlp must be a descriptor {'family':'unicycle_centralized'|'unicycle_obstacles'|"
+                         "'unicycle_moving_obstacles','Nr','N','T',...}")
+    if nlp.get("family") == "unicycle_moving_obstacles" and nlp.get("n_obs") is None:
+        raise ValueError("family 'unicycle_moving_obstacles' needs 'n_obs'")
     if nlp.get("family") == "unicycle_obstacles" and nlp.get("obstacles") is None:
         raise ValueError("family 'unicycle_obstacles' needs 'obstacles': [[x, y, clearance], ...]")
     ip = dict((opts or {}).get("ipopt", {}))
     ip.update({k: v for k, v in (opts or {}).items() if k in _IPOPT_KEYS})
     kw = {k: v for k, v in ip.items() if k in _IPOPT_KEYS}          # print_level etc. are accepted and ignored
     prob = Problem(nlp["Nr"], nlp["N"], nlp["T"], nlp.get("Q", (1.0, 5.0, 0.1)), nlp.get("R", (0.5, 0.05)),
-                   obstacles=nlp.get("obstacles") if nlp.get("family") == "unicycle_obstacles" else None, **kw)
+                   obstacles=nlp.get("obstacles") if nlp.get("family") == "unicycle_obstacles" else None,
+                   moving_obstacles=nlp.get("n_obs") if nlp.get("family") == "unicycle_moving_obstacles" else None, **kw)
     return NlpSolver(name, prob)
