@@ -105,7 +105,7 @@ int nmpc_create_tuned(const nmpc_desc *d, const nmpc_opts *o, const nmpc_tuning 
 
 int nmpc_n(const nmpc_handle *h);        /* decision variables                         */
 int nmpc_mg(const nmpc_handle *h);       /* constraint rows                            */
-int nmpc_np(const nmpc_handle *h);       /* parameters (6 Nr; + 3 N n_obs with obstacles in p) */
+int nmpc_np(const nmpc_handle *h);       /* parameters (6 Nr; + 3 N n_obs with obstacles in p; 3 Nr + 5 Nr N tracking) */
 int nmpc_nnz_jac(const nmpc_handle *h);  /* 3Nr + N(11Nr+4M)   CasADi's CCS of dg/dw   */
 int nmpc_nnz_hess(const nmpc_handle *h); /* N(6Nr+2M)          lower triangle          */
 
@@ -147,6 +147,20 @@ int nmpc_create_obstacles(const nmpc_desc *d, const nmpc_opts *o, int n_obs, con
  * data and are NOT validated (a negative one is the caller's responsibility).  1 <= n_obs <= 32, else NMPC_EINVAL; t == NULL
  * means the default tuning.  nmpc_eval and the CCS patterns return NMPC_ENOTSUP; nmpc_shift and nmpc_plant work. */
 int nmpc_create_moving_obstacles(const nmpc_desc *d, const nmpc_opts *o, const nmpc_tuning *t, int n_obs, nmpc_handle **out);
+
+/* Trajectory tracking: the centralized family with a time-varying state AND control reference per instance and stage (e.g. the
+ * output of a planner), instead of one goal xs.
+ *     p = [x0bar (3 Nr); Z[0]; ...; Z[N-1]],  Z[k] = [xr_k (3 Nr); ur_k (2 Nr)] laid out like the stage vector z_k = [X_k; U_k],
+ *     nmpc_np = 3 Nr + 5 Nr N,
+ *     cost = sum_{k<N} (X_k - xr_k)' Q (X_k - xr_k) + (U_k - ur_k)' R (U_k - ur_k)   (no terminal term, no wrap of theta).
+ * ur_k is the feed-forward control: with ur = 0, R pulls v and omega toward zero and the robot lags a moving reference.
+ * Everything else is what nmpc_create gives: variables, g rows (with the dummy rows of block 0), mg, bounds, nnz_jac / nnz_hess
+ * and the CCS patterns, status, stats, the path (warp-per-instance for 1..10 robots, dense blocks for 11..64;
+ * t->force_block_path is honoured, t == NULL means the default tuning), nmpc_shift, nmpc_plant and nmpc_set_order.
+ * Guarantee: if every Z[k] = [xs; 0], the outputs are bit for bit those of nmpc_create with p = [x0bar; xs].
+ * nmpc_eval works on the handle with p [B, nmpc_np]: its gradient includes both references, its Jacobian and Hessian are
+ * those of nmpc_create. */
+int nmpc_create_tracking(const nmpc_desc *d, const nmpc_opts *o, const nmpc_tuning *t, nmpc_handle **out);
 
 /* Small generic optimal-control problems, one GPU thread per instance.  model NMPC_OCP_VAN_DER_POL is the direct-multiple-shooting
  * demo of mpc_pose_control_casadi.py:22-114: 2 states, 1 control, N intervals over the horizon T, each integrated by rk_steps RK4
@@ -193,7 +207,7 @@ int nmpc_plant(nmpc_handle *h, int B, const double *state, const double *x_opt, 
                void *stream);
 
 /* Stand-alone derivative evaluation (what CasADi's AD hands IPOPT, SURVEY.md a17): for B points
- * w [B,n], p [B,6Nr], lam_g [B,mg]:  f [B], grad [B,n], g [B,mg], jac [B,nnz_jac] and
+ * w [B,n], p [B,nmpc_np] (6 Nr; a tracking handle's 3 Nr + 5 Nr N), lam_g [B,mg]:  f [B], grad [B,n], g [B,mg], jac [B,nnz_jac] and
  * hess [B,nnz_hess] (CCS value order of nmpc_jac_pattern / nmpc_hess_pattern).  Outputs may be NULL. */
 int nmpc_eval(nmpc_handle *h, int B, const double *w, const double *p, const double *lam_g,
               double *f, double *grad, double *g, double *jac, double *hess, void *stream);

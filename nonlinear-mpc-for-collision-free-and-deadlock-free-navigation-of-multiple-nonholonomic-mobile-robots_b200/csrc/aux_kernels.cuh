@@ -25,9 +25,11 @@ struct NmpcEvalTables {
 // the Jacobian and the Hessian of the Lagrangian through the position tables; returns this thread's share of f.  The arrays
 // may live in shared memory (eval_kernel: the record is assembled on chip and leaves through bulk stores) or directly in global
 // memory (eval_kernel_big: records too large for shared memory, e.g. 2.5 MB at 64 robots); NULL outputs are skipped.
+// rstr: stride of the reference in p after x0bar.  0: the setpoint xs (p = [x0bar; xs]); 5 Nr: a tracking handle's
+// p = [x0bar; Z[N][5 Nr]], Z[k] = [xr_k; ur_k], whose control reference enters the cost as (U_k - ur_k)' R (U_k - ur_k).
 __device__ __forceinline__ double eval_point_items(int Nr, int N, double T, const double *Qw, const double *Rw, const double *sw,
                                                    const double *sl, const double *sp, double *sgrad, double *sg, double *sj,
-                                                   double *shs, const NmpcEvalTables &tb, bool lam, bool hess)
+                                                   double *shs, const NmpcEvalTables &tb, bool lam, bool hess, int rstr)
 {
     const int ns = 3 * Nr, nc = 2 * Nr, M = Nr * (Nr - 1) / 2, S = N + 1, blk = ns + M, nX = ns * S;
     double facc = 0.0;
@@ -40,11 +42,13 @@ __device__ __forceinline__ double eval_point_items(int Nr, int N, double T, cons
                 const double x = sw[ix], y = sw[ix + 1], th = sw[ix + 2], v = sw[iu], om = sw[iu + 1];
                 double s_, c_;
                 sincos(th, &s_, &c_);
-                const double ex = x - sp[ns + 3 * i], ey = y - sp[ns + 3 * i + 1], et = th - sp[ns + 3 * i + 2];
-                facc += Qw[0] * ex * ex + Qw[1] * ey * ey + Qw[2] * et * et + Rw[0] * v * v + Rw[1] * om * om;
+                const double *rk = sp + ns + k * rstr;
+                const double ex = x - rk[3 * i], ey = y - rk[3 * i + 1], et = th - rk[3 * i + 2];
+                const double ev = rstr ? v - rk[ns + 2 * i] : v, eo = rstr ? om - rk[ns + 2 * i + 1] : om;
+                facc += Qw[0] * ex * ex + Qw[1] * ey * ey + Qw[2] * et * et + Rw[0] * ev * ev + Rw[1] * eo * eo;
                 if (sgrad) {
                     sgrad[ix] = 2 * Qw[0] * ex; sgrad[ix + 1] = 2 * Qw[1] * ey; sgrad[ix + 2] = 2 * Qw[2] * et;
-                    sgrad[iu] = 2 * Rw[0] * v; sgrad[iu + 1] = 2 * Rw[1] * om;
+                    sgrad[iu] = 2 * Rw[0] * ev; sgrad[iu + 1] = 2 * Rw[1] * eo;
                 }
                 if (sg) {
                     sg[r0] = sw[ix + ns] - (x + T * v * c_);
@@ -108,7 +112,8 @@ __device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.comm
 __device__ __forceinline__ void bulk_wait_read_all() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
 __device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 
-template <int PF>
+// TRK: a tracking handle's p (np = 3 Nr + 5 Nr N = n, so the prefetch of p takes PF registers like w); else p = [x0bar; xs]
+template <int PF, bool TRK>
 __global__ void __launch_bounds__(256) eval_kernel(int Nr, int N, double T, double Q0, double Q1, double Q2, double R0,
                                                    double R1, int B, const double *__restrict__ w, const double *__restrict__ p,
                                                    const double *__restrict__ lam, double *__restrict__ f, double *__restrict__ grad,
@@ -119,13 +124,14 @@ __global__ void __launch_bounds__(256) eval_kernel(int Nr, int N, double T, doub
     const int ns = 3 * Nr, nc = 2 * Nr, M = Nr * (Nr - 1) / 2, S = N + 1, blk = ns + M;
     const int n = ns * S + nc * N, mg = S * blk, nX = ns * S;
     const int nj = 3 * Nr + N * (11 * Nr + 4 * M), nh = N * (6 * Nr + 2 * M);
+    const int np = TRK ? ns + N * (ns + nc) : 2 * ns, rstr = TRK ? ns + nc : 0;
     auto ev = [](int v) { return (v + 1) & ~1; };   // every segment starts 16-byte aligned (128-bit write-back)
-    double *sw = sh, *sl = sw + ev(n), *sp = sl + ev(mg), *sgrad = sp + ev(2 * ns), *sg0 = sgrad + ev(n), *sj = sg0 + ev(mg + 1),
+    double *sw = sh, *sl = sw + ev(n), *sp = sl + ev(mg), *sgrad = sp + ev(np), *sg0 = sgrad + ev(n), *sj = sg0 + ev(mg + 1),
            *shs = sj + ev(nj), *sred = shs + ev(nh);
     const double Qw[3] = {Q0, Q1, Q2}, Rw[2] = {R0, R1};
     // The inputs of the next point are fetched into PF registers per array per thread right after the evaluation of
     // the current point, so their HBM latency overlaps the write-back (PF = ceil(max(n, mg) / 256), 0 = no prefetch).
-    double rw[PF > 0 ? PF : 1], rl[PF > 0 ? PF : 1], rp = 0.0;
+    double rw[PF > 0 ? PF : 1], rl[PF > 0 ? PF : 1], rq[(TRK && PF > 0) ? PF : 1], rp = 0.0;
     auto fetch = [&](int b) {
         if (PF == 0 || b >= B) return;
 #pragma unroll
@@ -133,8 +139,9 @@ __global__ void __launch_bounds__(256) eval_kernel(int Nr, int N, double T, doub
             const int i = threadIdx.x + j * 256;
             rw[j] = i < n ? w[(size_t)b * n + i] : 0.0;
             rl[j] = (lam && i < mg) ? lam[(size_t)b * mg + i] : 0.0;
+            if (TRK) rq[j] = i < np ? p[(size_t)b * np + i] : 0.0;
         }
-        rp = (int)threadIdx.x < 2 * ns ? p[(size_t)b * 2 * ns + threadIdx.x] : 0.0;
+        if (!TRK) rp = (int)threadIdx.x < 2 * ns ? p[(size_t)b * 2 * ns + threadIdx.x] : 0.0;
     };
     fetch(blockIdx.x);
     for (int b = blockIdx.x; b < B; b += gridDim.x) {
@@ -147,18 +154,20 @@ __global__ void __launch_bounds__(256) eval_kernel(int Nr, int N, double T, doub
                 const int i = threadIdx.x + j * 256;
                 if (i < n) sw[i] = rw[j];
                 if (lam && i < mg) sl[i] = rl[j];
+                if (TRK && i < np) sp[i] = rq[j];
             }
-            if ((int)threadIdx.x < 2 * ns) sp[threadIdx.x] = rp;
+            if (!TRK && (int)threadIdx.x < 2 * ns) sp[threadIdx.x] = rp;
             if (threadIdx.x == 0) bulk_wait_read_all();   // the previous point's bulk stores have finished reading the record
         } else {
             if (threadIdx.x == 0) bulk_wait_read_all();
             const double *wb = w + (size_t)b * n;
             for (int i = threadIdx.x; i < n; i += blockDim.x) sw[i] = wb[i];
-            for (int i = threadIdx.x; i < 2 * ns; i += blockDim.x) sp[i] = p[(size_t)b * 2 * ns + i];
+            for (int i = threadIdx.x; i < np; i += blockDim.x) sp[i] = p[(size_t)b * np + i];
             if (lam) for (int i = threadIdx.x; i < mg; i += blockDim.x) sl[i] = lam[(size_t)b * mg + i];
         }
         __syncthreads();
-        double facc = eval_point_items(Nr, N, T, Qw, Rw, sw, sl, sp, sgrad, sg, sj, shs, tb, lam != nullptr, hess != nullptr);
+        double facc = eval_point_items(Nr, N, T, Qw, Rw, sw, sl, sp, sgrad, sg, sj, shs, tb, lam != nullptr, hess != nullptr,
+                                       rstr);
         // block reduction of f
         for (int m = 16; m > 0; m >>= 1) facc += __shfl_xor_sync(0xffffffffu, facc, m);
         if ((threadIdx.x & 31) == 0) sred[threadIdx.x >> 5] = facc;
@@ -205,11 +214,12 @@ __global__ void __launch_bounds__(256) eval_kernel(int Nr, int N, double T, doub
 }
 
 // Records that do not fit shared memory (more than ~11 robots at N = 20): same work items, written straight to global memory.
+// np, rstr: width of p and stride of its reference (see eval_point_items)
 __global__ void __launch_bounds__(256) eval_kernel_big(int Nr, int N, double T, double Q0, double Q1, double Q2, double R0, double R1, int B,
                                                        const double *__restrict__ w, const double *__restrict__ p,
                                                        const double *__restrict__ lam, double *__restrict__ f, double *__restrict__ grad,
                                                        double *__restrict__ g, double *__restrict__ jac, double *__restrict__ hess,
-                                                       NmpcEvalTables tb)
+                                                       NmpcEvalTables tb, int np, int rstr)
 {
     __shared__ double sred[8];
     const int ns = 3 * Nr, nc = 2 * Nr, M = Nr * (Nr - 1) / 2, S = N + 1;
@@ -217,9 +227,9 @@ __global__ void __launch_bounds__(256) eval_kernel_big(int Nr, int N, double T, 
     const size_t nj = 3 * (size_t)Nr + (size_t)N * (11 * Nr + 4 * M), nh = (size_t)N * (6 * Nr + 2 * M);
     const double Qw[3] = {Q0, Q1, Q2}, Rw[2] = {R0, R1};
     for (int b = blockIdx.x; b < B; b += gridDim.x) {
-        double facc = eval_point_items(Nr, N, T, Qw, Rw, w + b * n, lam ? lam + b * mg : nullptr, p + (size_t)b * 2 * ns,
+        double facc = eval_point_items(Nr, N, T, Qw, Rw, w + b * n, lam ? lam + b * mg : nullptr, p + (size_t)b * np,
                                        grad ? grad + b * n : nullptr, g ? g + b * mg : nullptr, jac ? jac + b * nj : nullptr,
-                                       hess ? hess + b * nh : nullptr, tb, lam != nullptr, hess != nullptr);
+                                       hess ? hess + b * nh : nullptr, tb, lam != nullptr, hess != nullptr, rstr);
         for (int m = 16; m > 0; m >>= 1) facc += __shfl_xor_sync(0xffffffffu, facc, m);
         if ((threadIdx.x & 31) == 0) sred[threadIdx.x >> 5] = facc;
         __syncthreads();

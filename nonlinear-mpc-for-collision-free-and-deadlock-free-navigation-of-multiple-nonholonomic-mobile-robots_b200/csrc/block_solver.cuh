@@ -70,6 +70,7 @@ struct BlockSolver {
     int Mp, nobs, family;                                 // pair rows, obstacles per robot, row layout (0 centralized, 1 obstacles)
     const double *obs;                                    // [nobs][3] of stage 0: centre x, y, clearance radius
     int ostr;                                             // doubles from one stage's obstacle table to the next (0: static obstacles)
+    int nref, rstr;                                       // reference in p after x0bar: variables per stage, stride (see ref())
     const double *BL, *BU, *CE, *DL, *DU, *pp;
     const int *pairs;
     double *Pall, *Yall, *Lall, *Wg;   // Wg: Linv_II L_IJ blocks of the stage being factored (see factor, step D)
@@ -108,8 +109,9 @@ struct BlockSolver {
     __device__ __forceinline__ void mid_sync() const {}
     __device__ __forceinline__ int pairidx(int a, int b) const { return a * (2 * Nr - a - 1) / 2 + (b - a - 1); }
     __device__ __forceinline__ double qw(int l) const { return l < ns ? 2.0 * P.Q[l % 3] : 2.0 * P.R[(l - ns) & 1]; }
-    __device__ __forceinline__ double xs(int l) const { return l < ns ? pp[ns + l] : 0.0; }
-    __device__ __forceinline__ double gradf(int k, int l, double z) const { return k < N ? qw(l) * (z - xs(l)) : 0.0; }
+    // reference of variable l at stage k: the setpoint xs (nref = ns, rstr = 0), or Z[k] of a tracking handle (nref = rstr = nz)
+    __device__ __forceinline__ double ref(int k, int l) const { return l < nref ? pp[ns + k * rstr + l] : 0.0; }
+    __device__ __forceinline__ double gradf(int k, int l, double z) const { return k < N ? qw(l) * (z - ref(k, l)) : 0.0; }
     __device__ __forceinline__ int nvalid(int k) const { return k < N ? nz : ns; }
 
     // FP64 tensor instruction: D (8 x 8) += A (8 x 4) B (4 x 8) over a warp.  Lane l = 4 g + t holds A[g][t], B[t][g] and D[g][2 t], D[g][2 t + 1].
@@ -164,6 +166,12 @@ struct BlockSolver {
         CE = br + (long long)NMPC_BR_CE * S * W; DL = br + (long long)NMPC_BR_DL * S * W;
         DU = br + (long long)NMPC_BR_DU * S * W;
         pp = P.p + (long long)inst * P.np;
+        {   // reference after x0bar: one setpoint xs (np = 2 ns), or Z[N][nz] of a tracking handle (np = ns + N nz, never 2 ns).
+            // (Told apart by np rather than by a flag in NmpcSolveParams: a larger parameter block would change the frame, and so
+            // the code, of every warp-path kernel, which copies it to local memory.)
+            const bool trk = family == 0 && P.np == ns + N * nz;
+            nref = trk ? nz : ns; rstr = trk ? nz : 0;
+        }
         // obstacles in p: [N][nobs][3] after x0bar and xs, one table per stage; else the handle's table at every stage
         obs = P.obs_in_p ? pp + 2 * ns : P.obs; ostr = P.obs_in_p ? 3 * nobs : 0;
         pairs = P.pairs;
@@ -357,7 +365,7 @@ struct BlockSolver {
             if (hu) slog += log(hi - zk);
             if (hl && !hu) sdamp += zk - lo;
             if (hu && !hl) sdamp += hi - zk;
-            if (k < N) { const double e = zk - xs(l); fo += 0.5 * qw(l) * e * e; }
+            if (k < N) { const double e = zk - ref(k, l); fo += 0.5 * qw(l) * e * e; }
             if (full) {
                 const double zl = row(R_ZL, k)[l], zu = row(R_ZU, k)[l];
                 double r = df * gradf(k, l, zk) - zl + zu;
@@ -1255,7 +1263,7 @@ struct BlockSolver {
             const long long xi = l < ns ? (long long)k * ns + l : (long long)ns * S + (long long)k * nc + (l - ns);
             x[xi] = zk;
             if (lx) lx[xi] = (row(R_ZU, k)[l] - row(R_ZL, k)[l]) / df;
-            if (k < N) { const double e = zk - xs(l); fo += 0.5 * qw(l) * e * e; }
+            if (k < N) { const double e = zk - ref(k, l); fo += 0.5 * qw(l) * e * e; }
         }
         for (int idx = tid; idx < S * ns; idx += nt) {
             const int k = idx / ns, l = idx - k * ns;

@@ -60,23 +60,23 @@ extern "C" void nmpc_default_opts(nmpc_opts *o)
 // threads per CTA and instances ("teams") per CTA: one warp per instance up to 6 robots (4 per CTA, 3 CTAs per SM);
 // 7..10 robots use the two-warp team (2 per CTA on named barriers, 2 CTAs per SM: 255 registers per thread).  The
 // one-warp teams of a CTA are a convoy group (WarpSolver::iter_sync).
-template <int NR, bool OBS = false> struct SolveCfg {
-    static constexpr int LW = WarpSolver<NR, OBS>::LW;
+template <int NR, bool OBS = false, bool TRK = false> struct SolveCfg {
+    static constexpr int LW = WarpSolver<NR, OBS, TRK>::LW;
     static constexpr int THREADS = LW == 32 ? SOLVE_WARPS * 32 : 128;
     static constexpr int TEAMS = THREADS / LW;
     static constexpr int MIN_CTAS = LW == 32 ? SOLVE_MIN_CTAS : 2;
 };
 
-// OBS: the static-obstacle family (its own instantiation, see WarpSolver)
-template <int NR, bool OBS = false>
-__global__ void __launch_bounds__((SolveCfg<NR, OBS>::THREADS), (SolveCfg<NR, OBS>::MIN_CTAS)) solve_kernel(const NmpcSolveParams P)
+// OBS: the static-obstacle family; TRK: trajectory tracking (each its own instantiation, see WarpSolver)
+template <int NR, bool OBS = false, bool TRK = false>
+__global__ void __launch_bounds__((SolveCfg<NR, OBS, TRK>::THREADS), (SolveCfg<NR, OBS, TRK>::MIN_CTAS)) solve_kernel(const NmpcSolveParams P)
 {
     extern __shared__ double smem[];
-    typedef WarpSolver<NR, OBS> WSol;
-    constexpr int LW = SolveCfg<NR, OBS>::LW;
+    typedef WarpSolver<NR, OBS, TRK> WSol;
+    constexpr int LW = SolveCfg<NR, OBS, TRK>::LW;
     const int team = threadIdx.x / LW, tl = threadIdx.x & (LW - 1);
     double *sm = smem + (size_t)team * WSol::SM_DOUBLES;
-    double *ws = P.ws + ((long long)blockIdx.x * SolveCfg<NR, OBS>::TEAMS + team) * P.ws_stride;
+    double *ws = P.ws + ((long long)blockIdx.x * SolveCfg<NR, OBS, TRK>::TEAMS + team) * P.ws_stride;
     WSol s(P, sm, ws);
     s.init_team();
     for (;;) {
@@ -112,6 +112,7 @@ struct nmpc_handle {
     int nobs, family, rk_steps;               // static obstacles per robot; family: 0 centralized, 1 obstacles, 2 small OCP (thread per instance)
     double *d_obs;                            // [nobs][3] on the device
     bool obs_in_p;                            // obstacle family with the geometry in p (per instance and stage): no d_obs
+    bool tracking;                            // centralized family tracking a per-stage reference (nmpc_create_tracking)
     bool thread_ok;                           // a thread-per-instance kernel exists for this problem (small-OCP family; one robot with
                                               // static obstacles): used for the small-OCP family always, else from thread_min_batch on
     size_t t_ws_doubles;                      // its scratch per instance
@@ -180,21 +181,23 @@ static void build_tables(nmpc_handle *h, std::vector<int> &tab)
     tab.insert(tab.end(), hs.begin(), hs.end());
 }
 
-template <int NR, bool OBS = false> static size_t slot_doubles(int N) { return (size_t)WarpSolver<NR, OBS>::ws_doubles(N); }
-template <int NR, bool OBS = false> static cudaError_t config_solve(nmpc_handle *h)
+template <int NR, bool OBS = false, bool TRK = false> static size_t slot_doubles(int N) { return (size_t)WarpSolver<NR, OBS, TRK>::ws_doubles(N); }
+template <int NR, bool OBS = false, bool TRK = false> static cudaError_t config_solve(nmpc_handle *h)
 {
-    h->lw = SolveCfg<NR, OBS>::LW; h->teams_per_cta = SolveCfg<NR, OBS>::TEAMS; h->threads = SolveCfg<NR, OBS>::THREADS;
-    h->solve_smem = (size_t)SolveCfg<NR, OBS>::TEAMS * WarpSolver<NR, OBS>::SM_DOUBLES * sizeof(double);
-    cudaError_t e = cudaFuncSetAttribute(solve_kernel<NR, OBS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->solve_smem);
+    typedef SolveCfg<NR, OBS, TRK> Cfg;
+    h->lw = Cfg::LW; h->teams_per_cta = Cfg::TEAMS; h->threads = Cfg::THREADS;
+    h->solve_smem = (size_t)Cfg::TEAMS * WarpSolver<NR, OBS, TRK>::SM_DOUBLES * sizeof(double);
+    cudaError_t e = cudaFuncSetAttribute(solve_kernel<NR, OBS, TRK>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->solve_smem);
     if (e != cudaSuccess) return e;
     int nb = 0;
-    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, solve_kernel<NR, OBS>, SolveCfg<NR, OBS>::THREADS, h->solve_smem);
+    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, solve_kernel<NR, OBS, TRK>, Cfg::THREADS, h->solve_smem);
     h->ctas_per_sm = nb > 0 ? nb : 1;
     if (h->tune.ctas_per_sm >= 1 && h->tune.ctas_per_sm < h->ctas_per_sm) h->ctas_per_sm = h->tune.ctas_per_sm;
     return e;
 }
 
-static int create_impl(const nmpc_desc *d, const nmpc_opts *o, const nmpc_tuning *t, int nobs, const double *obs, bool obs_in_p, nmpc_handle **out);
+static int create_impl(const nmpc_desc *d, const nmpc_opts *o, const nmpc_tuning *t, int nobs, const double *obs, bool obs_in_p,
+                       bool tracking, nmpc_handle **out);
 
 extern "C" void nmpc_default_tuning(nmpc_tuning *t)
 {
@@ -202,7 +205,7 @@ extern "C" void nmpc_default_tuning(nmpc_tuning *t)
     t->ctas_per_sm = 0; t->force_block_path = 0; t->thread_min_batch = 0;
 }
 
-extern "C" int nmpc_create(const nmpc_desc *d, const nmpc_opts *o, nmpc_handle **out) { return create_impl(d, o, nullptr, 0, nullptr, false, out); }
+extern "C" int nmpc_create(const nmpc_desc *d, const nmpc_opts *o, nmpc_handle **out) { return create_impl(d, o, nullptr, 0, nullptr, false, false, out); }
 
 static int check_obstacles(int n_obs, const double *obs)
 {
@@ -216,21 +219,26 @@ static int check_obstacles(int n_obs, const double *obs)
 extern "C" int nmpc_create_tuned(const nmpc_desc *d, const nmpc_opts *o, const nmpc_tuning *t, int n_obs, const double *obs, nmpc_handle **out)
 {
     if (n_obs != 0) { int rc = check_obstacles(n_obs, obs); if (rc) return rc; }
-    return create_impl(d, o, t, n_obs, n_obs ? obs : nullptr, false, out);
+    return create_impl(d, o, t, n_obs, n_obs ? obs : nullptr, false, false, out);
 }
 
 extern "C" int nmpc_create_obstacles(const nmpc_desc *d, const nmpc_opts *o, int n_obs, const double *obs, nmpc_handle **out)
 {
     int rc = check_obstacles(n_obs, obs);
     if (rc) return rc;
-    return create_impl(d, o, nullptr, n_obs, obs, false, out);
+    return create_impl(d, o, nullptr, n_obs, obs, false, false, out);
 }
 
 extern "C" int nmpc_create_moving_obstacles(const nmpc_desc *d, const nmpc_opts *o, const nmpc_tuning *t, int n_obs, nmpc_handle **out)
 {
     if (n_obs < 1 || n_obs > NMPC_MAX_OBSTACLES)
         return fail(NMPC_EINVAL, "nmpc_create_moving_obstacles: need 1..%d obstacles, got %d", NMPC_MAX_OBSTACLES, n_obs);
-    return create_impl(d, o, t, n_obs, nullptr, true, out);
+    return create_impl(d, o, t, n_obs, nullptr, true, false, out);
+}
+
+extern "C" int nmpc_create_tracking(const nmpc_desc *d, const nmpc_opts *o, const nmpc_tuning *t, nmpc_handle **out)
+{
+    return create_impl(d, o, t, 0, nullptr, false, true, out);
 }
 
 // Small generic OCP family (thread per instance): currently the Van der Pol demo of mpc_pose_control_casadi.py
@@ -260,7 +268,22 @@ extern "C" int nmpc_create_ocp(int model, int N, double T, int rk_steps, const n
     return 0;
 }
 
-static int create_impl(const nmpc_desc *d, const nmpc_opts *o, const nmpc_tuning *t, int nobs, const double *obs, bool obs_in_p, nmpc_handle **out)
+template <bool TRK> static cudaError_t eval_smem_attrs(int sz)
+{
+    cudaError_t e = cudaFuncSetAttribute(eval_kernel<0, TRK>, cudaFuncAttributeMaxDynamicSharedMemorySize, sz);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(eval_kernel<1, TRK>, cudaFuncAttributeMaxDynamicSharedMemorySize, sz);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(eval_kernel<2, TRK>, cudaFuncAttributeMaxDynamicSharedMemorySize, sz);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(eval_kernel<3, TRK>, cudaFuncAttributeMaxDynamicSharedMemorySize, sz);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(eval_kernel<4, TRK>, cudaFuncAttributeMaxDynamicSharedMemorySize, sz);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(eval_kernel<5, TRK>, cudaFuncAttributeMaxDynamicSharedMemorySize, sz);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(eval_kernel<6, TRK>, cudaFuncAttributeMaxDynamicSharedMemorySize, sz);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(eval_kernel<7, TRK>, cudaFuncAttributeMaxDynamicSharedMemorySize, sz);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(eval_kernel<8, TRK>, cudaFuncAttributeMaxDynamicSharedMemorySize, sz);
+    return e;
+}
+
+static int create_impl(const nmpc_desc *d, const nmpc_opts *o, const nmpc_tuning *t, int nobs, const double *obs, bool obs_in_p,
+                       bool tracking, nmpc_handle **out)
 {
     if (!d || !out) return fail(NMPC_EINVAL, "nmpc_create: NULL argument");
     if (d->N < 1 || !(d->T > 0)) return fail(NMPC_EINVAL, "nmpc_create: need N >= 1 and T > 0");
@@ -274,9 +297,10 @@ static int create_impl(const nmpc_desc *d, const nmpc_opts *o, const nmpc_tuning
     if (o) h->o = *o; else nmpc_default_opts(&h->o);
     if (t) h->tune = *t; else nmpc_default_tuning(&h->tune);
     h->ns = 3 * d->Nr; h->nc = 2 * d->Nr; h->M = d->Nr * (d->Nr - 1) / 2; h->S = d->N + 1;
-    h->nobs = nobs; h->family = nobs > 0 ? 1 : 0; h->d_obs = nullptr; h->obs_in_p = obs_in_p;
-    // p = [x0bar; xs], then with the obstacles in p one [nobs][3] table per stage k = 0..N-1
-    h->n = h->ns * h->S + h->nc * d->N; h->np = 2 * h->ns + (obs_in_p ? 3 * d->N * nobs : 0);
+    h->nobs = nobs; h->family = nobs > 0 ? 1 : 0; h->d_obs = nullptr; h->obs_in_p = obs_in_p; h->tracking = tracking;
+    // p = [x0bar; xs], then with the obstacles in p one [nobs][3] table per stage k = 0..N-1; tracking: p = [x0bar; Z[N][5 Nr]]
+    h->n = h->ns * h->S + h->nc * d->N;
+    h->np = tracking ? h->ns + d->N * (h->ns + h->nc) : 2 * h->ns + (obs_in_p ? 3 * d->N * nobs : 0);
     // row layout: family 0 = (N+1) blocks of [ns equality rows ; M pair rows]; family 1 (static obstacles) = ns rows, then N
     // blocks of [ns ; M + Nr n_obs]   (first_scenario_mpc_obstacle_avoidance.py:109-125)
     h->mg = h->family ? h->ns + d->N * (h->ns + h->M + d->Nr * nobs) : h->S * (h->ns + h->M);
@@ -311,8 +335,18 @@ static int create_impl(const nmpc_desc *d, const nmpc_opts *o, const nmpc_tuning
     h->tb.jac_init = h->tb.jac_ps + (size_t)N * M * 4;
     h->tb.hes_rs = h->d_tables + h->nnzj;
     h->tb.hes_ps = h->tb.hes_rs + (size_t)N * Nr * 6;
-    switch (h->block_path ? 0 : (h->family ? 100 + Nr : Nr)) {
+    switch (h->block_path ? 0 : (h->family ? 100 + Nr : (tracking ? 200 + Nr : Nr))) {
 #ifndef NMPC_DEV_ONLY_NR
+        case 201: h->ws_doubles_per_slot = slot_doubles<1, false, true>(N); e = config_solve<1, false, true>(h); break;
+        case 202: h->ws_doubles_per_slot = slot_doubles<2, false, true>(N); e = config_solve<2, false, true>(h); break;
+        case 203: h->ws_doubles_per_slot = slot_doubles<3, false, true>(N); e = config_solve<3, false, true>(h); break;
+        case 204: h->ws_doubles_per_slot = slot_doubles<4, false, true>(N); e = config_solve<4, false, true>(h); break;
+        case 205: h->ws_doubles_per_slot = slot_doubles<5, false, true>(N); e = config_solve<5, false, true>(h); break;
+        case 206: h->ws_doubles_per_slot = slot_doubles<6, false, true>(N); e = config_solve<6, false, true>(h); break;
+        case 207: h->ws_doubles_per_slot = slot_doubles<7, false, true>(N); e = config_solve<7, false, true>(h); break;
+        case 208: h->ws_doubles_per_slot = slot_doubles<8, false, true>(N); e = config_solve<8, false, true>(h); break;
+        case 209: h->ws_doubles_per_slot = slot_doubles<9, false, true>(N); e = config_solve<9, false, true>(h); break;
+        case 210: h->ws_doubles_per_slot = slot_doubles<10, false, true>(N); e = config_solve<10, false, true>(h); break;
         case 101: h->ws_doubles_per_slot = slot_doubles<1, true>(N); e = config_solve<1, true>(h); break;
         case 102: h->ws_doubles_per_slot = slot_doubles<2, true>(N); e = config_solve<2, true>(h); break;
         case 103: h->ws_doubles_per_slot = slot_doubles<3, true>(N); e = config_solve<3, true>(h); break;
@@ -361,20 +395,10 @@ static int create_impl(const nmpc_desc *d, const nmpc_opts *o, const nmpc_tuning
         if (e == cudaSuccess) e = cudaMemcpy(h->d_obs, obs, (size_t)3 * h->nobs * sizeof(double), cudaMemcpyHostToDevice);
     }
     if (e != cudaSuccess) { nmpc_destroy(h); return fail(NMPC_ECUDA, "nmpc_create: kernel configuration failed: %s", cudaGetErrorString(e)); }
-    h->eval_smem = (size_t)(2 * h->n + 2 * h->mg + 2 * h->ns + h->nnzj + h->nnzh + 32 + 8) * sizeof(double);
+    // the record stages all of p: 2 ns values, or a tracking handle's ns + N nz
+    h->eval_smem = (size_t)(2 * h->n + 2 * h->mg + h->np + h->nnzj + h->nnzh + 32 + 8) * sizeof(double);
     if (h->eval_smem > (size_t)220 * 1024 || h->family != 0) h->eval_ok = false;   // large swarms: the stand-alone evaluation record exceeds shared memory
-    else {
-        const int sz = (int)h->eval_smem;
-        e = cudaFuncSetAttribute(eval_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, sz);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(eval_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, sz);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(eval_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, sz);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(eval_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, sz);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(eval_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, sz);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(eval_kernel<5>, cudaFuncAttributeMaxDynamicSharedMemorySize, sz);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(eval_kernel<6>, cudaFuncAttributeMaxDynamicSharedMemorySize, sz);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(eval_kernel<7>, cudaFuncAttributeMaxDynamicSharedMemorySize, sz);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(eval_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, sz);
-    }
+    else e = tracking ? eval_smem_attrs<true>((int)h->eval_smem) : eval_smem_attrs<false>((int)h->eval_smem);
     if (e != cudaSuccess) { const size_t es = h->eval_smem; nmpc_destroy(h); return fail(NMPC_ENOTSUP, "nmpc_create: eval record (%zu B) exceeds shared memory: %s", es, cudaGetErrorString(e)); }
     *out = h;
     return 0;
@@ -474,8 +498,18 @@ static int solve_impl(nmpc_handle *h, int B, const double *x0, const double *p, 
     if (thr && h->family == 2) solve_kernel_small_ocp<VanDerPol><<<grid, 64, 0, st>>>(P);
     else if (thr) solve_kernel_small_ocp<UnicycleObstacles><<<grid, 64, 0, st>>>(P);
     else if (h->block_path) solve_kernel_block<<<grid, h->threads, h->solve_smem, st>>>(P);
-    else switch (h->family ? 100 + h->d.Nr : h->d.Nr) {
+    else switch (h->family ? 100 + h->d.Nr : (h->tracking ? 200 + h->d.Nr : h->d.Nr)) {
 #ifndef NMPC_DEV_ONLY_NR
+        case 201: solve_kernel<1, false, true><<<grid, h->threads, h->solve_smem, st>>>(P); break;
+        case 202: solve_kernel<2, false, true><<<grid, h->threads, h->solve_smem, st>>>(P); break;
+        case 203: solve_kernel<3, false, true><<<grid, h->threads, h->solve_smem, st>>>(P); break;
+        case 204: solve_kernel<4, false, true><<<grid, h->threads, h->solve_smem, st>>>(P); break;
+        case 205: solve_kernel<5, false, true><<<grid, h->threads, h->solve_smem, st>>>(P); break;
+        case 206: solve_kernel<6, false, true><<<grid, h->threads, h->solve_smem, st>>>(P); break;
+        case 207: solve_kernel<7, false, true><<<grid, h->threads, h->solve_smem, st>>>(P); break;
+        case 208: solve_kernel<8, false, true><<<grid, h->threads, h->solve_smem, st>>>(P); break;
+        case 209: solve_kernel<9, false, true><<<grid, h->threads, h->solve_smem, st>>>(P); break;
+        case 210: solve_kernel<10, false, true><<<grid, h->threads, h->solve_smem, st>>>(P); break;
         case 101: solve_kernel<1, true><<<grid, h->threads, h->solve_smem, st>>>(P); break;
         case 102: solve_kernel<2, true><<<grid, h->threads, h->solve_smem, st>>>(P); break;
         case 103: solve_kernel<3, true><<<grid, h->threads, h->solve_smem, st>>>(P); break;
@@ -614,7 +648,8 @@ extern "C" int nmpc_eval(nmpc_handle *h, int B, const double *w, const double *p
     if (h->family) return fail(NMPC_ENOTSUP, "nmpc_eval: not available for this problem family");
     if (!h->eval_ok) {   // record larger than shared memory: global-memory variant
         eval_kernel_big<<<std::min(B, h->sm_count * 8), 256, 0, (cudaStream_t)stream>>>(h->d.Nr, h->d.N, h->d.T, h->d.Q[0], h->d.Q[1], h->d.Q[2],
-                                                                                        h->d.R[0], h->d.R[1], B, w, p, lam_g, f, grad, g, jac, hess, h->tb);
+                                                                                        h->d.R[0], h->d.R[1], B, w, p, lam_g, f, grad, g, jac, hess, h->tb,
+                                                                                        h->np, h->tracking ? h->ns + h->nc : 0);
         h->launches++;
         CUDA_OK(cudaGetLastError());
         return 0;
@@ -623,8 +658,14 @@ extern "C" int nmpc_eval(nmpc_handle *h, int B, const double *w, const double *p
     int blocks = std::min(B, h->sm_count * per_sm);
     const int pf = (std::max(h->n, h->mg) + 255) / 256;
 #define EVAL_LAUNCH(PFV)                                                                                                          \
-    eval_kernel<PFV><<<blocks, 256, h->eval_smem, (cudaStream_t)stream>>>(h->d.Nr, h->d.N, h->d.T, h->d.Q[0], h->d.Q[1], h->d.Q[2], \
-                                                                            h->d.R[0], h->d.R[1], B, w, p, lam_g, f, grad, g, jac, hess, h->tb)
+    do {                                                                                                                          \
+        if (h->tracking)                                                                                                          \
+            eval_kernel<PFV, true><<<blocks, 256, h->eval_smem, (cudaStream_t)stream>>>(h->d.Nr, h->d.N, h->d.T, h->d.Q[0], h->d.Q[1], \
+                h->d.Q[2], h->d.R[0], h->d.R[1], B, w, p, lam_g, f, grad, g, jac, hess, h->tb);                                    \
+        else                                                                                                                      \
+            eval_kernel<PFV, false><<<blocks, 256, h->eval_smem, (cudaStream_t)stream>>>(h->d.Nr, h->d.N, h->d.T, h->d.Q[0], h->d.Q[1], \
+                h->d.Q[2], h->d.R[0], h->d.R[1], B, w, p, lam_g, f, grad, g, jac, hess, h->tb);                                    \
+    } while (0)
     switch (pf <= 8 ? pf : 0) {
         case 1: EVAL_LAUNCH(1); break; case 2: EVAL_LAUNCH(2); break; case 3: EVAL_LAUNCH(3); break; case 4: EVAL_LAUNCH(4); break;
         case 5: EVAL_LAUNCH(5); break; case 6: EVAL_LAUNCH(6); break; case 7: EVAL_LAUNCH(7); break; case 8: EVAL_LAUNCH(8); break;

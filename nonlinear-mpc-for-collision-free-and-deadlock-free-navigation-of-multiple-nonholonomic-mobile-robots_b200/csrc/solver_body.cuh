@@ -17,6 +17,7 @@
 // The file is written against the small `wp::` interface (warp_prims.cuh) so that the tests can
 // step the same source through a CPU fibre emulation of a warp (tests/emul/).
 #pragma once
+#include <type_traits>
 #include "nmpc_internal.h"
 #include "ipm_driver.cuh"
 
@@ -49,7 +50,7 @@
     auto brow = [=](int x, int k) -> const double * { return br + ((long long)k * NMPC_BR_COUNT + x) * LW; }; \
     (void)brow;                                                                                        \
     auto zvalid = [=](int k) -> bool { return l < (k < N ? NZ : NS); };                                \
-    auto gradf = [=](int k, double z) -> double { return (k < N && isz) ? qw * (z - xs_l) : 0.0; };    \
+    auto gradf = [=](int k, double z, double xr) -> double { return (k < N && isz) ? qw * (z - xr) : 0.0; }; \
     (void)row; (void)frow; (void)zvalid; (void)gradf;
 
 struct alignas(16) NmpcD2 { double x, y; };   // one 128-bit shared-memory load
@@ -63,7 +64,11 @@ struct alignas(16) NmpcD2 { double x, y; };   // one 128-bit shared-memory load
 
 // OBS: the static-obstacle family (obstacle rows after the pair rows).  A separate instantiation: the generalised row geometry and
 // the wider addend tables cost the pair-only benchmark path 8 % when they are merely switched off at run time (measured).
-template <int NR, bool OBS = false>
+// TRK: trajectory tracking (nmpc_create_tracking), the centralized family with a per-stage reference Z[k] = [xr_k; ur_k] in p
+// (p = [x0bar; Z[0..N-1]]) instead of one setpoint xs.  The reference is copied once per solve into row R_REF of each stage record
+// (lane l: Z[k][l], lanes >= NZ and record N: 0), where the passes load it with the rows they already stage; the instantiations
+// without TRK keep the setpoint in a register (xs_l) and have no R_REF row.
+template <int NR, bool OBS = false, bool TRK = false>
 struct WarpSolver {
     static constexpr int NS = 3 * NR, NC = 2 * NR, NZ = 5 * NR, M = NR * (NR - 1) / 2;
     static constexpr int LIN = NZ, NM = NZ + 1;
@@ -79,25 +84,29 @@ struct WarpSolver {
     // Scratch layout: one RECORD of R_COUNT rows (LW doubles each) per stage, records consecutive in memory.  The rows are ordered
     // so that what a pass stages for one stage is two contiguous ranges: rows indexed by the stage k (from record k) and rows indexed
     // by the block k + 1 (from record k + 1):
-    //     factorisation:  record k  [R_TRIG2 .. R_ZU]                record k + 1  [R_YC .. R_VU]
+    //     factorisation:  record k  [R_REF .. R_ZU]                  record k + 1  [R_YC .. R_VU]
     //     forward pass:   record k  [R_Z .. R_F0 + NS - 1]           record k + 1  [R_S .. R_DQ]
     // (round 1 kept one array per row, [row][stage][LW]: the 16 rows a stage needs were 16 separate 256-byte pieces 5 KB apart).
     // The (relaxed) bound rows are laid out the same way by prep_bounds_kernel ([stage][BL, BU, CE, DL, DU][LW]); they are shared by the
     // batch unless bounds_batched and stay L2 resident (copying them into every instance's records cost 10 MB of DRAM traffic per solve).
     enum Row {
-        R_TRIG2, R_TRIG, R_Z, R_ZL, R_ZU, R_LIN, R_DG, R_GX, R_COEF, R_F0,          // R_F0 .. R_F0 + NS - 1: Riccati factor rows
+        R_REF, R_TRIG2 = R_REF + (TRK ? 1 : 0),
+        R_TRIG, R_Z, R_ZL, R_ZU, R_LIN, R_DG, R_GX, R_COEF, R_F0,                  // R_F0 .. R_F0 + NS - 1: Riccati factor rows
         R_YC = R_F0 + NS, R_YD, R_CSOC, R_DSOC, R_S, R_VL, R_VU, R_RC, R_GS, R_GXQ, R_GYQ, R_RD, R_DQ,
         R_DZ, R_DZ2, R_YTC, R_YTC2, R_DS, R_DS2, R_YTD, R_YTD2,
         R_COUNT
     };
-    // slots of the factorisation's staging buffer (sm + SM_STG): rows [R_TRIG2 .. R_ZU] of record k, bound rows [BL, BU] of stage k,
-    // rows [R_YC .. R_VU] of record k + 1, bound rows [CE, DL, DU] of block k + 1
-    enum { FS_TRIG2, FS_TRIG, FS_Z, FS_ZL, FS_ZU, FS_BL, FS_BU, FS_YC, FS_YD, FS_CSOC, FS_DSOC, FS_S, FS_VL, FS_VU, FS_CE, FS_DL, FS_DU, FS_COUNT };
+    // slots of the factorisation's staging buffer (sm + SM_STG): rows [R_REF .. R_ZU] of record k, bound rows [BL, BU] of stage k,
+    // rows [R_YC .. R_VU] of record k + 1, bound rows [CE, DL, DU] of block k + 1  (R_REF / FS_REF: TRK only, else an alias of
+    // R_TRIG2 / FS_TRIG2)
+    enum { FS_REF, FS_TRIG2 = FS_REF + (TRK ? 1 : 0),
+           FS_TRIG, FS_Z, FS_ZL, FS_ZU, FS_BL, FS_BU, FS_YC, FS_YD, FS_CSOC, FS_DSOC, FS_S, FS_VL, FS_VU, FS_CE, FS_DL, FS_DU, FS_COUNT };
     // slots of the forward pass's staging buffer (the whole big region): rows [R_Z .. last factor row] of record k, [BL, BU] of stage k,
     // rows [R_S .. R_DQ] of record k + 1, [DL, DU] of block k + 1
     enum { WS_Z, WS_ZL, WS_ZU, WS_LIN, WS_DG, WS_GX, WS_COEF, WS_F0, WS_BL = WS_F0 + NS, WS_BU,
            WS_S, WS_VL, WS_VU, WS_RC, WS_GS, WS_GXQ, WS_GYQ, WS_RD, WS_DQ, WS_DL, WS_DU, WS_COUNT };
-    static_assert(R_ZU - R_TRIG2 == FS_ZU - FS_TRIG2 && R_VU - R_YC == FS_VU - FS_YC && R_F0 + NS - 1 - R_Z == WS_F0 + NS - 1 - WS_Z &&
+    static_assert(R_ZU - R_REF == FS_ZU - FS_REF && R_TRIG2 - R_REF == FS_TRIG2 - FS_REF && R_VU - R_YC == FS_VU - FS_YC &&
+                  R_F0 + NS - 1 - R_Z == WS_F0 + NS - 1 - WS_Z &&
                   R_DQ - R_S == WS_DQ - WS_S && NMPC_BR_BU == NMPC_BR_BL + 1 && NMPC_BR_DL == NMPC_BR_CE + 1 && NMPC_BR_DU == NMPC_BR_DL + 1,
                   "staging slots follow the record layouts");
     // shared-memory carve-up (doubles, per team): small buffers that live for the whole solve, then one big region that the
@@ -235,13 +244,13 @@ struct WarpSolver {
                 for (int b = a + 1; b < NR; b++) { if (q == l) { pi = a; pj = b; } q++; }
         }
         br = P.brows + (long long)inst * P.bstride;
-        const double *pp = P.p + (long long)inst * (OBS ? P.np : 2 * NS);
+        const double *pp = P.p + (long long)inst * ((OBS || TRK) ? P.np : 2 * NS);
         if (OBS) {   // obstacles in p: [N][nobs][3] after x0bar and xs, one table per stage; else the handle's table at every stage
             qtab = P.obs_in_p ? pp + 2 * NS : P.obs; qos = P.obs_in_p ? 3 * nobs : 0;
             if (isobs) qob = qtab + 3 * ((l - M) % nobs);
         }
         x0bar_l = isx ? pp[l] : 0.0;
-        xs_l = isx ? pp[NS + l] : 0.0;
+        xs_l = (isx && !TRK) ? pp[NS + l] : 0.0;   // TRK: the reference is in the R_REF rows (init_point)
         qw = isx ? 2.0 * P.Q[comp] : (isu ? 2.0 * P.R[comp] : 0.0);
         df = 1.0; fn = 0;
         n_reg = n_resto = n_soc = n_fact = n_ls = 0;
@@ -249,7 +258,8 @@ struct WarpSolver {
         tsync();
     }
 
-    NMPC_DEV double gradf(int k, double z) const { return (k < N && isz) ? qw * (z - xs_l) : 0.0; }
+    // gradient of the stage cost of variable l at stage k; xr: its reference (xs_l, or row R_REF of record k with TRK)
+    NMPC_DEV double gradf(int k, double z, double xr) const { return (k < N && isz) ? qw * (z - xr) : 0.0; }
 
     static NMPC_DEV double push_in(double x, double lo, double hi, double k1, double k2)
     {
@@ -270,9 +280,12 @@ struct WarpSolver {
         const double *x0 = P.x0 + (long long)inst * (NS * S + NC * N);
         const nmpc_opts &o = P.o;
         double gmax = 0.0;
+        const double *zref = TRK ? P.p + (long long)inst * P.np + NS : nullptr;   // Z[0] of this instance
         for (int k = 0; k <= N; k++) {
             double z = isx ? x0[k * NS + l] : ((isu && k < N) ? x0[NS * S + k * NC + (l - NS)] : 0.0);
-            gmax = fmax(gmax, fabs(gradf(k, z)));
+            double xr = xs_l;
+            if (TRK) { xr = (k < N && isz) ? zref[(long long)k * NZ + l] : 0.0; row(R_REF, k)[l] = xr; }
+            gmax = fmax(gmax, fabs(gradf(k, z, xr)));
             row(R_Z, k)[l] = z;
         }
         gmax = tred_max(gmax);
@@ -336,7 +349,11 @@ struct WarpSolver {
 
     // Rows of one stage / inequality block, loaded one stage ahead of their use (register software pipeline:
     // the loads of stage k+1 are in flight while stage k is processed, so HBM latency is paid once per pass).
-    struct ZRows { double z, dz, lo, hi, zl, zu, yc, ce, csoc, cs, sn; };
+    struct ZRowsB { double z, dz, lo, hi, zl, zu, yc, ce, csoc, cs, sn; };
+    struct ZRowsR : ZRowsB { double ref; };   // TRK: with the reference row (a member the other instantiations do not carry)
+    typedef typename std::conditional<TRK, ZRowsR, ZRowsB>::type ZRows;
+    static NMPC_DEV double zref(const ZRowsR &r) { return r.ref; }
+    static NMPC_DEV double zref(const ZRowsB &) { return 0.0; }
     struct QRows { double s, ds, lo, hi, yd, vl, vu, dsoc; };
 
     // FULL (dual / complementarity terms as well) is a run-time flag: one copy of this pass serves the iterate and the
@@ -369,6 +386,7 @@ struct WarpSolver {
             r.lo = brow(NMPC_BR_BL, k)[l]; r.hi = brow(NMPC_BR_BU, k)[l]; r.ce = brow(NMPC_BR_CE, k)[l];
             r.zl = FULL ? row(R_ZL, k)[l] : 0.0; r.zu = FULL ? row(R_ZU, k)[l] : 0.0; r.yc = FULL ? row(R_YC, k)[l] : 0.0;
             r.csoc = socacc ? row(R_CSOC, k)[l] : 0.0;
+            if constexpr (TRK) r.ref = row(R_REF, k)[l];
             return r;
         };
         auto load_q = [&](int b) {
@@ -441,10 +459,11 @@ struct WarpSolver {
                 if (hu) addlog(hi - zk);
                 if (hl && !hu) sdamp += zk - lo;
                 if (hu && !hl) sdamp += hi - zk;
-                if (k < N) { double e = zk - xs_l; fo += 0.5 * qw * e * e; }
+                const double xr = TRK ? zref(zc) : xs_l;
+                if (k < N) { double e = zk - xr; fo += 0.5 * qw * e * e; }
                 if (FULL) {
                     const double zl = zc.zl, zu = zc.zu;
-                    double r = df * gradf(k, zk) - zl + zu;
+                    double r = df * gradf(k, zk, xr) - zl + zu;
                     if (hl && !hu) r += kd * mu;
                     if (hu && !hl) r -= kd * mu;
                     if (isx) r += zc.yc;
@@ -613,7 +632,7 @@ struct WarpSolver {
             if (l == 0) {
                 wp::fence_proxy_async();
                 wp::bulk_expect(bar, (unsigned)(FS_COUNT * LW * sizeof(double)));
-                bulk_rows(bar, stg + FS_TRIG2 * LW, row(R_TRIG2, k), FS_BL - FS_TRIG2);
+                bulk_rows(bar, stg + FS_REF * LW, row(R_REF, k), FS_BL - FS_REF);
                 bulk_rows(bar, stg + FS_BL * LW, brow(NMPC_BR_BL, k), 2);
                 bulk_rows(bar, stg + FS_YC * LW, row(R_YC, k + 1), FS_CE - FS_YC);
                 bulk_rows(bar, stg + FS_CE * LW, brow(NMPC_BR_CE, k + 1), 3);
@@ -719,7 +738,8 @@ struct WarpSolver {
             // stage gradient h_l (variable l) and diagonal curvature
             double sig = 0.0, gx = 0.0, dg = 0.0;
             if (isz) {
-                sig_g<MODE>(kd, zk, stg[FS_BL * LW + l], stg[FS_BU * LW + l], stg[FS_ZL * LW + l], stg[FS_ZU * LW + l], mu, df * gradf(k, zk), sig, gx);
+                sig_g<MODE>(kd, zk, stg[FS_BL * LW + l], stg[FS_BU * LW + l], stg[FS_ZL * LW + l], stg[FS_ZU * LW + l], mu,
+                            df * gradf(k, zk, TRK ? stg[FS_REF * LW + l] : xs_l), sig, gx);
                 dg = sig + delta + zeta;
                 if (MODE == 0) { dg += df * qw; if (isx && comp == 2) dg += thd[rob]; }
             }
@@ -1162,7 +1182,7 @@ struct WarpSolver {
                 long long idx = isx ? (long long)k * NS + l : (long long)NS * S + (long long)k * NC + (l - NS);
                 x[idx] = zk;
                 if (lx) lx[idx] = (row(R_ZU, k)[l] - row(R_ZL, k)[l]) / df;
-                if (k < N) { double e = zk - xs_l; fo += 0.5 * qw * e * e; }
+                if (k < N) { double e = zk - (TRK ? row(R_REF, k)[l] : xs_l); fo += 0.5 * qw * e * e; }
             }
             tsync();
             if (k < N && l < NR) { double s_, c_; wp::sincos_(zb[3 * l + 2], &s_, &c_); cs[l] = c_; sn[l] = s_; }

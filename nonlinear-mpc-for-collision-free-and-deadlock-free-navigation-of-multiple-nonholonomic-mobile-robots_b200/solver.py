@@ -97,14 +97,19 @@ def _flat(a, size, name):
 class Problem:
     """Handle on the CUDA library for one (Nr, N, T, Q, R) problem family."""
 
-    def __init__(self, Nr, N, T, Q=(1.0, 5.0, 0.1), R=(0.5, 0.05), obstacles=None, tuning=None, moving_obstacles=None, **opts):
+    def __init__(self, Nr, N, T, Q=(1.0, 5.0, 0.1), R=(0.5, 0.05), obstacles=None, tuning=None, moving_obstacles=None,
+                 tracking=False, **opts):
         """obstacles: optional [n_obs, 3] array of static circular obstacles (centre x, y, clearance = rob_dim + r_obs): the
         reference's obstacle-avoidance family (first_scenario_mpc_obstacle_avoidance.py:96-152), see nmpc_create_obstacles.
         moving_obstacles: n_obs instead of `obstacles` -> the same family with the obstacles in p, one [n_obs, 3] table per
         instance and stage (p = [x0bar; xs; O[N][n_obs][3]], see nmpc_create_moving_obstacles and params()).
+        tracking: True -> the centralized family tracking a per-instance, per-stage state and control reference instead of one
+        goal (p = [x0bar; Z[N][5Nr]], Z[k] = [xr_k; ur_k], see nmpc_create_tracking and params()); no obstacles.
         tuning: optional dict of nmpc_tuning fields (convoy, ctas_per_sm, force_block_path, thread_min_batch)."""
         if obstacles is not None and moving_obstacles is not None:
             raise ValueError("obstacles= and moving_obstacles= are mutually exclusive")
+        if tracking and (obstacles is not None or moving_obstacles is not None):
+            raise ValueError("tracking=True cannot be combined with obstacles= or moving_obstacles=")
         self.L = lib()
         self.desc = Desc(int(Nr), int(N), float(T), (C.c_double * 3)(*[float(q) for q in Q]),
                          (C.c_double * 2)(*[float(r) for r in R]))
@@ -113,7 +118,11 @@ class Problem:
         self.obstacles = None if obstacles is None else np.ascontiguousarray(np.asarray(obstacles, dtype=np.float64).reshape(-1, 3))
         self.tuning = default_tuning(**(tuning or {}))
         self.moving = moving_obstacles is not None
-        if self.moving:
+        self.tracking = bool(tracking)
+        if self.tracking:
+            check(self.L.nmpc_create_tracking(C.byref(self.desc), C.byref(self.opts), C.byref(self.tuning), C.byref(self.h)))
+            self.nobs = 0
+        elif self.moving:
             check(self.L.nmpc_create_moving_obstacles(C.byref(self.desc), C.byref(self.opts), C.byref(self.tuning),
                                                       int(moving_obstacles), C.byref(self.h)))
             self.nobs = int(moving_obstacles)
@@ -167,10 +176,16 @@ class Problem:
             return np.concatenate([np.tile(x0, self.N + 1), np.zeros(self.nc * self.N)])
         return np.concatenate([np.tile(x0, (1, self.N + 1)), np.zeros((x0.shape[0], self.nc * self.N))], axis=1)
 
-    def params(self, x0bar, xs, obstacles=None):
+    def params(self, x0bar, xs, obstacles=None, uref=None):
         """p [B, np] from x0bar [B, 3Nr], xs [B, 3Nr] and, for moving_obstacles, obstacles [B, N, n_obs, 3] (ox, oy, clearance of
-        every obstacle at every stage).  NumPy arrays give a NumPy array, CUDA tensors a contiguous float64 tensor on their device."""
+        every obstacle at every stage).  For tracking: xs is the state reference [B, N, 3Nr] (or [B, 3Nr], the same at every
+        stage) and uref the control reference [B, N, 2Nr] (default zeros).  NumPy arrays give a NumPy array, CUDA tensors a
+        contiguous float64 tensor on their device."""
         B = x0bar.shape[0]
+        if getattr(self, "tracking", False):
+            return self._tracking_params(x0bar, xs, uref, obstacles)
+        if uref is not None:
+            raise ValueError("uref goes into p only for Problem(tracking=True)")
         if tuple(x0bar.shape) != (B, self.ns) or tuple(xs.shape) != (B, self.ns):
             raise ValueError("x0bar and xs must be [B, %d]" % self.ns)
         parts = [x0bar, xs]
@@ -184,6 +199,24 @@ class Problem:
             return np.ascontiguousarray(np.concatenate([np.asarray(a, np.float64) for a in parts], axis=1))
         torch = self._torch()
         return torch.cat([a.to(torch.float64) for a in parts], dim=1).contiguous()
+
+    def _tracking_params(self, x0bar, xs, uref, obstacles):
+        B, N = x0bar.shape[0], self.N
+        if obstacles is not None:
+            raise ValueError("obstacles go into p only for Problem(moving_obstacles=n_obs)")
+        if tuple(x0bar.shape) != (B, self.ns) or tuple(xs.shape) not in ((B, self.ns), (B, N, self.ns)):
+            raise ValueError("x0bar must be [B, %d] and xs [B, N, %d] or [B, %d]" % (self.ns, self.ns, self.ns))
+        if uref is not None and tuple(uref.shape) != (B, N, self.nc):
+            raise ValueError("uref must be [B, N, 2Nr] = [%d, %d, %d]" % (B, N, self.nc))
+        if isinstance(x0bar, np.ndarray):
+            xr = np.broadcast_to(np.asarray(xs, np.float64).reshape(B, -1, self.ns), (B, N, self.ns))
+            ur = np.zeros((B, N, self.nc)) if uref is None else np.asarray(uref, np.float64)
+            Z = np.concatenate([xr, ur], axis=2).reshape(B, -1)
+            return np.ascontiguousarray(np.concatenate([np.asarray(x0bar, np.float64), Z], axis=1))
+        torch = self._torch()
+        xr = xs.to(torch.float64).reshape(B, -1, self.ns).expand(B, N, self.ns)
+        ur = (torch.zeros((B, N, self.nc), dtype=torch.float64, device=xs.device) if uref is None else uref.to(torch.float64))
+        return torch.cat([x0bar.to(torch.float64), torch.cat([xr, ur], dim=2).reshape(B, -1)], dim=1).contiguous()
 
     def launch_count(self):
         return int(self.L.nmpc_launch_count(self.h))
@@ -320,7 +353,7 @@ class Problem:
         return o
 
 
-def closed_loop(prob, P, lbx, ubx, lbg, ubg, steps, tol=1e-1, dmin=None, obstacles=None):
+def closed_loop(prob, P, lbx, ubx, lbg, ubg, steps, tol=1e-1, dmin=None, obstacles=None, reference=None):
     """Batched closed-loop driver, device resident (SURVEY.md 8f-1): the reference's loop body
     (centralized_six_robots_implementation.py:416-465 with the Euler plant of casadi_test.py:17-26) for B
     independent instances at once.  Per step: solve -> apply u_0 through the plant -> reference shift as the next
@@ -329,10 +362,21 @@ def closed_loop(prob, P, lbx, ubx, lbg, ubg, steps, tol=1e-1, dmin=None, obstacl
     obstacles (Problem(moving_obstacles=n_obs) only): CUDA float64 [steps+N, B, n_obs, 3], the obstacles' positions and
     clearances over time; step t solves with the window t..t+N-1 in p (P then needs only its first 6Nr columns), and the
     result gains min_clearance [B] = min over time, robots and obstacles of rho - clearance between the plant state and the
-    obstacles at the same time."""
+    obstacles at the same time.
+    reference (required by, and only for, Problem(tracking=True)): CUDA float64 [steps+N, B, 5Nr], rows [xr_t; ur_t] of the
+    reference over time; step t solves with rows t..t+N-1 as Z in p (P then needs only its first 3Nr columns, x0bar), there is
+    no stop test (every instance is active at every step), and the result gains track_err [steps+1, B] = the largest xy distance
+    over robots between the plant state and the reference state at the same time."""
     torch = prob._torch()
     B, ns, nc, N = P.shape[0], prob.ns, prob.nc, prob.N
-    if obstacles is not None:
+    tracking = getattr(prob, "tracking", False)
+    if tracking != (reference is not None):
+        raise ValueError("reference= is required by, and only accepted for, a Problem(tracking=True)")
+    if tracking:
+        if not (reference.is_cuda and reference.dtype == torch.float64) or tuple(reference.shape) != (steps + N, B, ns + nc):
+            raise ValueError("reference must be a float64 CUDA tensor [steps + N, B, 5Nr] = [%d, %d, %d]" % (steps + N, B, ns + nc))
+        p = torch.cat([P[:, :ns], torch.empty((B, N * (ns + nc)), dtype=torch.float64, device=P.device)], dim=1)
+    elif obstacles is not None:
         if not getattr(prob, "moving", False):
             raise ValueError("obstacles= needs a Problem(moving_obstacles=n_obs)")
         if not (obstacles.is_cuda and obstacles.dtype == torch.float64) or tuple(obstacles.shape) != (steps + N, B, prob.nobs, 3):
@@ -354,7 +398,11 @@ def closed_loop(prob, P, lbx, ubx, lbg, ubg, steps, tol=1e-1, dmin=None, obstacl
             prob.set_order(None)
         if obstacles is not None:
             p[:, 2 * ns:] = obstacles[t:t + N].permute(1, 0, 2, 3).reshape(B, -1)
-        active = (p[:, :ns] - p[:, ns:2 * ns]).norm(dim=1) > tol
+        if tracking:
+            p[:, ns:] = reference[t:t + N].permute(1, 0, 2).reshape(B, -1)
+            active = torch.ones(B, dtype=torch.bool, device=P.device)
+        else:
+            active = (p[:, :ns] - p[:, ns:2 * ns]).norm(dim=1) > tol
         act[t] = active
         prob.solve(x0, p, lbx, ubx, lbg, ubg, want=(), out=out)
         u0 = out["x"][:, ns * (N + 1):ns * (N + 1) + nc]
@@ -377,6 +425,10 @@ def closed_loop(prob, P, lbx, ubx, lbg, ubg, steps, tol=1e-1, dmin=None, obstacl
         ob = obstacles[:steps + 1]
         rho = (pos[:, :, :, None, :] - ob[:, :, None, :, :2]).norm(dim=-1)
         res["min_clearance"] = (rho - ob[:, :, None, :, 2]).amin(dim=(0, 2, 3))
+    if tracking:
+        pos = traj.reshape(steps + 1, B, prob.Nr, 3)[..., :2]
+        ref = reference[:steps + 1, :, :ns].reshape(steps + 1, B, prob.Nr, 3)[..., :2]
+        res["track_err"] = (pos - ref).norm(dim=-1).amax(dim=2)
     return res
 
 
@@ -438,7 +490,15 @@ class NlpSolver:
             Xk = o["x"][0, :P.ns * (P.N + 1)].reshape(P.N + 1, P.ns)[:P.N]
             Qd = np.tile(np.asarray(list(P.desc.Q), float), P.Nr)
             pv = np.asarray(_flat(p, P.np_, "p"))
-            lam_p[P.ns:2 * P.ns] = -2.0 * Qd * (Xk - pv[P.ns:2 * P.ns][None]).sum(axis=0)
+            if getattr(P, "tracking", False):
+                # Z[k] = [xr_k; ur_k] enters only the cost (X_k - xr_k)'Q(X_k - xr_k) + (U_k - ur_k)'R(U_k - ur_k)
+                Z = pv[P.ns:].reshape(P.N, P.ns + P.nc)
+                Uk = o["x"][0, P.ns * (P.N + 1):].reshape(P.N, P.nc)
+                Rd = np.tile(np.asarray(list(P.desc.R), float), P.Nr)
+                lam_z = np.concatenate([-2.0 * Qd * (Xk - Z[:, :P.ns]), -2.0 * Rd * (Uk - Z[:, P.ns:])], axis=1)
+                lam_p[P.ns:] = lam_z.ravel()
+            else:
+                lam_p[P.ns:2 * P.ns] = -2.0 * Qd * (Xk - pv[P.ns:2 * P.ns][None]).sum(axis=0)
             if getattr(P, "moving", False):
                 # obstacle block O[k][o] = (ox, oy, c): row (k, i, o) = rho - c with rho = |pos_{k,i} - (ox, oy)|, so
                 # dL/d(ox, oy) = -sum_i lam (pos - o) / rho and dL/dc = -sum_i lam
@@ -467,6 +527,7 @@ def nlpsol(name, plugin, nlp, opts=None):
         {'family': 'unicycle_centralized', 'Nr', 'N', 'T', 'Q': (3,), 'R': (2,)}
         {'family': 'unicycle_obstacles', ..., 'obstacles': [[x, y, clearance], ...]}
         {'family': 'unicycle_moving_obstacles', ..., 'n_obs'}: the obstacles in p = [x0bar; xs; O[N][n_obs][3]]
+        {'family': 'unicycle_tracking', 'Nr', 'N', 'T', 'Q', 'R'}: a per-stage reference in p = [x0bar; Z[N][5Nr]]
     `opts` uses the reference's layout: {'print_time': 0, 'ipopt': {'max_iter': 2000, ...}}.
     """
     if plugin not in ("ipopt", "b200ipm"):
@@ -476,9 +537,9 @@ def nlpsol(name, plugin, nlp, opts=None):
         kw = {k: v for k, v in ip.items() if k in _IPOPT_KEYS}
         return NlpSolver(name, SmallOcp("van_der_pol", nlp.get("N", 20), nlp.get("T", 10.0), nlp.get("rk_steps", 4), **kw))
     if not isinstance(nlp, dict) or nlp.get("family", "unicycle_centralized") not in ("unicycle_centralized", "unicycle_obstacles",
-                                                                                   "unicycle_moving_obstacles"):
+                                                                                   "unicycle_moving_obstacles", "unicycle_tracking"):
         raise ValueError("nlp must be a descriptor {'family':'unicycle_centralized'|'unicycle_obstacles'|"
-                         "'unicycle_moving_obstacles','Nr','N','T',...}")
+                         "'unicycle_moving_obstacles'|'unicycle_tracking','Nr','N','T',...}")
     if nlp.get("family") == "unicycle_moving_obstacles" and nlp.get("n_obs") is None:
         raise ValueError("family 'unicycle_moving_obstacles' needs 'n_obs'")
     if nlp.get("family") == "unicycle_obstacles" and nlp.get("obstacles") is None:
@@ -488,5 +549,6 @@ def nlpsol(name, plugin, nlp, opts=None):
     kw = {k: v for k, v in ip.items() if k in _IPOPT_KEYS}          # print_level etc. are accepted and ignored
     prob = Problem(nlp["Nr"], nlp["N"], nlp["T"], nlp.get("Q", (1.0, 5.0, 0.1)), nlp.get("R", (0.5, 0.05)),
                    obstacles=nlp.get("obstacles") if nlp.get("family") == "unicycle_obstacles" else None,
-                   moving_obstacles=nlp.get("n_obs") if nlp.get("family") == "unicycle_moving_obstacles" else None, **kw)
+                   moving_obstacles=nlp.get("n_obs") if nlp.get("family") == "unicycle_moving_obstacles" else None,
+                   tracking=nlp.get("family") == "unicycle_tracking", **kw)
     return NlpSolver(name, prob)
