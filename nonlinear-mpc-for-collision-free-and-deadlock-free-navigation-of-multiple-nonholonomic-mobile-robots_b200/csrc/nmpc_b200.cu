@@ -612,7 +612,11 @@ extern "C" int nmpc_solve_host(nmpc_handle *h, int B, const double *x0, const do
     if (iters) CUDA_OK(cudaMemcpyAsync(iters, b + o_it, (size_t)B * 4, cudaMemcpyDeviceToHost, st));
     if (stats) CUDA_OK(cudaMemcpyAsync(stats, b + o_stats, (size_t)B * NMPC_NSTATS * D, cudaMemcpyDeviceToHost, st));
     CUDA_OK(cudaStreamSynchronize(st));
-    if (stp[0] < 0) return fail(stp[0], "nmpc_solve_host: bounds rejected (%s)", stp[0] == NMPC_EBOUNDS ? "lb > ub" : "fixed variable, non-equality dynamics row or equality distance row");
+    // the warp and block paths reject the whole batch, the thread path only the instance whose bounds are bad: look at all
+    for (int i = 0; i < B; i++)
+        if (stp[i] < 0)
+            return fail(stp[i], "nmpc_solve_host: bounds of instance %d rejected (%s)", i,
+                        stp[i] == NMPC_EBOUNDS ? "lb > ub" : "fixed variable, non-equality dynamics row or equality distance row");
     return 0;
 }
 

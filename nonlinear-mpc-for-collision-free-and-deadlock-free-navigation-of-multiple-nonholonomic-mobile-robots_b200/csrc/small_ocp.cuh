@@ -700,6 +700,15 @@ struct ThreadSolver {
                 if (P.lam_x) P.lam_x[inst * n + Model::xidx(ctx, k, l)] = valid(k, l) ? (row(R_ZU, k)[l] - row(R_ZL, k)[l]) / df : 0.0;
             }
         for (int k = 0; k < N; k++) { model(k, row(R_Z, k)); fo += cst(k)[C_Q]; }
+        // A fixed initial state is a parameter (IPOPT's make_parameter): its bound multiplier is -(grad f + J' lam_g), the
+        // cost's sensitivity to X_0, so that grad f + J' lam_g + lam_x = 0 holds in every component.
+        if (P.lam_x && fixed0)
+            for (int l = 0; l < NX; l++) {
+                double r = df * cst(0)[C_GQ + l];
+                for (int i = 0; i < NX; i++) r += cst(0)[C_J + i * NZ + l] * row(R_YC, 1)[i];
+                for (int i = 0; i < ni; i++) r += cin(0, i)[1 + l] * row(R_YD, 0)[i];
+                P.lam_x[inst * n + Model::xidx(ctx, 0, l)] = -r / df;
+            }
         for (int k = kfirst(); k <= N; k++)
             for (int i = 0; i < NX; i++) {
                 const long long r = inst * mg + Model::grow_eq(ctx, k, i);

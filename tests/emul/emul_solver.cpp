@@ -78,6 +78,7 @@ extern "C" int emu_solve(const nmpc_desc *d, const nmpc_opts *o, int B, const do
     P.o = *o; P.x0 = x0; P.p = p; P.brows = brows.data(); P.bstride = bounds_batched ? bstride : 0;
     P.bound_err = &berr; P.x = x; P.f = f; P.g = g; P.lam_x = lam_x; P.lam_g = lam_g; P.status = status; P.iters = iters;
     P.stats = stats; P.trace = trace; P.max_trace = max_trace; P.ws = ws.data(); P.ws_stride = wsd;
+    P.np = 6 * Nr;      // p = [x0bar; xs] per instance (the obstacle instantiation strides p by P.np, as nmpc_solve sets it)
     P.nobs = nobs; P.family = family; P.obs = obs;
     const size_t STK = 512 * 1024;
     std::vector<char> stacks(64 * STK);
