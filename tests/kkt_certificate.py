@@ -79,8 +79,9 @@ def _one_sided(v, lam, lo, hi, relax):
     return compl, viol, wrong
 
 
-def measure(nlp, x, lam_x, lam_g, p, lbx, ubx, lbg, ubg, df, relax=1e-8):
-    """The certificate's quantities (unscaled unless named *_scaled)."""
+def measure(nlp, x, lam_x, lam_g, p, lbx, ubx, lbg, ubg, df, relax=1e-8, feas=None):
+    """The certificate's quantities (unscaled unless named *_scaled).  feas: the tolerance of the constraint rows' feasibility
+    (default relax); a solver stops with |g - s| <= tol, so with bound_relax_factor < tol a row may miss its bound by tol."""
     x, lam_x, lam_g = (np.asarray(a, float).reshape(-1) for a in (x, lam_x, lam_g))
     lbx, ubx, lbg, ubg = (np.asarray(a, float).reshape(-1) for a in (lbx, ubx, lbg, ubg))
     grad, g, J = derivatives(nlp, x, p)
@@ -91,6 +92,8 @@ def measure(nlp, x, lam_x, lam_g, p, lbx, ubx, lbg, ubg, df, relax=1e-8):
     ineq = rows & (lbg != ubg)
     cx, vx, wx = _one_sided(x, lam_x, lbx, ubx, relax)
     cg, vg, wg = _one_sided(g[~dummy], lam_g[~dummy], lbg[~dummy], ubg[~dummy], relax)
+    if feas is not None:
+        vg = _one_sided(g[~dummy], lam_g[~dummy], lbg[~dummy], ubg[~dummy], feas)[1]
     # IPOPT's scaling of the dual infeasibility and of the complementarity (ipm_driver.cuh), from the scaled multipliers
     nzb = np.isfinite(lbx).sum() + np.isfinite(ubx).sum() + np.isfinite(lbg[ineq]).sum() + np.isfinite(ubg[ineq]).sum()
     ysum = df * np.abs(lam_g[rows]).sum()
@@ -106,9 +109,9 @@ def measure(nlp, x, lam_x, lam_g, p, lbx, ubx, lbg, ubg, df, relax=1e-8):
                 scaled_err=max(df * stat_inf / s_d, pinf, df * compl / s_c))
 
 
-def certify(nlp, x, lam_x, lam_g, p, lbx, ubx, lbg, ubg, df, relax=1e-8, tol=1e-8):
+def certify(nlp, x, lam_x, lam_g, p, lbx, ubx, lbg, ubg, df, relax=1e-8, tol=1e-8, feas=None):
     """Assert that (x, lam_x, lam_g) is a KKT point of the NLP at tolerance tol; return the measured quantities."""
-    m = measure(nlp, x, lam_x, lam_g, p, lbx, ubx, lbg, ubg, df, relax)
+    m = measure(nlp, x, lam_x, lam_g, p, lbx, ubx, lbg, ubg, df, relax, feas)
     stat_tol = 2 * tol * m["s_d"] / df + 1e-11 * (1.0 + m["grad"])
     sign_tol = 10 * tol / df
     compl_tol = max(1e-7, 2 * tol * m["s_c"] / df)
