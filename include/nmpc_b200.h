@@ -97,7 +97,8 @@ void nmpc_destroy(nmpc_handle *h);
  *   ctas_per_sm       > 0: cap on resident CTAs per SM (occupancy experiments); 0 = as many as fit
  *   force_block_path  != 0: run any Nr on the CTA-per-instance dense-block solver (test hook)
  *   thread_min_batch  > 0: batches at least this large of the one-robot static-obstacle family use the thread-per-instance
- *                     solver; 0 = never.  Ignored by nmpc_create_moving_obstacles (that solver takes one static table) */
+ *                     solver; 0 = never.  Ignored by nmpc_create_moving_obstacles and nmpc_create_tracking_obstacles (that
+ *                     solver takes one static table) */
 typedef struct nmpc_tuning { int convoy, ctas_per_sm, force_block_path, thread_min_batch; } nmpc_tuning;
 void nmpc_default_tuning(nmpc_tuning *t);
 /* nmpc_create / nmpc_create_obstacles (n_obs > 0) with explicit tuning; t == NULL means the defaults. */
@@ -105,7 +106,7 @@ int nmpc_create_tuned(const nmpc_desc *d, const nmpc_opts *o, const nmpc_tuning 
 
 int nmpc_n(const nmpc_handle *h);        /* decision variables                         */
 int nmpc_mg(const nmpc_handle *h);       /* constraint rows                            */
-int nmpc_np(const nmpc_handle *h);       /* parameters (6 Nr; + 3 N n_obs with obstacles in p; 3 Nr + 5 Nr N tracking) */
+int nmpc_np(const nmpc_handle *h);       /* parameters (6 Nr, or 3 Nr + 5 Nr N tracking; + 3 N n_obs with obstacles in p) */
 int nmpc_nnz_jac(const nmpc_handle *h);  /* 3Nr + N(11Nr+4M)   CasADi's CCS of dg/dw   */
 int nmpc_nnz_hess(const nmpc_handle *h); /* N(6Nr+2M)          lower triangle          */
 
@@ -161,6 +162,21 @@ int nmpc_create_moving_obstacles(const nmpc_desc *d, const nmpc_opts *o, const n
  * nmpc_eval works on the handle with p [B, nmpc_np]: its gradient includes both references, its Jacobian and Hessian are
  * those of nmpc_create. */
 int nmpc_create_tracking(const nmpc_desc *d, const nmpc_opts *o, const nmpc_tuning *t, nmpc_handle **out);
+
+/* Trajectory tracking among obstacles: the moving-obstacle family (nmpc_create_moving_obstacles) with the per-stage reference of
+ * nmpc_create_tracking in place of the goal xs, e.g. a planner's path with feed-forward controls, tracked while the collision and
+ * obstacle rows stay hard constraints.
+ *     p = [x0bar (3 Nr); Z[0]; ...; Z[N-1]; O],  Z[k] = [xr_k (3 Nr); ur_k (2 Nr)],  O = [N][n_obs][3] = (ox, oy, clearance),
+ *     nmpc_np = 3 Nr + 5 Nr N + 3 N n_obs,
+ *     cost = sum_{k<N} (X_k - xr_k)' Q (X_k - xr_k) + (U_k - ur_k)' R (U_k - ur_k).
+ * Row (k, i, o), on X_k, is that of nmpc_create_moving_obstacles against table O[k].  Everything else is what
+ * nmpc_create_moving_obstacles gives: variables, g row layout (no dummy rows in block 0), mg = 3 Nr + N (3 Nr + M + Nr n_obs),
+ * bounds, status, stats and the path (warp-per-instance for 1..4 robots while M + Nr n_obs <= 32, else the dense-block path;
+ * t->force_block_path is honoured, t->thread_min_batch is ignored, t == NULL means the default tuning).
+ * Guarantee: if every Z[k] = [xs; 0], the outputs are bit for bit those of nmpc_create_moving_obstacles with p = [x0bar; xs; O].
+ * 1 <= n_obs <= 32, else NMPC_EINVAL.  nmpc_eval and the CCS patterns return NMPC_ENOTSUP; nmpc_shift, nmpc_plant,
+ * nmpc_set_order, nmpc_solve_host and nmpc_solve_trace work. */
+int nmpc_create_tracking_obstacles(const nmpc_desc *d, const nmpc_opts *o, const nmpc_tuning *t, int n_obs, nmpc_handle **out);
 
 /* Small generic optimal-control problems, one GPU thread per instance.  model NMPC_OCP_VAN_DER_POL is the direct-multiple-shooting
  * demo of mpc_pose_control_casadi.py:22-114: 2 states, 1 control, N intervals over the horizon T, each integrated by rk_steps RK4

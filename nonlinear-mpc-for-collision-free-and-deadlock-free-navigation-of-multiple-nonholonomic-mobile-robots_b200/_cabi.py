@@ -16,7 +16,7 @@ SYMBOLS = ["nmpc_default_opts", "nmpc_last_error", "nmpc_create", "nmpc_destroy"
            "nmpc_plant", "nmpc_eval", "nmpc_jac_pattern", "nmpc_hess_pattern", "nmpc_launch_count", "nmpc_probe_fp64",
            "nmpc_debug_block_profile", "nmpc_set_order", "nmpc_create_obstacles", "nmpc_create_ocp",
            "nmpc_default_tuning", "nmpc_create_tuned", "nmpc_probe_dmma", "nmpc_create_moving_obstacles",
-           "nmpc_create_tracking"]
+           "nmpc_create_tracking", "nmpc_create_tracking_obstacles"]
 
 
 class Desc(C.Structure):
@@ -66,6 +66,7 @@ def lib():
     L.nmpc_create_tuned.argtypes = [C.POINTER(Desc), C.POINTER(Opts), C.POINTER(Tuning), C.c_int, vp, C.POINTER(H)]
     L.nmpc_create_moving_obstacles.argtypes = [C.POINTER(Desc), C.POINTER(Opts), C.POINTER(Tuning), C.c_int, C.POINTER(H)]
     L.nmpc_create_tracking.argtypes = [C.POINTER(Desc), C.POINTER(Opts), C.POINTER(Tuning), C.POINTER(H)]
+    L.nmpc_create_tracking_obstacles.argtypes = [C.POINTER(Desc), C.POINTER(Opts), C.POINTER(Tuning), C.c_int, C.POINTER(H)]
     L.nmpc_create_ocp.argtypes = [C.c_int, C.c_int, C.c_double, C.c_int, C.POINTER(Opts), C.POINTER(H)]
     L.nmpc_destroy.argtypes = [H]
     L.nmpc_destroy.restype = None

@@ -166,14 +166,17 @@ struct BlockSolver {
         CE = br + (long long)NMPC_BR_CE * S * W; DL = br + (long long)NMPC_BR_DL * S * W;
         DU = br + (long long)NMPC_BR_DU * S * W;
         pp = P.p + (long long)inst * P.np;
-        {   // reference after x0bar: one setpoint xs (np = 2 ns), or Z[N][nz] of a tracking handle (np = ns + N nz, never 2 ns).
-            // (Told apart by np rather than by a flag in NmpcSolveParams: a larger parameter block would change the frame, and so
-            // the code, of every warp-path kernel, which copies it to local memory.)
-            const bool trk = family == 0 && P.np == ns + N * nz;
-            nref = trk ? nz : ns; rstr = trk ? nz : 0;
-        }
-        // obstacles in p: [N][nobs][3] after x0bar and xs, one table per stage; else the handle's table at every stage
-        obs = P.obs_in_p ? pp + 2 * ns : P.obs; ostr = P.obs_in_p ? 3 * nobs : 0;
+        // Reference after x0bar: one setpoint xs, or Z[N][nz] of a tracking handle; then, with the obstacles in p, one [nobs][3]
+        // table per stage.  The four layouts and their np:
+        //     [x0bar; xs]                 2 ns                 [x0bar; Z]         ns + N nz
+        //     [x0bar; xs; O[N]]           2 ns + 3 N nobs      [x0bar; Z; O[N]]   ns + N nz + 3 N nobs
+        // Since N nz = 5 Nr N never equals ns = 3 Nr, a tracking np never equals the setpoint np with the same obstacle block.
+        // (Told apart by np rather than by a flag in NmpcSolveParams: a larger parameter block would change the frame, and so
+        // the code, of every warp-path kernel, which copies it to local memory.)
+        const bool trk = P.np == ns + N * nz + (P.obs_in_p ? 3 * N * nobs : 0);
+        nref = trk ? nz : ns; rstr = trk ? nz : 0;
+        // obstacles in p: after x0bar and the reference, one table per stage; else the handle's table at every stage
+        obs = P.obs_in_p ? pp + ns + (trk ? N * nz : ns) : P.obs; ostr = P.obs_in_p ? 3 * nobs : 0;
         pairs = P.pairs;
         Pall = ws + (long long)R_COUNT * S * W;
         ldy = ((ns + 4) & ~7) + 4; ncp = (nc + 31) & ~31;

@@ -112,7 +112,7 @@ struct nmpc_handle {
     int nobs, family, rk_steps;               // static obstacles per robot; family: 0 centralized, 1 obstacles, 2 small OCP (thread per instance)
     double *d_obs;                            // [nobs][3] on the device
     bool obs_in_p;                            // obstacle family with the geometry in p (per instance and stage): no d_obs
-    bool tracking;                            // centralized family tracking a per-stage reference (nmpc_create_tracking)
+    bool tracking;                            // a per-stage reference in p (nmpc_create_tracking, nmpc_create_tracking_obstacles)
     bool thread_ok;                           // a thread-per-instance kernel exists for this problem (small-OCP family; one robot with
                                               // static obstacles): used for the small-OCP family always, else from thread_min_batch on
     size_t t_ws_doubles;                      // its scratch per instance
@@ -241,6 +241,13 @@ extern "C" int nmpc_create_tracking(const nmpc_desc *d, const nmpc_opts *o, cons
     return create_impl(d, o, t, 0, nullptr, false, true, out);
 }
 
+extern "C" int nmpc_create_tracking_obstacles(const nmpc_desc *d, const nmpc_opts *o, const nmpc_tuning *t, int n_obs, nmpc_handle **out)
+{
+    if (n_obs < 1 || n_obs > NMPC_MAX_OBSTACLES)
+        return fail(NMPC_EINVAL, "nmpc_create_tracking_obstacles: need 1..%d obstacles, got %d", NMPC_MAX_OBSTACLES, n_obs);
+    return create_impl(d, o, t, n_obs, nullptr, true, true, out);
+}
+
 // Small generic OCP family (thread per instance): currently the Van der Pol demo of mpc_pose_control_casadi.py
 extern "C" int nmpc_create_ocp(int model, int N, double T, int rk_steps, const nmpc_opts *o, nmpc_handle **out)
 {
@@ -298,9 +305,9 @@ static int create_impl(const nmpc_desc *d, const nmpc_opts *o, const nmpc_tuning
     if (t) h->tune = *t; else nmpc_default_tuning(&h->tune);
     h->ns = 3 * d->Nr; h->nc = 2 * d->Nr; h->M = d->Nr * (d->Nr - 1) / 2; h->S = d->N + 1;
     h->nobs = nobs; h->family = nobs > 0 ? 1 : 0; h->d_obs = nullptr; h->obs_in_p = obs_in_p; h->tracking = tracking;
-    // p = [x0bar; xs], then with the obstacles in p one [nobs][3] table per stage k = 0..N-1; tracking: p = [x0bar; Z[N][5 Nr]]
+    // p = [x0bar; xs] (tracking: [x0bar; Z[N][5 Nr]]), then with the obstacles in p one [nobs][3] table per stage k = 0..N-1
     h->n = h->ns * h->S + h->nc * d->N;
-    h->np = tracking ? h->ns + d->N * (h->ns + h->nc) : 2 * h->ns + (obs_in_p ? 3 * d->N * nobs : 0);
+    h->np = (tracking ? h->ns + d->N * (h->ns + h->nc) : 2 * h->ns) + (obs_in_p ? 3 * d->N * nobs : 0);
     // row layout: family 0 = (N+1) blocks of [ns equality rows ; M pair rows]; family 1 (static obstacles) = ns rows, then N
     // blocks of [ns ; M + Nr n_obs]   (first_scenario_mpc_obstacle_avoidance.py:109-125)
     h->mg = h->family ? h->ns + d->N * (h->ns + h->M + d->Nr * nobs) : h->S * (h->ns + h->M);
@@ -335,8 +342,12 @@ static int create_impl(const nmpc_desc *d, const nmpc_opts *o, const nmpc_tuning
     h->tb.jac_init = h->tb.jac_ps + (size_t)N * M * 4;
     h->tb.hes_rs = h->d_tables + h->nnzj;
     h->tb.hes_ps = h->tb.hes_rs + (size_t)N * Nr * 6;
-    switch (h->block_path ? 0 : (h->family ? 100 + Nr : (tracking ? 200 + Nr : Nr))) {
+    switch (h->block_path ? 0 : (h->family ? (tracking ? 300 : 100) + Nr : (tracking ? 200 + Nr : Nr))) {
 #ifndef NMPC_DEV_ONLY_NR
+        case 301: h->ws_doubles_per_slot = slot_doubles<1, true, true>(N); e = config_solve<1, true, true>(h); break;
+        case 302: h->ws_doubles_per_slot = slot_doubles<2, true, true>(N); e = config_solve<2, true, true>(h); break;
+        case 303: h->ws_doubles_per_slot = slot_doubles<3, true, true>(N); e = config_solve<3, true, true>(h); break;
+        case 304: h->ws_doubles_per_slot = slot_doubles<4, true, true>(N); e = config_solve<4, true, true>(h); break;
         case 201: h->ws_doubles_per_slot = slot_doubles<1, false, true>(N); e = config_solve<1, false, true>(h); break;
         case 202: h->ws_doubles_per_slot = slot_doubles<2, false, true>(N); e = config_solve<2, false, true>(h); break;
         case 203: h->ws_doubles_per_slot = slot_doubles<3, false, true>(N); e = config_solve<3, false, true>(h); break;
@@ -498,8 +509,12 @@ static int solve_impl(nmpc_handle *h, int B, const double *x0, const double *p, 
     if (thr && h->family == 2) solve_kernel_small_ocp<VanDerPol><<<grid, 64, 0, st>>>(P);
     else if (thr) solve_kernel_small_ocp<UnicycleObstacles><<<grid, 64, 0, st>>>(P);
     else if (h->block_path) solve_kernel_block<<<grid, h->threads, h->solve_smem, st>>>(P);
-    else switch (h->family ? 100 + h->d.Nr : (h->tracking ? 200 + h->d.Nr : h->d.Nr)) {
+    else switch (h->family ? (h->tracking ? 300 : 100) + h->d.Nr : (h->tracking ? 200 + h->d.Nr : h->d.Nr)) {
 #ifndef NMPC_DEV_ONLY_NR
+        case 301: solve_kernel<1, true, true><<<grid, h->threads, h->solve_smem, st>>>(P); break;
+        case 302: solve_kernel<2, true, true><<<grid, h->threads, h->solve_smem, st>>>(P); break;
+        case 303: solve_kernel<3, true, true><<<grid, h->threads, h->solve_smem, st>>>(P); break;
+        case 304: solve_kernel<4, true, true><<<grid, h->threads, h->solve_smem, st>>>(P); break;
         case 201: solve_kernel<1, false, true><<<grid, h->threads, h->solve_smem, st>>>(P); break;
         case 202: solve_kernel<2, false, true><<<grid, h->threads, h->solve_smem, st>>>(P); break;
         case 203: solve_kernel<3, false, true><<<grid, h->threads, h->solve_smem, st>>>(P); break;

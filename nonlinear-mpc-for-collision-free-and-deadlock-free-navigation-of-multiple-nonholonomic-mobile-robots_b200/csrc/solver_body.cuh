@@ -245,8 +245,9 @@ struct WarpSolver {
         }
         br = P.brows + (long long)inst * P.bstride;
         const double *pp = P.p + (long long)inst * ((OBS || TRK) ? P.np : 2 * NS);
-        if (OBS) {   // obstacles in p: [N][nobs][3] after x0bar and xs, one table per stage; else the handle's table at every stage
-            qtab = P.obs_in_p ? pp + 2 * NS : P.obs; qos = P.obs_in_p ? 3 * nobs : 0;
+        if (OBS) {   // obstacles in p: [N][nobs][3] after x0bar and xs (TRK: after x0bar and Z[0..N-1]), one table per stage;
+                     // else the handle's table at every stage
+            qtab = P.obs_in_p ? pp + (TRK ? NS + N * NZ : 2 * NS) : P.obs; qos = P.obs_in_p ? 3 * nobs : 0;
             if (isobs) qob = qtab + 3 * ((l - M) % nobs);
         }
         x0bar_l = isx ? pp[l] : 0.0;

@@ -98,18 +98,23 @@ class Problem:
     """Handle on the CUDA library for one (Nr, N, T, Q, R) problem family."""
 
     def __init__(self, Nr, N, T, Q=(1.0, 5.0, 0.1), R=(0.5, 0.05), obstacles=None, tuning=None, moving_obstacles=None,
-                 tracking=False, **opts):
+                 tracking=False, tracking_obstacles=None, **opts):
         """obstacles: optional [n_obs, 3] array of static circular obstacles (centre x, y, clearance = rob_dim + r_obs): the
         reference's obstacle-avoidance family (first_scenario_mpc_obstacle_avoidance.py:96-152), see nmpc_create_obstacles.
         moving_obstacles: n_obs instead of `obstacles` -> the same family with the obstacles in p, one [n_obs, 3] table per
         instance and stage (p = [x0bar; xs; O[N][n_obs][3]], see nmpc_create_moving_obstacles and params()).
         tracking: True -> the centralized family tracking a per-instance, per-stage state and control reference instead of one
         goal (p = [x0bar; Z[N][5Nr]], Z[k] = [xr_k; ur_k], see nmpc_create_tracking and params()); no obstacles.
+        tracking_obstacles: n_obs -> both: the moving-obstacle family tracking a per-stage reference, p = [x0bar; Z[N][5Nr];
+        O[N][n_obs][3]] (see nmpc_create_tracking_obstacles and params()); exclusive with the three keywords above.  The
+        handle has tracking = moving = True.
         tuning: optional dict of nmpc_tuning fields (convoy, ctas_per_sm, force_block_path, thread_min_batch)."""
         if obstacles is not None and moving_obstacles is not None:
             raise ValueError("obstacles= and moving_obstacles= are mutually exclusive")
         if tracking and (obstacles is not None or moving_obstacles is not None):
             raise ValueError("tracking=True cannot be combined with obstacles= or moving_obstacles=")
+        if tracking_obstacles is not None and (tracking or obstacles is not None or moving_obstacles is not None):
+            raise ValueError("tracking_obstacles= cannot be combined with tracking=, obstacles= or moving_obstacles=")
         self.L = lib()
         self.desc = Desc(int(Nr), int(N), float(T), (C.c_double * 3)(*[float(q) for q in Q]),
                          (C.c_double * 2)(*[float(r) for r in R]))
@@ -117,9 +122,13 @@ class Problem:
         self.h = C.c_void_p()
         self.obstacles = None if obstacles is None else np.ascontiguousarray(np.asarray(obstacles, dtype=np.float64).reshape(-1, 3))
         self.tuning = default_tuning(**(tuning or {}))
-        self.moving = moving_obstacles is not None
-        self.tracking = bool(tracking)
-        if self.tracking:
+        self.moving = moving_obstacles is not None or tracking_obstacles is not None
+        self.tracking = bool(tracking) or tracking_obstacles is not None
+        if tracking_obstacles is not None:
+            check(self.L.nmpc_create_tracking_obstacles(C.byref(self.desc), C.byref(self.opts), C.byref(self.tuning),
+                                                        int(tracking_obstacles), C.byref(self.h)))
+            self.nobs = int(tracking_obstacles)
+        elif self.tracking:
             check(self.L.nmpc_create_tracking(C.byref(self.desc), C.byref(self.opts), C.byref(self.tuning), C.byref(self.h)))
             self.nobs = 0
         elif self.moving:
@@ -179,8 +188,8 @@ class Problem:
     def params(self, x0bar, xs, obstacles=None, uref=None):
         """p [B, np] from x0bar [B, 3Nr], xs [B, 3Nr] and, for moving_obstacles, obstacles [B, N, n_obs, 3] (ox, oy, clearance of
         every obstacle at every stage).  For tracking: xs is the state reference [B, N, 3Nr] (or [B, 3Nr], the same at every
-        stage) and uref the control reference [B, N, 2Nr] (default zeros).  NumPy arrays give a NumPy array, CUDA tensors a
-        contiguous float64 tensor on their device."""
+        stage) and uref the control reference [B, N, 2Nr] (default zeros); with tracking_obstacles also obstacles as above.
+        NumPy arrays give a NumPy array, CUDA tensors a contiguous float64 tensor on their device."""
         B = x0bar.shape[0]
         if getattr(self, "tracking", False):
             return self._tracking_params(x0bar, xs, uref, obstacles)
@@ -202,7 +211,10 @@ class Problem:
 
     def _tracking_params(self, x0bar, xs, uref, obstacles):
         B, N = x0bar.shape[0], self.N
-        if obstacles is not None:
+        if self.moving:     # tracking_obstacles: O[N][n_obs][3] after Z
+            if obstacles is None or tuple(obstacles.shape) != (B, N, self.nobs, 3):
+                raise ValueError("obstacles must be [B, N, n_obs, 3] = [%d, %d, %d, 3]" % (B, N, self.nobs))
+        elif obstacles is not None:
             raise ValueError("obstacles go into p only for Problem(moving_obstacles=n_obs)")
         if tuple(x0bar.shape) != (B, self.ns) or tuple(xs.shape) not in ((B, self.ns), (B, N, self.ns)):
             raise ValueError("x0bar must be [B, %d] and xs [B, N, %d] or [B, %d]" % (self.ns, self.ns, self.ns))
@@ -212,11 +224,17 @@ class Problem:
             xr = np.broadcast_to(np.asarray(xs, np.float64).reshape(B, -1, self.ns), (B, N, self.ns))
             ur = np.zeros((B, N, self.nc)) if uref is None else np.asarray(uref, np.float64)
             Z = np.concatenate([xr, ur], axis=2).reshape(B, -1)
-            return np.ascontiguousarray(np.concatenate([np.asarray(x0bar, np.float64), Z], axis=1))
+            parts = [np.asarray(x0bar, np.float64), Z]
+            if obstacles is not None:
+                parts.append(np.asarray(obstacles, np.float64).reshape(B, -1))
+            return np.ascontiguousarray(np.concatenate(parts, axis=1))
         torch = self._torch()
         xr = xs.to(torch.float64).reshape(B, -1, self.ns).expand(B, N, self.ns)
         ur = (torch.zeros((B, N, self.nc), dtype=torch.float64, device=xs.device) if uref is None else uref.to(torch.float64))
-        return torch.cat([x0bar.to(torch.float64), torch.cat([xr, ur], dim=2).reshape(B, -1)], dim=1).contiguous()
+        parts = [x0bar.to(torch.float64), torch.cat([xr, ur], dim=2).reshape(B, -1)]
+        if obstacles is not None:
+            parts.append(obstacles.to(torch.float64).reshape(B, -1))
+        return torch.cat(parts, dim=1).contiguous()
 
     def launch_count(self):
         return int(self.L.nmpc_launch_count(self.h))
@@ -366,13 +384,26 @@ def closed_loop(prob, P, lbx, ubx, lbg, ubg, steps, tol=1e-1, dmin=None, obstacl
     reference (required by, and only for, Problem(tracking=True)): CUDA float64 [steps+N, B, 5Nr], rows [xr_t; ur_t] of the
     reference over time; step t solves with rows t..t+N-1 as Z in p (P then needs only its first 3Nr columns, x0bar), there is
     no stop test (every instance is active at every step), and the result gains track_err [steps+1, B] = the largest xy distance
-    over robots between the plant state and the reference state at the same time."""
+    over robots between the plant state and the reference state at the same time.
+    Problem(tracking_obstacles=n_obs) requires both: step t solves with Z = reference rows t..t+N-1 and O = obstacle tables
+    t..t+N-1 (P then needs only x0bar), without a stop test, and the result carries both track_err and min_clearance."""
     torch = prob._torch()
     B, ns, nc, N = P.shape[0], prob.ns, prob.nc, prob.N
     tracking = getattr(prob, "tracking", False)
+    both = tracking and getattr(prob, "moving", False)      # Problem(tracking_obstacles=n_obs)
+    if both and (reference is None or obstacles is None):
+        raise ValueError("a Problem(tracking_obstacles=n_obs) needs both reference= and obstacles=")
     if tracking != (reference is not None):
         raise ValueError("reference= is required by, and only accepted for, a Problem(tracking=True)")
-    if tracking:
+    if both:
+        if not (reference.is_cuda and reference.dtype == torch.float64) or tuple(reference.shape) != (steps + N, B, ns + nc):
+            raise ValueError("reference must be a float64 CUDA tensor [steps + N, B, 5Nr] = [%d, %d, %d]" % (steps + N, B, ns + nc))
+        if not (obstacles.is_cuda and obstacles.dtype == torch.float64) or tuple(obstacles.shape) != (steps + N, B, prob.nobs, 3):
+            raise ValueError("obstacles must be a float64 CUDA tensor [steps + N, B, n_obs, 3] = [%d, %d, %d, 3]"
+                             % (steps + N, B, prob.nobs))
+        p = torch.empty((B, prob.np_), dtype=torch.float64, device=P.device)
+        p[:, :ns] = P[:, :ns]
+    elif tracking:
         if not (reference.is_cuda and reference.dtype == torch.float64) or tuple(reference.shape) != (steps + N, B, ns + nc):
             raise ValueError("reference must be a float64 CUDA tensor [steps + N, B, 5Nr] = [%d, %d, %d]" % (steps + N, B, ns + nc))
         p = torch.cat([P[:, :ns], torch.empty((B, N * (ns + nc)), dtype=torch.float64, device=P.device)], dim=1)
@@ -396,10 +427,14 @@ def closed_loop(prob, P, lbx, ubx, lbg, ubg, steps, tol=1e-1, dmin=None, obstacl
     for t in range(steps):
         if t == 0:
             prob.set_order(None)
-        if obstacles is not None:
+        if both:
+            p[:, ns:ns + N * (ns + nc)] = reference[t:t + N].permute(1, 0, 2).reshape(B, -1)
+            p[:, ns + N * (ns + nc):] = obstacles[t:t + N].permute(1, 0, 2, 3).reshape(B, -1)
+        elif obstacles is not None:
             p[:, 2 * ns:] = obstacles[t:t + N].permute(1, 0, 2, 3).reshape(B, -1)
         if tracking:
-            p[:, ns:] = reference[t:t + N].permute(1, 0, 2).reshape(B, -1)
+            if not both:
+                p[:, ns:] = reference[t:t + N].permute(1, 0, 2).reshape(B, -1)
             active = torch.ones(B, dtype=torch.bool, device=P.device)
         else:
             active = (p[:, :ns] - p[:, ns:2 * ns]).norm(dim=1) > tol
@@ -492,24 +527,25 @@ class NlpSolver:
             pv = np.asarray(_flat(p, P.np_, "p"))
             if getattr(P, "tracking", False):
                 # Z[k] = [xr_k; ur_k] enters only the cost (X_k - xr_k)'Q(X_k - xr_k) + (U_k - ur_k)'R(U_k - ur_k)
-                Z = pv[P.ns:].reshape(P.N, P.ns + P.nc)
+                Z = pv[P.ns:P.ns + P.N * (P.ns + P.nc)].reshape(P.N, P.ns + P.nc)
                 Uk = o["x"][0, P.ns * (P.N + 1):].reshape(P.N, P.nc)
                 Rd = np.tile(np.asarray(list(P.desc.R), float), P.Nr)
                 lam_z = np.concatenate([-2.0 * Qd * (Xk - Z[:, :P.ns]), -2.0 * Rd * (Uk - Z[:, P.ns:])], axis=1)
-                lam_p[P.ns:] = lam_z.ravel()
+                lam_p[P.ns:P.ns + lam_z.size] = lam_z.ravel()
             else:
                 lam_p[P.ns:2 * P.ns] = -2.0 * Qd * (Xk - pv[P.ns:2 * P.ns][None]).sum(axis=0)
             if getattr(P, "moving", False):
                 # obstacle block O[k][o] = (ox, oy, c): row (k, i, o) = rho - c with rho = |pos_{k,i} - (ox, oy)|, so
                 # dL/d(ox, oy) = -sum_i lam (pos - o) / rho and dL/dc = -sum_i lam
-                O = pv[2 * P.ns:].reshape(P.N, P.nobs, 3)
+                o0 = P.np_ - 3 * P.N * P.nobs      # after xs (6Nr), or after Z with tracking_obstacles (3Nr + 5Nr N)
+                O = pv[o0:].reshape(P.N, P.nobs, 3)
                 lam = o["lam_g"][0, P.ns:].reshape(P.N, P.ns + P.M + P.Nr * P.nobs)[:, P.ns + P.M:].reshape(P.N, P.Nr, P.nobs)
                 d = Xk.reshape(P.N, P.Nr, 3)[:, :, None, :2] - O[:, None, :, :2]
                 gxy = d / np.linalg.norm(d, axis=-1, keepdims=True)
                 lam_o = np.empty((P.N, P.nobs, 3))
                 lam_o[..., :2] = -(lam[..., None] * gxy).sum(axis=1)
                 lam_o[..., 2] = -lam.sum(axis=1)
-                lam_p[2 * P.ns:] = lam_o.ravel()
+                lam_p[o0:] = lam_o.ravel()
         return {"x": DM(o["x"][0]), "f": DM(o["f"][:1]), "g": DM(o["g"][0]), "lam_x": DM(o["lam_x"][0]),
                 "lam_g": DM(o["lam_g"][0]), "lam_p": DM(lam_p)}
 
@@ -528,6 +564,7 @@ def nlpsol(name, plugin, nlp, opts=None):
         {'family': 'unicycle_obstacles', ..., 'obstacles': [[x, y, clearance], ...]}
         {'family': 'unicycle_moving_obstacles', ..., 'n_obs'}: the obstacles in p = [x0bar; xs; O[N][n_obs][3]]
         {'family': 'unicycle_tracking', 'Nr', 'N', 'T', 'Q', 'R'}: a per-stage reference in p = [x0bar; Z[N][5Nr]]
+        {'family': 'unicycle_tracking_obstacles', ..., 'n_obs'}: both, p = [x0bar; Z[N][5Nr]; O[N][n_obs][3]]
     `opts` uses the reference's layout: {'print_time': 0, 'ipopt': {'max_iter': 2000, ...}}.
     """
     if plugin not in ("ipopt", "b200ipm"):
@@ -537,11 +574,13 @@ def nlpsol(name, plugin, nlp, opts=None):
         kw = {k: v for k, v in ip.items() if k in _IPOPT_KEYS}
         return NlpSolver(name, SmallOcp("van_der_pol", nlp.get("N", 20), nlp.get("T", 10.0), nlp.get("rk_steps", 4), **kw))
     if not isinstance(nlp, dict) or nlp.get("family", "unicycle_centralized") not in ("unicycle_centralized", "unicycle_obstacles",
-                                                                                   "unicycle_moving_obstacles", "unicycle_tracking"):
+                                                                                   "unicycle_moving_obstacles", "unicycle_tracking",
+                                                                                   "unicycle_tracking_obstacles"):
         raise ValueError("nlp must be a descriptor {'family':'unicycle_centralized'|'unicycle_obstacles'|"
-                         "'unicycle_moving_obstacles'|'unicycle_tracking','Nr','N','T',...}")
-    if nlp.get("family") == "unicycle_moving_obstacles" and nlp.get("n_obs") is None:
-        raise ValueError("family 'unicycle_moving_obstacles' needs 'n_obs'")
+                         "'unicycle_moving_obstacles'|'unicycle_tracking'|'unicycle_tracking_obstacles','Nr','N','T',...}")
+    for fam in ("unicycle_moving_obstacles", "unicycle_tracking_obstacles"):
+        if nlp.get("family") == fam and nlp.get("n_obs") is None:
+            raise ValueError("family '%s' needs 'n_obs'" % fam)
     if nlp.get("family") == "unicycle_obstacles" and nlp.get("obstacles") is None:
         raise ValueError("family 'unicycle_obstacles' needs 'obstacles': [[x, y, clearance], ...]")
     ip = dict((opts or {}).get("ipopt", {}))
@@ -550,5 +589,6 @@ def nlpsol(name, plugin, nlp, opts=None):
     prob = Problem(nlp["Nr"], nlp["N"], nlp["T"], nlp.get("Q", (1.0, 5.0, 0.1)), nlp.get("R", (0.5, 0.05)),
                    obstacles=nlp.get("obstacles") if nlp.get("family") == "unicycle_obstacles" else None,
                    moving_obstacles=nlp.get("n_obs") if nlp.get("family") == "unicycle_moving_obstacles" else None,
-                   tracking=nlp.get("family") == "unicycle_tracking", **kw)
+                   tracking=nlp.get("family") == "unicycle_tracking",
+                   tracking_obstacles=nlp.get("n_obs") if nlp.get("family") == "unicycle_tracking_obstacles" else None, **kw)
     return NlpSolver(name, prob)
