@@ -206,6 +206,37 @@ int nmpc_solve_trace(nmpc_handle *h, int B, const double *x0, const double *p,
                      int32_t *status, int32_t *iters, double *stats, double *trace, int max_trace,
                      void *workspace, size_t workspace_bytes, void *stream);
 
+/* Parametric sensitivities of returned solutions: how x* moves when p moves (sIPOPT's sensitivity; CasADi's forward and reverse
+ * derivatives of an nlpsol's x with respect to p).  Inputs are what nmpc_solve returned for B instances (x, lam_x [B,n],
+ * lam_g [B,mg], DEVICE) with the p [B,np] and the bounds of that solve (bounds_batched as in nmpc_solve).  From them the call
+ * rebuilds, per instance, the interior-point KKT matrix at the point, with CasADi's signs (L = f + lam_g'g + lam_x'x):
+ *     K = [[W + Sx, J'], [J, -Ss^-1]],  W = Hessian of L,  Sx_i = |lam_x_i| / d_i,  Ss_j = |lam_g_j| / d_j on inequality rows,
+ * d the distance of x_i (of g_j(x)) to the bound its multiplier pushes against, relaxed by bound_relax_factor (max(1,|b|)
+ * scaled) as in the solve; no finite bound: 0; equality rows stay equalities, the constant block-0 rows get weight 0.  One
+ * factorisation of K (the solve's stage-wise Riccati sweep, no regularisation) and one forward pass give
+ *     nmpc_solution_vjp:  K [a; b] = [x_bar; 0],  p_bar = -(d2L/dx dp)' a - (dg/dp)' b          (reverse mode, [B,n] -> [B,np])
+ *                         i.e. p_bar[x0bar] = b of the block-0 rows, p_bar[xs] = 2Q sum_{k<N} a[X_k];
+ *                         tracking: p_bar[xr_k] = 2Q a[X_k], p_bar[ur_k] = 2R a[U_k]
+ *     nmpc_solution_jvp:  K [x_dot; lam_dot] = -[d2L/dx dp p_dot; dg/dp p_dot]                  (forward mode, [B,np] -> [B,n])
+ * At a strictly complementary KKT point this is the active-set implicit-function derivative of x* with respect to p up to O(1/S) on the active
+ * bounds, i.e. about bound_relax_factor relative.  sens_status [B] (int32, may be NULL): 0 ok; 1 wrong inertia (a pivot <= 0:
+ * second-order sufficiency fails at the point, the derivative is not defined) -- the instance's outputs are NaN; a negative
+ * NMPC_E* code when the bounds are rejected as nmpc_solve rejects them (outputs NaN).  Handles from nmpc_create and
+ * nmpc_create_tracking with 1..10 robots, whatever their tuning or solve path; the obstacle families, 11..64 robots and the
+ * small-OCP family return NMPC_ENOTSUP.  NULL inputs, B <= 0, a handle created on another device or a workspace smaller than
+ * nmpc_sensitivity_workspace_bytes(h, B, bounds_batched) return NMPC_EINVAL.  Asynchronous on stream; the handle's state
+ * (including the nmpc_set_order hint, which does not apply) is left unchanged. */
+int nmpc_solution_vjp(nmpc_handle *h, int B, const double *x, const double *lam_x, const double *lam_g, const double *p,
+                      const double *lbx, const double *ubx, const double *lbg, const double *ubg, int bounds_batched,
+                      const double *x_bar, double *p_bar, int32_t *sens_status, void *workspace, size_t workspace_bytes,
+                      void *stream);
+int nmpc_solution_jvp(nmpc_handle *h, int B, const double *x, const double *lam_x, const double *lam_g, const double *p,
+                      const double *lbx, const double *ubx, const double *lbg, const double *ubg, int bounds_batched,
+                      const double *p_dot, double *x_dot, int32_t *sens_status, void *workspace, size_t workspace_bytes,
+                      void *stream);
+/* Device scratch of both calls (0 for an unsupported handle or B <= 0). */
+size_t nmpc_sensitivity_workspace_bytes(const nmpc_handle *h, int B, int bounds_batched);
+
 /* Same call with HOST buffers (what a CasADi-style caller has): H2D of the inputs, solve, D2H of
  * the requested outputs, synchronous.  Staging buffers live in the handle and grow on demand. */
 int nmpc_solve_host(nmpc_handle *h, int B, const double *x0, const double *p,

@@ -16,7 +16,8 @@ SYMBOLS = ["nmpc_default_opts", "nmpc_last_error", "nmpc_create", "nmpc_destroy"
            "nmpc_plant", "nmpc_eval", "nmpc_jac_pattern", "nmpc_hess_pattern", "nmpc_launch_count", "nmpc_probe_fp64",
            "nmpc_debug_block_profile", "nmpc_set_order", "nmpc_create_obstacles", "nmpc_create_ocp",
            "nmpc_default_tuning", "nmpc_create_tuned", "nmpc_probe_dmma", "nmpc_create_moving_obstacles",
-           "nmpc_create_tracking", "nmpc_create_tracking_obstacles"]
+           "nmpc_create_tracking", "nmpc_create_tracking_obstacles", "nmpc_solution_vjp", "nmpc_solution_jvp",
+           "nmpc_sensitivity_workspace_bytes"]
 
 
 class Desc(C.Structure):
@@ -88,6 +89,10 @@ def lib():
     L.nmpc_probe_fp64.argtypes = [C.POINTER(C.c_double)]
     L.nmpc_debug_block_profile.argtypes = [C.POINTER(C.c_longlong), C.c_int]
     L.nmpc_set_order.argtypes = [H, vp, C.c_int]
+    L.nmpc_solution_vjp.argtypes = [H, C.c_int] + [dp] * 8 + [C.c_int, dp, dp, ip, vp, C.c_size_t, vp]
+    L.nmpc_solution_jvp.argtypes = [H, C.c_int] + [dp] * 8 + [C.c_int, dp, dp, ip, vp, C.c_size_t, vp]
+    L.nmpc_sensitivity_workspace_bytes.argtypes = [H, C.c_int, C.c_int]
+    L.nmpc_sensitivity_workspace_bytes.restype = C.c_size_t
     L.nmpc_probe_dmma.argtypes = [C.POINTER(C.c_double)]
     L.nmpc_launch_count.restype = C.c_longlong
     _LIB = L

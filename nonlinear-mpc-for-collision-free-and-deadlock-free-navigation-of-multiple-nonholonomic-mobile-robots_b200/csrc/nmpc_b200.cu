@@ -7,6 +7,7 @@
 #include <stdlib.h>
 
 #include <algorithm>
+#include <type_traits>
 #include <vector>
 
 #include "nmpc_b200.h"
@@ -96,6 +97,23 @@ __global__ void __launch_bounds__((SolveCfg<NR, OBS, TRK>::THREADS), (SolveCfg<N
     }
 }
 
+// parametric sensitivities of returned solutions (nmpc_solution_vjp / nmpc_solution_jvp): the warp solver's layout and launch
+// bounds, one instance per team at a time, instances strided over a grid of at most SENS_CTAS_PER_SM CTAs per SM
+template <int NR, bool TRK>
+__global__ void __launch_bounds__((SolveCfg<NR, false, TRK>::THREADS), (SolveCfg<NR, false, TRK>::MIN_CTAS)) sens_kernel(const NmpcSolveParams P, const NmpcSensParams S)
+{
+    extern __shared__ double smem[];
+    typedef WarpSolver<NR, false, TRK> WSol;
+    typedef SolveCfg<NR, false, TRK> Cfg;
+    const int team = threadIdx.x / Cfg::LW;
+    WSol s(P, smem + (size_t)team * WSol::SM_DOUBLES, P.ws + ((long long)blockIdx.x * Cfg::TEAMS + team) * P.ws_stride);
+    s.init_team();
+    for (int inst = blockIdx.x * Cfg::TEAMS + team; inst < P.B; inst += gridDim.x * Cfg::TEAMS) {
+        s.setup(inst);
+        s.sensitivity(S);
+    }
+}
+
 struct nmpc_handle {
     nmpc_desc d;
     nmpc_opts o;
@@ -120,6 +138,7 @@ struct nmpc_handle {
     int convoy;                               // warp path: iteration-level convoy of the CTA's warps (instruction-cache locality)
     bool block_path, eval_ok;                 // Nr > 10: CTA-per-instance dense-block solver; eval record fits shared memory
     int *d_pairs;                             // pair table (i, j) of the inequality rows, block path
+    bool sens_smem_set;                       // sens_kernel's shared-memory attribute is set (first sensitivity call)
     // host-pointer API staging
     char *d_buf;
     size_t d_bytes;
@@ -575,6 +594,143 @@ extern "C" int nmpc_solve_trace(nmpc_handle *h, int B, const double *x0, const d
 {
     return solve_impl(h, B, x0, p, lbx, ubx, lbg, ubg, bounds_batched, x, f, g, lam_x, lam_g, status, iters, stats, trace, max_trace,
                       workspace, workspace_bytes, (cudaStream_t)stream);
+}
+
+// ------------------------------------------------------------------------------------------------
+// parametric sensitivities (nmpc_solution_vjp / nmpc_solution_jvp): the warp layout whatever path the handle's solve takes
+// ------------------------------------------------------------------------------------------------
+#define SENS_CTAS_PER_SM 3
+static int sens_lw(const nmpc_handle *h) { return 5 * h->d.Nr + 1 <= 32 ? 32 : 64; }
+static int sens_teams(const nmpc_handle *h) { return sens_lw(h) == 32 ? SOLVE_WARPS : 2; }
+static int sens_grid(const nmpc_handle *h, int B)
+{
+    const int need = (B + sens_teams(h) - 1) / sens_teams(h), cap = h->sm_count * SENS_CTAS_PER_SM;
+    return need < cap ? need : cap;
+}
+template <int NR, bool TRK> struct SensLaunch {
+    static size_t slot_doubles(int N) { return (size_t)WarpSolver<NR, false, TRK>::ws_doubles(N); }
+    static size_t smem() { return (size_t)SolveCfg<NR, false, TRK>::TEAMS * WarpSolver<NR, false, TRK>::SM_DOUBLES * sizeof(double); }
+    static cudaError_t run(nmpc_handle *h, int grid, const NmpcSolveParams &P, const NmpcSensParams &S, cudaStream_t st)
+    {
+        if (!h->sens_smem_set) {
+            cudaError_t e = cudaFuncSetAttribute(sens_kernel<NR, TRK>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem());
+            if (e != cudaSuccess) return e;
+            h->sens_smem_set = true;
+        }
+        sens_kernel<NR, TRK><<<grid, SolveCfg<NR, false, TRK>::THREADS, smem(), st>>>(P, S);
+        return cudaGetLastError();
+    }
+};
+// f(integral_constant<int, Nr>, bool_constant<tracking>) for the handle's Nr (1..10; development builds: NMPC_DEV_ONLY_NR only)
+template <int R> using SensNr = std::integral_constant<int, R>;
+template <class F> static auto sens_dispatch(const nmpc_handle *h, F &&f) -> decltype(f(SensNr<1>(), std::false_type()))
+{
+    const bool t = h->tracking;
+    switch (h->d.Nr) {
+#ifndef NMPC_DEV_ONLY_NR
+        case 1: return t ? f(SensNr<1>(), std::true_type()) : f(SensNr<1>(), std::false_type());
+        case 2: return t ? f(SensNr<2>(), std::true_type()) : f(SensNr<2>(), std::false_type());
+        case 3: return t ? f(SensNr<3>(), std::true_type()) : f(SensNr<3>(), std::false_type());
+        case 4: return t ? f(SensNr<4>(), std::true_type()) : f(SensNr<4>(), std::false_type());
+        case 5: return t ? f(SensNr<5>(), std::true_type()) : f(SensNr<5>(), std::false_type());
+        case 6: return t ? f(SensNr<6>(), std::true_type()) : f(SensNr<6>(), std::false_type());
+        case 7: return t ? f(SensNr<7>(), std::true_type()) : f(SensNr<7>(), std::false_type());
+        case 8: return t ? f(SensNr<8>(), std::true_type()) : f(SensNr<8>(), std::false_type());
+        case 9: return t ? f(SensNr<9>(), std::true_type()) : f(SensNr<9>(), std::false_type());
+        default: return t ? f(SensNr<10>(), std::true_type()) : f(SensNr<10>(), std::false_type());
+#else
+        default: return f(SensNr<NMPC_DEV_ONLY_NR>(), std::false_type());
+#endif
+    }
+}
+static size_t sens_slot_doubles(const nmpc_handle *h)
+{
+    return sens_dispatch(h, [&](auto nr, auto trk) { return SensLaunch<decltype(nr)::value, decltype(trk)::value>::slot_doubles(h->d.N); });
+}
+static cudaError_t sens_launch(nmpc_handle *h, int grid, const NmpcSolveParams &P, const NmpcSensParams &S, cudaStream_t st)
+{
+    return sens_dispatch(h, [&](auto nr, auto trk) { return SensLaunch<decltype(nr)::value, decltype(trk)::value>::run(h, grid, P, S, st); });
+}
+static int sens_supported(const nmpc_handle *h, const char *fn)
+{
+    if (!h) return fail(NMPC_EINVAL, "%s: NULL handle", fn);
+    if (h->family == 2) return fail(NMPC_ENOTSUP, "%s: not available for the small-OCP family", fn);
+    if (h->family == 1) return fail(NMPC_ENOTSUP, "%s: not available for the obstacle families (static, moving, tracking among obstacles)", fn);
+    if (h->d.Nr > 10) return fail(NMPC_ENOTSUP, "%s: Nr = %d; supported: 1..10 robots", fn, h->d.Nr);
+    return 0;
+}
+static size_t sens_ws_bytes(const nmpc_handle *h, int B, int nb)
+{
+    return 256 + (size_t)nb * NMPC_BR_COUNT * h->S * sens_lw(h) * sizeof(double) +
+           (size_t)sens_grid(h, B) * sens_teams(h) * sens_slot_doubles(h) * sizeof(double);
+}
+
+extern "C" size_t nmpc_sensitivity_workspace_bytes(const nmpc_handle *h, int B, int bounds_batched)
+{
+    if (!h || B <= 0 || h->family != 0 || h->d.Nr > 10) return 0;
+    return sens_ws_bytes(h, B, bounds_batched ? B : 1);
+}
+
+static int sens_impl(const char *fn, nmpc_handle *h, int B, const double *x, const double *lam_x, const double *lam_g, const double *p,
+                     const double *lbx, const double *ubx, const double *lbg, const double *ubg, int bounds_batched, const double *seed,
+                     double *out, int32_t *status, void *workspace, size_t workspace_bytes, cudaStream_t st, int reverse)
+{
+    int rc = sens_supported(h, fn);
+    if (rc) return rc;
+    if (!x || !lam_x || !lam_g || !p || !lbx || !ubx || !lbg || !ubg || !seed || !out || !workspace)
+        return fail(NMPC_EINVAL, "%s: NULL argument", fn);
+    if (B <= 0) return fail(NMPC_EINVAL, "%s: B must be positive", fn);
+    {
+        int cur = -1;
+        if (cudaGetDevice(&cur) != cudaSuccess || cur != h->dev)
+            return fail(NMPC_EINVAL, "%s: the handle was created on CUDA device %d but device %d is current", fn, h->dev, cur);
+    }
+    const int nb = bounds_batched ? B : 1, lw = sens_lw(h);
+    const size_t need = sens_ws_bytes(h, B, nb);
+    if (workspace_bytes < need) return fail(NMPC_EINVAL, "%s: workspace %zu B < %zu B required (nmpc_sensitivity_workspace_bytes)", fn, workspace_bytes, need);
+    char *base = (char *)workspace;
+    int *berr = (int *)base + 1;
+    double *brows = (double *)(base + 256);
+    CUDA_OK(cudaMemsetAsync(base, 0, 256, st));
+    {
+        long long total = (long long)nb * h->S * lw;
+        int blocks = (int)std::min<long long>((total + 255) / 256, 4096);
+        prep_bounds_kernel<<<blocks, 256, 0, st>>>(h->d.Nr, h->d.N, h->o.bound_relax_factor, nb, lw, lbx, ubx, lbg, ubg, brows, berr, 0, 0, 1);
+        h->launches++;
+    }
+    NmpcSolveParams P;
+    memset(&P, 0, sizeof P);
+    P.Nr = h->d.Nr; P.N = h->d.N; P.B = B; P.T = h->d.T;
+    memcpy(P.Q, h->d.Q, sizeof P.Q); memcpy(P.R, h->d.R, sizeof P.R);
+    P.o = h->o; P.p = p; P.brows = brows;
+    P.bstride = bounds_batched ? (long long)NMPC_BR_COUNT * h->S * lw : 0;
+    P.bound_err = berr; P.np = h->np;
+    P.ws = (double *)(base + 256 + (size_t)nb * NMPC_BR_COUNT * h->S * lw * sizeof(double));
+    P.ws_stride = (long long)sens_slot_doubles(h);
+    NmpcSensParams S;
+    S.x = x; S.lam_x = lam_x; S.lam_g = lam_g; S.seed = seed; S.out = out; S.status = status; S.reverse = reverse;
+    cudaError_t e = sens_launch(h, sens_grid(h, B), P, S, st);
+    h->launches++;
+    if (e != cudaSuccess) return fail(NMPC_ECUDA, "%s: launch failed: %s", fn, cudaGetErrorString(e));
+    return 0;
+}
+
+extern "C" int nmpc_solution_vjp(nmpc_handle *h, int B, const double *x, const double *lam_x, const double *lam_g, const double *p,
+                                 const double *lbx, const double *ubx, const double *lbg, const double *ubg, int bounds_batched,
+                                 const double *x_bar, double *p_bar, int32_t *sens_status, void *workspace, size_t workspace_bytes,
+                                 void *stream)
+{
+    return sens_impl("nmpc_solution_vjp", h, B, x, lam_x, lam_g, p, lbx, ubx, lbg, ubg, bounds_batched, x_bar, p_bar, sens_status,
+                     workspace, workspace_bytes, (cudaStream_t)stream, 1);
+}
+
+extern "C" int nmpc_solution_jvp(nmpc_handle *h, int B, const double *x, const double *lam_x, const double *lam_g, const double *p,
+                                 const double *lbx, const double *ubx, const double *lbg, const double *ubg, int bounds_batched,
+                                 const double *p_dot, double *x_dot, int32_t *sens_status, void *workspace, size_t workspace_bytes,
+                                 void *stream)
+{
+    return sens_impl("nmpc_solution_jvp", h, B, x, lam_x, lam_g, p, lbx, ubx, lbg, ubg, bounds_batched, p_dot, x_dot, sens_status,
+                     workspace, workspace_bytes, (cudaStream_t)stream, 0);
 }
 
 static size_t al(size_t v) { return (v + 255) & ~(size_t)255; }

@@ -43,4 +43,14 @@ typedef struct NmpcSolveParams {
     int obs_in_p;                    /* obstacle family: geometry from p ([N][nobs][3] after x0bar, xs), not from obs */
 } NmpcSolveParams;
 
+/* Inputs and outputs of nmpc_solution_vjp / nmpc_solution_jvp (sens_kernel).  A struct of its own, passed next to
+ * NmpcSolveParams, so that the solve kernels' parameter block stays as it is. */
+typedef struct NmpcSensParams {
+    const double *x, *lam_x, *lam_g; /* a returned point [B,n], [B,n], [B,mg]             */
+    const double *seed;              /* reverse: x_bar [B,n];  forward: p_dot [B,np]      */
+    double *out;                     /* reverse: p_bar [B,np]; forward: x_dot [B,n]       */
+    int *status;                     /* [B] or NULL: 0 ok, 1 wrong inertia, < 0 bounds rejected */
+    int reverse;
+} NmpcSensParams;
+
 #endif

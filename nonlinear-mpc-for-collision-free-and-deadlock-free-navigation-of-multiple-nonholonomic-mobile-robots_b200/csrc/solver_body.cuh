@@ -585,11 +585,15 @@ struct WarpSolver {
     //   last lane:          a0p..a4p = HH[0..4]  (the gradient, one row per component class);   every other row: zeros.
     // (The first version built the column through a [5Nr][32] shared-memory column buffer with rolled loops over robots and
     // pairs: 7.7 KB per instance and ~570 instructions per stage, against ~200 and 2.6 KB here.)
+    // MODE 3 (sensitivity(), never called by the solve): the matrix of MODE 0 with the stage gradient read from the R_GX rows
+    // (a seed) instead of the cost's gradient; with mu = 0 and soc the right-hand side is entirely what the caller put in R_GX,
+    // R_CSOC and R_DSOC.
     // ---------------------------------------------------------------------------------------
     template <int MODE>
     NMPC_PASS bool factor(double mu, double delta, bool soc)
     {
         NMPC_LOCALS
+        constexpr int MB = MODE == 3 ? 0 : MODE;   // the mode that defines the matrix
         const double zeta = MODE == 2 ? sqrt(mu) : 0.0, kd = this->P.o.kappa_d;
         const bool isL = (l == LW - 1);
         double X[NS], U[NC];
@@ -644,7 +648,8 @@ struct WarpSolver {
         // terminal stage: X_N carries no cost and no distance rows, only its box
         {
             double sig = 0.0, gx = 0.0;
-            if (isx) sig_g<MODE>(kd, row(R_Z, N)[l], brow(NMPC_BR_BL, N)[l], brow(NMPC_BR_BU, N)[l], row(R_ZL, N)[l], row(R_ZU, N)[l], mu, 0.0, sig, gx);
+            if (isx) sig_g<MB>(kd, row(R_Z, N)[l], brow(NMPC_BR_BL, N)[l], brow(NMPC_BR_BU, N)[l], row(R_ZL, N)[l], row(R_ZU, N)[l], mu,
+                               MODE == 3 ? row(R_GX, N)[l] : 0.0, sig, gx);
             hb[l] = isx ? gx : 0.0;
             tsync();
             NMPC_UNROLL
@@ -674,7 +679,7 @@ struct WarpSolver {
                 c4[4 * l] = a_; c4[4 * l + 1] = b_; c4[4 * l + 2] = tc; c4[4 * l + 3] = ts;
                 double *cf = row(R_COEF, k);
                 cf[l] = a_; cf[CFS + l] = b_; cf[2 * CFS + l] = tc; cf[3 * CFS + l] = ts;
-                if (MODE == 0) {
+                if (MB == 0) {
                     const double *yc = stg + FS_YC * LW;
                     double lx = yc[3 * l], ly = yc[3 * l + 1];
                     crs[l] = T * (lx * s_ - ly * c_); thd[l] = T * v * (lx * c_ + ly * s_);
@@ -705,7 +710,7 @@ struct WarpSolver {
                 QIn in;
                 in.lo = stg[FS_DL * LW + l]; in.hi = stg[FS_DU * LW + l]; in.s = stg[FS_S * LW + l]; in.vl = stg[FS_VL * LW + l];
                 in.vu = stg[FS_VU * LW + l]; in.yd = stg[FS_YD * LW + l]; in.dsoc = stg[FS_DSOC * LW + l];
-                ineq_block<MODE>(row, in, l, pi, pj, isobs, qob + k * qos, kd, k + 1, mu, delta, soc, zb, a0, a1, a2, a3, a4);
+                ineq_block<MB>(row, in, l, pi, pj, isobs, qob + k * qos, kd, k + 1, mu, delta, soc, zb, a0, a1, a2, a3, a4);
                 // pair row: entries (pi, pj) and (pj, pi); obstacle row: column NR + o of robot pi (it only feeds the row sum)
                 const int e1 = isobs ? pi * TCOLS + NR + (l - M) % nobs : pi * TCOLS + pj, e2 = isobs ? e1 : pj * TCOLS + pi;
                 tt[e2] = -a0; tt[TSZ + e2] = -a2; tt[2 * TSZ + e2] = -a1; tt[3 * TSZ + e2] = -a3; tt[4 * TSZ + e2] = -a4;
@@ -739,14 +744,14 @@ struct WarpSolver {
             // stage gradient h_l (variable l) and diagonal curvature
             double sig = 0.0, gx = 0.0, dg = 0.0;
             if (isz) {
-                sig_g<MODE>(kd, zk, stg[FS_BL * LW + l], stg[FS_BU * LW + l], stg[FS_ZL * LW + l], stg[FS_ZU * LW + l], mu,
-                            df * gradf(k, zk, TRK ? stg[FS_REF * LW + l] : xs_l), sig, gx);
+                sig_g<MB>(kd, zk, stg[FS_BL * LW + l], stg[FS_BU * LW + l], stg[FS_ZL * LW + l], stg[FS_ZU * LW + l], mu,
+                          MODE == 3 ? row(R_GX, k)[l] : df * gradf(k, zk, TRK ? stg[FS_REF * LW + l] : xs_l), sig, gx);
                 dg = sig + delta + zeta;
-                if (MODE == 0) { dg += df * qw; if (isx && comp == 2) dg += thd[rob]; }
+                if (MB == 0) { dg += df * qw; if (isx && comp == 2) dg += thd[rob]; }
             }
             row(R_GX, k)[l] = gx;
             dgx = isx ? dg : 0.0;                                                   // state diagonal is carried lazily
-            if (selfp) *selfp = isu ? dg : (MODE == 0 ? crs[rob] : 0.0);           // control diagonal / theta-v cross term
+            if (selfp) *selfp = isu ? dg : (MB == 0 ? crs[rob] : 0.0);           // control diagonal / theta-v cross term
             tsync();
             if (isz) *hslot = gx + ((rsum_any && isx && comp < 2) ? tt[(3 + comp) * TSZ + rob * (TCOLS + 1)] : 0.0);
             tsync();
@@ -870,8 +875,8 @@ struct WarpSolver {
             double a0, a1, a2, a3, a4;
             QIn in;
             in.lo = brow(NMPC_BR_DL, 0)[l]; in.hi = brow(NMPC_BR_DU, 0)[l]; in.s = row(R_S, 0)[l]; in.vl = row(R_VL, 0)[l]; in.vu = row(R_VU, 0)[l];
-            in.yd = MODE == 0 ? row(R_YD, 0)[l] : 0.0; in.dsoc = soc ? row(R_DSOC, 0)[l] : 0.0;
-            ineq_block<MODE>(row, in, l, pi, pj, isobs, qob, kd, 0, mu, delta, soc, zb, a0, a1, a2, a3, a4);
+            in.yd = MB == 0 ? row(R_YD, 0)[l] : 0.0; in.dsoc = soc ? row(R_DSOC, 0)[l] : 0.0;
+            ineq_block<MB>(row, in, l, pi, pj, isobs, qob, kd, 0, mu, delta, soc, zb, a0, a1, a2, a3, a4);
         }
         tsync();
         return true;
@@ -1235,6 +1240,82 @@ struct WarpSolver {
         if (ftype && theta <= theta_min) ok = cmp_le(ph_t - phi, 1e-8 * alpha_test * gbd, phi);
         else ok = cmp_le(th_t, (1.0 - 1e-5) * theta, theta) || cmp_le(ph_t - phi, -1e-8 * theta, phi);
         return ok && filter_ok(th_t, ph_t);
+    }
+
+    // ---------------------------------------------------------------------------------------
+    // Parametric sensitivity of a returned solution (nmpc_solution_vjp / nmpc_solution_jvp), centralized family only.  The
+    // point (x, lam_x, lam_g) is loaded in place of an iterate, unscaled (df = 1, so the stored multipliers are CasADi's): the
+    // bound multipliers split by sign into zL / zU, the slacks set to the row values at x, block 0's constant rows weighted 0.
+    // factor<3> with mu = delta = 0 then builds K = [[W + Sx, J'], [J, -Ss^-1]] (W = Hessian of the Lagrangian, Sx / Ss the
+    // interior-point weights |lam| / distance to the relaxed bound) and the forward pass solves K [dz; y] = -[g; c] for the
+    // seeded g (R_GX) and c (R_CSOC; R_DSOC = 0: no row depends on p):
+    //   reverse: g = -x_bar, c = 0                     ->  p_bar[x0bar] = y of block 0,  p_bar[ref] = 2Q / 2R times dz
+    //   forward: g = d(grad f)/dp p_dot, c = dg/dp p_dot ->  x_dot = dz
+    // A pivot <= 0 (wrong inertia: second-order sufficiency fails, the derivative is not defined) gives status 1 and NaN.
+    // ---------------------------------------------------------------------------------------
+    NMPC_PASS void sensitivity(const NmpcSensParams &SP)
+    {
+        NMPC_LOCALS
+        static_assert(!OBS, "the obstacle families have no sensitivity pass");
+        const long long n = (long long)NS * S + (long long)NC * N, blk = NS + M, np = TRK ? NS + (long long)N * NZ : 2 * NS;
+        const double *x = SP.x + inst * n, *lx = SP.lam_x + inst * n, *lg = SP.lam_g + inst * (S * blk);
+        const double *sd = SP.seed + inst * (SP.reverse ? n : np);
+        double *out = SP.out + inst * (SP.reverse ? np : n);
+        auto xidx = [=](int k) -> long long { return isx ? (long long)k * NS + l : (long long)NS * S + (long long)k * NC + (l - NS); };
+        const int berr = P.bound_err ? *P.bound_err : 0;
+        bool ok = berr == 0;
+        if (ok) {
+            for (int k = 0; k <= N; k++) {
+                const bool zv = zvalid(k);
+                const double lam = zv ? lx[xidx(k)] : 0.0;
+                row(R_Z, k)[l] = zv ? x[xidx(k)] : 0.0;
+                row(R_ZL, k)[l] = (zv && brow(NMPC_BR_BL, k)[l] > -NMPC_INF) ? fmax(-lam, 0.0) : 0.0;
+                row(R_ZU, k)[l] = (zv && brow(NMPC_BR_BU, k)[l] < NMPC_INF) ? fmax(lam, 0.0) : 0.0;
+                row(R_YC, k)[l] = isx ? lg[k * blk + l] : 0.0;
+                row(R_YD, k)[l] = isq ? lg[k * blk + NS + l] : 0.0;
+                double g = 0.0;
+                if (SP.reverse) g = zv ? -sd[xidx(k)] : 0.0;
+                else if (k < N && isz) g = -qw * (TRK ? sd[NS + k * NZ + l] : (isx ? sd[NS + l] : 0.0));
+                row(R_GX, k)[l] = g;
+                row(R_CSOC, k)[l] = (!SP.reverse && k == 0 && isx) ? -sd[l] : 0.0;
+                row(R_DSOC, k)[l] = 0.0;
+            }
+            tsync();
+            for (int b = 0; b <= N; b++) {
+                double s = NMPC_DUMMY_ROW_VALUE, vl = 0.0, vu = 0.0;
+                if (isq && b > 0) {
+                    const double yd = row(R_YD, b)[l];
+                    s = rowg(row(R_Z, b - 1), pi, pj, false, nullptr).dv;
+                    vl = brow(NMPC_BR_DL, b)[l] > -NMPC_INF ? fmax(-yd, 0.0) : 0.0;
+                    vu = brow(NMPC_BR_DU, b)[l] < NMPC_INF ? fmax(yd, 0.0) : 0.0;
+                }
+                row(R_S, b)[l] = s; row(R_VL, b)[l] = vl; row(R_VU, b)[l] = vu;
+            }
+            tsync();
+            trig_rows(row, l, N, 0.0, 0, false, R_TRIG);
+            this->r_trig = R_TRIG; this->trig_valid = true;
+            ok = factor<3>(0.0, 0.0, true);
+        }
+        if (ok) {
+            StepInfo si;
+            forward(0.0, 1.0, R_DZ, R_DS, R_YTC, R_YTD, si);
+        }
+        const double nan = (double)NAN;
+        if (SP.reverse) {
+            if (isx) out[l] = ok ? row(R_YTC, 0)[l] : nan;
+            double acc = 0.0;
+            for (int k = 0; k < N; k++) {
+                const double a = ok ? row(R_DZ, k)[l] : nan;
+                if (TRK && isz) out[NS + (long long)k * NZ + l] = qw * a;
+                acc += a;
+            }
+            if (!TRK && isx) out[NS + l] = qw * acc;
+        } else {
+            for (int k = 0; k <= N; k++)
+                if (zvalid(k)) out[xidx(k)] = ok ? row(R_DZ, k)[l] : nan;
+        }
+        if (SP.status && l == 0) SP.status[inst] = berr ? berr : (ok ? 0 : 1);
+        tsync();
     }
 
     // ---------------------------------------------------------------------------------------

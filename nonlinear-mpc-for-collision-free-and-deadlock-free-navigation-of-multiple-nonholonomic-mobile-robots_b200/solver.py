@@ -329,6 +329,46 @@ class Problem:
             check(self.L.nmpc_solve(*args, ws.data_ptr(), ws.numel(), stream))
         return o
 
+    # ---- parametric sensitivities of returned solutions (nmpc_solution_vjp / nmpc_solution_jvp) ---------------------------
+    def _sensitivity(self, fn, out, p, lbx, ubx, lbg, ubg, seed, seed_cols, out_cols):
+        torch = self._torch()
+        x, lam_x, lam_g = out["x"], out["lam_x"], out["lam_g"]
+        B, dev = x.shape[0], x.device
+        for t in (x, lam_x, lam_g, p, lbx, ubx, lbg, ubg, seed):
+            if not (t.is_cuda and t.dtype == torch.float64 and t.is_contiguous() and t.device == dev):
+                raise ValueError("inputs must be contiguous float64 CUDA tensors on one device")
+        if tuple(seed.shape) != (B, seed_cols) or tuple(p.shape) != (B, self.np_):
+            raise ValueError("p must be [B, %d] and the seed [B, %d]" % (self.np_, seed_cols))
+        batched = 1 if lbx.dim() == 2 else 0
+        need = int(self.L.nmpc_sensitivity_workspace_bytes(self.h, B, batched))
+        if getattr(self, "_sws", None) is None or self._sws.numel() < need or self._sws.device != dev:
+            self._sws = torch.empty(max(need, 1), dtype=torch.uint8, device=dev)
+        res = torch.empty((B, out_cols), dtype=torch.float64, device=dev)
+        st = torch.empty(B, dtype=torch.int32, device=dev)
+        check(fn(self.h, B, x.data_ptr(), lam_x.data_ptr(), lam_g.data_ptr(), p.data_ptr(), lbx.data_ptr(), ubx.data_ptr(),
+                 lbg.data_ptr(), ubg.data_ptr(), batched, seed.data_ptr(), res.data_ptr(), st.data_ptr(), self._sws.data_ptr(), need,
+                 self._stream(dev)))
+        return res, st
+
+    def solution_vjp(self, out, p, lbx, ubx, lbg, ubg, x_bar):
+        """Reverse-mode derivative of the solution: p_bar [B, np] = x_bar' dx*/dp for x_bar [B, n], at the solutions `out` (the
+        dict solve() returned: x, lam_x, lam_g) of the solve with this p and these bounds.  Returns (p_bar, sens_status):
+        status 0 ok, 1 wrong inertia at the point (p_bar is NaN there), < 0 bounds rejected.  See nmpc_solution_vjp."""
+        return self._sensitivity(self.L.nmpc_solution_vjp, out, p, lbx, ubx, lbg, ubg, x_bar, self.n, self.np_)
+
+    def solution_jvp(self, out, p, lbx, ubx, lbg, ubg, p_dot):
+        """Forward-mode derivative of the solution: x_dot [B, n] = dx*/dp p_dot for p_dot [B, np]; (x_dot, sens_status) as in
+        solution_vjp.  x + x_dot is the first-order prediction of the solution at p + p_dot (the sensitivity correction of an
+        advanced-step controller)."""
+        return self._sensitivity(self.L.nmpc_solution_jvp, out, p, lbx, ubx, lbg, ubg, p_dot, self.np_, self.n)
+
+    def solve_differentiable(self, x0, p, lbx, ubx, lbg, ubg):
+        """solve() as a torch.autograd function of p: returns x [B, n]; x.backward / torch.autograd.grad give the gradient with
+        respect to p through nmpc_solution_vjp at the returned solutions.  x0 and the bounds get no gradient (x* does not depend
+        on the start point; derivatives with respect to the bounds are not provided).  An instance whose solve did not converge
+        gets the derivative of its returned point all the same; one with the wrong inertia there gets NaN."""
+        return _solve_function().apply(self, x0, p, lbx, ubx, lbg, ubg)
+
     def set_order(self, order=None):
         """Scheduling hint (nmpc_set_order): int32 CUDA tensor [B], a permutation of the instances, longest expected solve
         first; None restores index order.  The tensor is kept alive by the handle."""
@@ -369,6 +409,35 @@ class Problem:
         check(self.L.nmpc_eval(self.h, B, w.data_ptr(), p.data_ptr(), lam_g.data_ptr() if lam_g is not None else None,
                                ptr("f"), ptr("grad"), ptr("g"), ptr("jac"), ptr("hess"), self._stream(dev)))
         return o
+
+
+_SOLVE_FUNCTION = None
+
+
+def _solve_function():
+    """The torch.autograd.Function behind Problem.solve_differentiable (built on first use: torch is imported lazily)."""
+    global _SOLVE_FUNCTION
+    if _SOLVE_FUNCTION is None:
+        import torch
+
+        class SolveFunction(torch.autograd.Function):
+            @staticmethod
+            def forward(ctx, prob, x0, p, lbx, ubx, lbg, ubg):
+                out = prob.solve(x0, p.detach(), lbx, ubx, lbg, ubg, want=("lam_x", "lam_g"))
+                ctx.prob = prob
+                ctx.save_for_backward(p.detach(), lbx, ubx, lbg, ubg, out["x"], out["lam_x"], out["lam_g"])
+                return out["x"]
+
+            @staticmethod
+            @torch.autograd.function.once_differentiable
+            def backward(ctx, x_bar):
+                p, lbx, ubx, lbg, ubg, x, lam_x, lam_g = ctx.saved_tensors
+                p_bar, _ = ctx.prob.solution_vjp(dict(x=x, lam_x=lam_x, lam_g=lam_g), p, lbx, ubx, lbg, ubg,
+                                                 x_bar.to(torch.float64).contiguous())
+                return None, None, p_bar, None, None, None, None
+
+        _SOLVE_FUNCTION = SolveFunction
+    return _SOLVE_FUNCTION
 
 
 def closed_loop(prob, P, lbx, ubx, lbg, ubg, steps, tol=1e-1, dmin=None, obstacles=None, reference=None):

@@ -6,7 +6,8 @@ Extracts the sm_100a cubin of both libraries (cuobjdump -xelf), disassembles it 
 its functions: the kernel body and each device function it calls (the solver's noinline passes).  Instruction addresses and
 encodings are stripped, return addresses loaded into registers are made relative to their function, branch labels are
 renumbered within each function, and the compiler's numbering of specialised
-copies (`_$_specialized_$_N`) is dropped, so that two builds compare equal when every function has the same instructions,
+copies (`_$_specialized_$_N`) and of the CUDA math helpers (`__internal_N_$__cuda_sm20_div_rn_f64_full`, numbered in the order
+the file's kernels use them, so a kernel added to the file renumbers them everywhere) is dropped, so that two builds compare equal when every function has the same instructions,
 wherever the linker placed it.  Kernel and function names are compared with a trailing `false` template argument removed, so
 that WarpSolver<NR, OBS> / solve_kernel<NR, OBS> of an older build pair with <NR, OBS, false> of a newer one.
 REGEX selects kernels by mangled name (default: the warp-path solve kernels without the tracking flag, solve_kernel<1..10,
@@ -23,6 +24,7 @@ DEFAULT = r"^_Z12solve_kernelILi\d+ELb[01]EEv15NmpcSolveParams$"
 
 def _norm(name):
     name = re.sub(r"(ILi\d+ELb[01])ELb0EE", r"\1EE", name)
+    name = re.sub(r"__internal_\d+_", "__internal_", name)
     return re.sub(r"_\$_specialized_\$_\d+", "_$_specialized", name)
 
 
