@@ -234,8 +234,28 @@ int nmpc_solution_jvp(nmpc_handle *h, int B, const double *x, const double *lam_
                       const double *lbx, const double *ubx, const double *lbg, const double *ubg, int bounds_batched,
                       const double *p_dot, double *x_dot, int32_t *sens_status, void *workspace, size_t workspace_bytes,
                       void *stream);
-/* Device scratch of both calls (0 for an unsupported handle or B <= 0). */
+/* Device scratch of both calls and of nmpc_solution_x0_jacobian (0 for an unsupported handle or B <= 0). */
 size_t nmpc_sensitivity_workspace_bytes(const nmpc_handle *h, int B, int bounds_batched);
+
+/* Advanced-step NMPC (asNMPC, Zavala & Biegler 2009): solve for a predicted initial state x0bar = p[0:3Nr] while the system
+ * moves (preparation), then, once the state is measured, correct that solution to first order in one cheap launch (feedback).
+ * nmpc_solution_x0_jacobian: jac [B][3Nr][n] (DEVICE), jac[b][j] = (dx* / dp) e_j, j < 3Nr -- exactly what
+ *     nmpc_solution_jvp returns for that seed (same layout as x, X_0 rows = e_j).  One factorisation of K per instance and 3Nr
+ *     forward passes; inputs, sens_status, workspace (nmpc_sensitivity_workspace_bytes), supported handles and error codes as
+ *     nmpc_solution_jvp.
+ * nmpc_advanced_step: x_corr [B,n] = x + sum_j jac[j] (x0bar_meas - p[0:3Nr])_j (x0bar_meas [B][3Nr], summed in order
+ *     j = 0..3Nr-1); a variable with a finite bound is then clamped to [min(lbx_i, x_i), max(ubx_i, x_i)] (never pulled further
+ *     outside a bound the solve left it just beyond); the X_0 rows are x0bar_meas exactly; an instance with sens_status != 0
+ *     keeps x (X_0 = x0bar_meas).  Collision rows are not projected: the correction is first order, the next solve restores
+ *     them.  lbx / ubx [n] or [B,n] (bounds_batched); all pointers DEVICE and non-NULL.  One launch, asynchronous on stream;
+ *     supported handles and error codes as nmpc_solution_jvp (no workspace).
+ * Both calls leave the handle's state unchanged. */
+int nmpc_solution_x0_jacobian(nmpc_handle *h, int B, const double *x, const double *lam_x, const double *lam_g, const double *p,
+                              const double *lbx, const double *ubx, const double *lbg, const double *ubg, int bounds_batched,
+                              double *jac, int32_t *sens_status, void *workspace, size_t workspace_bytes, void *stream);
+int nmpc_advanced_step(nmpc_handle *h, int B, const double *x, const double *jac, const int32_t *sens_status, const double *p,
+                       const double *x0bar_meas, const double *lbx, const double *ubx, int bounds_batched, double *x_corr,
+                       void *stream);
 
 /* Same call with HOST buffers (what a CasADi-style caller has): H2D of the inputs, solve, D2H of
  * the requested outputs, synchronous.  Staging buffers live in the handle and grow on demand. */

@@ -8,6 +8,7 @@
 //   K4  shift_kernel  -- warm-start shift of the MPC loop (shift() :160-169 and the X0 line :465)
 //       plant_kernel  -- Euler plant (casadi_test.py:17-26)
 //       prep_bounds_kernel -- flat lbx/ubx/lbg/ubg (:349-352) -> relaxed stage-layout rows
+//       advanced_step_kernel -- first-order correction of a solution for the measured state (nmpc_advanced_step)
 #pragma once
 #include "bounds_prep.cuh"
 #include "nmpc_internal.h"
@@ -309,5 +310,33 @@ __global__ void prep_bounds_kernel(int Nr, int N, double relax, int nb, int lw, 
         const int k = (int)((e / lw) % S), lane = (int)(e % lw);
         int rc = nmpc_prep_bounds_elem(Nr, N, relax, lbx + b * n, ubx + b * n, lbg + b * mg, ubg + b * mg, k, lane, lw, rows + b * bstride, nobs, family, stage_major);
         if (rc) atomicCAS(err, 0, rc);
+    }
+}
+
+// Advanced-step feedback (nmpc_advanced_step): x_corr = x + jac' (x0bar_meas - p[0:ns]) per instance, one thread per (instance,
+// variable), jac [B][ns][n] read coalesced along n; the sum runs over j = 0..ns-1 in order.  A variable with a finite bound is
+// clamped to [min(lb, x), max(ub, x)], so a component the solve left just outside its bound (bound_relax_factor) is never pulled
+// further; the X_0 rows are x0bar_meas exactly.  An instance with sens_status != 0 keeps x (X_0 = x0bar_meas all the same).
+__global__ void __launch_bounds__(256) advanced_step_kernel(int ns, int n, int np, long long total, const double *__restrict__ x,
+                                                            const double *__restrict__ jac, const int *__restrict__ sens_status,
+                                                            const double *__restrict__ p, const double *__restrict__ x0m,
+                                                            const double *__restrict__ lbx, const double *__restrict__ ubx,
+                                                            long long bstride, double *__restrict__ xc)
+{
+    for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < total; e += (long long)gridDim.x * blockDim.x) {
+        const long long b = e / n;
+        const int i = (int)(e - b * n);
+        const double *meas = x0m + b * ns;
+        if (i < ns) { xc[e] = meas[i]; continue; }
+        const double xi = x[e];
+        if (sens_status[b] != 0) { xc[e] = xi; continue; }
+        const double *jb = jac + b * ns * n + i, *pb = p + b * np;
+        double s = 0.0;
+        for (int j = 0; j < ns; j++) s = fma(jb[(long long)j * n], meas[j] - pb[j], s);
+        double v = xi + s;
+        const double lb = lbx[b * bstride + i], ub = ubx[b * bstride + i];
+        if (lb > -NMPC_INF) v = fmax(v, fmin(lb, xi));
+        if (ub < NMPC_INF) v = fmin(v, fmax(ub, xi));
+        xc[e] = v;
     }
 }

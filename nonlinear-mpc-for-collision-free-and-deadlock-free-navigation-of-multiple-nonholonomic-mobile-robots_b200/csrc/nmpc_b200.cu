@@ -114,6 +114,22 @@ __global__ void __launch_bounds__((SolveCfg<NR, false, TRK>::THREADS), (SolveCfg
     }
 }
 
+// Jacobian of the solution with respect to x0bar (nmpc_solution_x0_jacobian): sens_kernel's layout, launch and scratch
+template <int NR, bool TRK>
+__global__ void __launch_bounds__((SolveCfg<NR, false, TRK>::THREADS), (SolveCfg<NR, false, TRK>::MIN_CTAS)) sens_x0_kernel(const NmpcSolveParams P, const NmpcSensParams S)
+{
+    extern __shared__ double smem[];
+    typedef WarpSolver<NR, false, TRK> WSol;
+    typedef SolveCfg<NR, false, TRK> Cfg;
+    const int team = threadIdx.x / Cfg::LW;
+    WSol s(P, smem + (size_t)team * WSol::SM_DOUBLES, P.ws + ((long long)blockIdx.x * Cfg::TEAMS + team) * P.ws_stride);
+    s.init_team();
+    for (int inst = blockIdx.x * Cfg::TEAMS + team; inst < P.B; inst += gridDim.x * Cfg::TEAMS) {
+        s.setup(inst);
+        s.sensitivity_x0(S);
+    }
+}
+
 struct nmpc_handle {
     nmpc_desc d;
     nmpc_opts o;
@@ -139,6 +155,7 @@ struct nmpc_handle {
     bool block_path, eval_ok;                 // Nr > 10: CTA-per-instance dense-block solver; eval record fits shared memory
     int *d_pairs;                             // pair table (i, j) of the inequality rows, block path
     bool sens_smem_set;                       // sens_kernel's shared-memory attribute is set (first sensitivity call)
+    bool sens_x0_smem_set;                    // ... and sens_x0_kernel's (first nmpc_solution_x0_jacobian call)
     // host-pointer API staging
     char *d_buf;
     size_t d_bytes;
@@ -610,14 +627,16 @@ static int sens_grid(const nmpc_handle *h, int B)
 template <int NR, bool TRK> struct SensLaunch {
     static size_t slot_doubles(int N) { return (size_t)WarpSolver<NR, false, TRK>::ws_doubles(N); }
     static size_t smem() { return (size_t)SolveCfg<NR, false, TRK>::TEAMS * WarpSolver<NR, false, TRK>::SM_DOUBLES * sizeof(double); }
-    static cudaError_t run(nmpc_handle *h, int grid, const NmpcSolveParams &P, const NmpcSensParams &S, cudaStream_t st)
+    static cudaError_t run(nmpc_handle *h, int grid, const NmpcSolveParams &P, const NmpcSensParams &S, cudaStream_t st, bool x0)
     {
-        if (!h->sens_smem_set) {
-            cudaError_t e = cudaFuncSetAttribute(sens_kernel<NR, TRK>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem());
+        auto kern = x0 ? sens_x0_kernel<NR, TRK> : sens_kernel<NR, TRK>;
+        bool &smem_set = x0 ? h->sens_x0_smem_set : h->sens_smem_set;
+        if (!smem_set) {
+            cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem());
             if (e != cudaSuccess) return e;
-            h->sens_smem_set = true;
+            smem_set = true;
         }
-        sens_kernel<NR, TRK><<<grid, SolveCfg<NR, false, TRK>::THREADS, smem(), st>>>(P, S);
+        kern<<<grid, SolveCfg<NR, false, TRK>::THREADS, smem(), st>>>(P, S);
         return cudaGetLastError();
     }
 };
@@ -647,9 +666,9 @@ static size_t sens_slot_doubles(const nmpc_handle *h)
 {
     return sens_dispatch(h, [&](auto nr, auto trk) { return SensLaunch<decltype(nr)::value, decltype(trk)::value>::slot_doubles(h->d.N); });
 }
-static cudaError_t sens_launch(nmpc_handle *h, int grid, const NmpcSolveParams &P, const NmpcSensParams &S, cudaStream_t st)
+static cudaError_t sens_launch(nmpc_handle *h, int grid, const NmpcSolveParams &P, const NmpcSensParams &S, cudaStream_t st, bool x0)
 {
-    return sens_dispatch(h, [&](auto nr, auto trk) { return SensLaunch<decltype(nr)::value, decltype(trk)::value>::run(h, grid, P, S, st); });
+    return sens_dispatch(h, [&](auto nr, auto trk) { return SensLaunch<decltype(nr)::value, decltype(trk)::value>::run(h, grid, P, S, st, x0); });
 }
 static int sens_supported(const nmpc_handle *h, const char *fn)
 {
@@ -657,6 +676,15 @@ static int sens_supported(const nmpc_handle *h, const char *fn)
     if (h->family == 2) return fail(NMPC_ENOTSUP, "%s: not available for the small-OCP family", fn);
     if (h->family == 1) return fail(NMPC_ENOTSUP, "%s: not available for the obstacle families (static, moving, tracking among obstacles)", fn);
     if (h->d.Nr > 10) return fail(NMPC_ENOTSUP, "%s: Nr = %d; supported: 1..10 robots", fn, h->d.Nr);
+    return 0;
+}
+// after the NULL-argument check: B and the current device
+static int sens_batch_device(const nmpc_handle *h, int B, const char *fn)
+{
+    if (B <= 0) return fail(NMPC_EINVAL, "%s: B must be positive", fn);
+    int cur = -1;
+    if (cudaGetDevice(&cur) != cudaSuccess || cur != h->dev)
+        return fail(NMPC_EINVAL, "%s: the handle was created on CUDA device %d but device %d is current", fn, h->dev, cur);
     return 0;
 }
 static size_t sens_ws_bytes(const nmpc_handle *h, int B, int nb)
@@ -671,20 +699,16 @@ extern "C" size_t nmpc_sensitivity_workspace_bytes(const nmpc_handle *h, int B, 
     return sens_ws_bytes(h, B, bounds_batched ? B : 1);
 }
 
+enum { SENS_JVP, SENS_VJP, SENS_X0 };
 static int sens_impl(const char *fn, nmpc_handle *h, int B, const double *x, const double *lam_x, const double *lam_g, const double *p,
                      const double *lbx, const double *ubx, const double *lbg, const double *ubg, int bounds_batched, const double *seed,
-                     double *out, int32_t *status, void *workspace, size_t workspace_bytes, cudaStream_t st, int reverse)
+                     double *out, int32_t *status, void *workspace, size_t workspace_bytes, cudaStream_t st, int mode)
 {
     int rc = sens_supported(h, fn);
     if (rc) return rc;
-    if (!x || !lam_x || !lam_g || !p || !lbx || !ubx || !lbg || !ubg || !seed || !out || !workspace)
+    if (!x || !lam_x || !lam_g || !p || !lbx || !ubx || !lbg || !ubg || (!seed && mode != SENS_X0) || !out || !workspace)
         return fail(NMPC_EINVAL, "%s: NULL argument", fn);
-    if (B <= 0) return fail(NMPC_EINVAL, "%s: B must be positive", fn);
-    {
-        int cur = -1;
-        if (cudaGetDevice(&cur) != cudaSuccess || cur != h->dev)
-            return fail(NMPC_EINVAL, "%s: the handle was created on CUDA device %d but device %d is current", fn, h->dev, cur);
-    }
+    if ((rc = sens_batch_device(h, B, fn))) return rc;
     const int nb = bounds_batched ? B : 1, lw = sens_lw(h);
     const size_t need = sens_ws_bytes(h, B, nb);
     if (workspace_bytes < need) return fail(NMPC_EINVAL, "%s: workspace %zu B < %zu B required (nmpc_sensitivity_workspace_bytes)", fn, workspace_bytes, need);
@@ -708,8 +732,8 @@ static int sens_impl(const char *fn, nmpc_handle *h, int B, const double *x, con
     P.ws = (double *)(base + 256 + (size_t)nb * NMPC_BR_COUNT * h->S * lw * sizeof(double));
     P.ws_stride = (long long)sens_slot_doubles(h);
     NmpcSensParams S;
-    S.x = x; S.lam_x = lam_x; S.lam_g = lam_g; S.seed = seed; S.out = out; S.status = status; S.reverse = reverse;
-    cudaError_t e = sens_launch(h, sens_grid(h, B), P, S, st);
+    S.x = x; S.lam_x = lam_x; S.lam_g = lam_g; S.seed = seed; S.out = out; S.status = status; S.reverse = mode == SENS_VJP;
+    cudaError_t e = sens_launch(h, sens_grid(h, B), P, S, st, mode == SENS_X0);
     h->launches++;
     if (e != cudaSuccess) return fail(NMPC_ECUDA, "%s: launch failed: %s", fn, cudaGetErrorString(e));
     return 0;
@@ -721,7 +745,7 @@ extern "C" int nmpc_solution_vjp(nmpc_handle *h, int B, const double *x, const d
                                  void *stream)
 {
     return sens_impl("nmpc_solution_vjp", h, B, x, lam_x, lam_g, p, lbx, ubx, lbg, ubg, bounds_batched, x_bar, p_bar, sens_status,
-                     workspace, workspace_bytes, (cudaStream_t)stream, 1);
+                     workspace, workspace_bytes, (cudaStream_t)stream, SENS_VJP);
 }
 
 extern "C" int nmpc_solution_jvp(nmpc_handle *h, int B, const double *x, const double *lam_x, const double *lam_g, const double *p,
@@ -730,7 +754,35 @@ extern "C" int nmpc_solution_jvp(nmpc_handle *h, int B, const double *x, const d
                                  void *stream)
 {
     return sens_impl("nmpc_solution_jvp", h, B, x, lam_x, lam_g, p, lbx, ubx, lbg, ubg, bounds_batched, p_dot, x_dot, sens_status,
-                     workspace, workspace_bytes, (cudaStream_t)stream, 0);
+                     workspace, workspace_bytes, (cudaStream_t)stream, SENS_JVP);
+}
+
+extern "C" int nmpc_solution_x0_jacobian(nmpc_handle *h, int B, const double *x, const double *lam_x, const double *lam_g,
+                                         const double *p, const double *lbx, const double *ubx, const double *lbg, const double *ubg,
+                                         int bounds_batched, double *jac, int32_t *sens_status, void *workspace,
+                                         size_t workspace_bytes, void *stream)
+{
+    return sens_impl("nmpc_solution_x0_jacobian", h, B, x, lam_x, lam_g, p, lbx, ubx, lbg, ubg, bounds_batched, nullptr, jac,
+                     sens_status, workspace, workspace_bytes, (cudaStream_t)stream, SENS_X0);
+}
+
+extern "C" int nmpc_advanced_step(nmpc_handle *h, int B, const double *x, const double *jac, const int32_t *sens_status,
+                                  const double *p, const double *x0bar_meas, const double *lbx, const double *ubx, int bounds_batched,
+                                  double *x_corr, void *stream)
+{
+    const char *fn = "nmpc_advanced_step";
+    int rc = sens_supported(h, fn);
+    if (rc) return rc;
+    if (!x || !jac || !sens_status || !p || !x0bar_meas || !lbx || !ubx || !x_corr) return fail(NMPC_EINVAL, "%s: NULL argument", fn);
+    if ((rc = sens_batch_device(h, B, fn))) return rc;
+    const long long total = (long long)B * h->n;
+    const int blocks = (int)std::min<long long>((total + 255) / 256, (long long)h->sm_count * 8);
+    advanced_step_kernel<<<blocks, 256, 0, (cudaStream_t)stream>>>(h->ns, h->n, h->np, total, x, jac, sens_status, p, x0bar_meas,
+                                                                    lbx, ubx, bounds_batched ? h->n : 0, x_corr);
+    h->launches++;
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return fail(NMPC_ECUDA, "%s: launch failed: %s", fn, cudaGetErrorString(e));
+    return 0;
 }
 
 static size_t al(size_t v) { return (v + 255) & ~(size_t)255; }

@@ -1253,17 +1253,16 @@ struct WarpSolver {
     //   forward: g = d(grad f)/dp p_dot, c = dg/dp p_dot ->  x_dot = dz
     // A pivot <= 0 (wrong inertia: second-order sufficiency fails, the derivative is not defined) gives status 1 and NaN.
     // ---------------------------------------------------------------------------------------
-    NMPC_PASS void sensitivity(const NmpcSensParams &SP)
+    // the point (and, SEEDED, the seeds of sensitivity()) loaded in place of an iterate, then factor<3>; false when the bounds were
+    // rejected (ok = false on entry) or a pivot is <= 0.  Unseeded, R_GX and R_CSOC are zero: K is the same, the right-hand side 0.
+    template <bool SEEDED>
+    NMPC_DEV bool sens_factor(const NmpcSensParams &SP, bool ok)
     {
         NMPC_LOCALS
-        static_assert(!OBS, "the obstacle families have no sensitivity pass");
         const long long n = (long long)NS * S + (long long)NC * N, blk = NS + M, np = TRK ? NS + (long long)N * NZ : 2 * NS;
         const double *x = SP.x + inst * n, *lx = SP.lam_x + inst * n, *lg = SP.lam_g + inst * (S * blk);
-        const double *sd = SP.seed + inst * (SP.reverse ? n : np);
-        double *out = SP.out + inst * (SP.reverse ? np : n);
+        const double *sd = SEEDED ? SP.seed + inst * (SP.reverse ? n : np) : nullptr;
         auto xidx = [=](int k) -> long long { return isx ? (long long)k * NS + l : (long long)NS * S + (long long)k * NC + (l - NS); };
-        const int berr = P.bound_err ? *P.bound_err : 0;
-        bool ok = berr == 0;
         if (ok) {
             for (int k = 0; k <= N; k++) {
                 const bool zv = zvalid(k);
@@ -1274,10 +1273,12 @@ struct WarpSolver {
                 row(R_YC, k)[l] = isx ? lg[k * blk + l] : 0.0;
                 row(R_YD, k)[l] = isq ? lg[k * blk + NS + l] : 0.0;
                 double g = 0.0;
-                if (SP.reverse) g = zv ? -sd[xidx(k)] : 0.0;
-                else if (k < N && isz) g = -qw * (TRK ? sd[NS + k * NZ + l] : (isx ? sd[NS + l] : 0.0));
+                if (SEEDED) {
+                    if (SP.reverse) g = zv ? -sd[xidx(k)] : 0.0;
+                    else if (k < N && isz) g = -qw * (TRK ? sd[NS + k * NZ + l] : (isx ? sd[NS + l] : 0.0));
+                }
                 row(R_GX, k)[l] = g;
-                row(R_CSOC, k)[l] = (!SP.reverse && k == 0 && isx) ? -sd[l] : 0.0;
+                row(R_CSOC, k)[l] = (SEEDED && !SP.reverse && k == 0 && isx) ? -sd[l] : 0.0;
                 row(R_DSOC, k)[l] = 0.0;
             }
             tsync();
@@ -1296,6 +1297,18 @@ struct WarpSolver {
             this->r_trig = R_TRIG; this->trig_valid = true;
             ok = factor<3>(0.0, 0.0, true);
         }
+        return ok;
+    }
+
+    NMPC_PASS void sensitivity(const NmpcSensParams &SP)
+    {
+        NMPC_LOCALS
+        static_assert(!OBS, "the obstacle families have no sensitivity pass");
+        const long long n = (long long)NS * S + (long long)NC * N, np = TRK ? NS + (long long)N * NZ : 2 * NS;
+        double *out = SP.out + inst * (SP.reverse ? np : n);
+        auto xidx = [=](int k) -> long long { return isx ? (long long)k * NS + l : (long long)NS * S + (long long)k * NC + (l - NS); };
+        const int berr = P.bound_err ? *P.bound_err : 0;
+        const bool ok = sens_factor<true>(SP, berr == 0);
         if (ok) {
             StepInfo si;
             forward(0.0, 1.0, R_DZ, R_DS, R_YTC, R_YTD, si);
@@ -1311,6 +1324,37 @@ struct WarpSolver {
             }
             if (!TRK && isx) out[NS + l] = qw * acc;
         } else {
+            for (int k = 0; k <= N; k++)
+                if (zvalid(k)) out[xidx(k)] = ok ? row(R_DZ, k)[l] : nan;
+        }
+        if (SP.status && l == 0) SP.status[inst] = berr ? berr : (ok ? 0 : 1);
+        tsync();
+    }
+
+    // ---------------------------------------------------------------------------------------
+    // Jacobian of the solution with respect to the measured state x0bar = p[0:NS] (nmpc_solution_x0_jacobian): column j is
+    // sensitivity()'s forward mode for p_dot = e_j.  That seed enters only through c of block 0 (R_CSOC row 0, which factor<3>
+    // copies to R_RC row 0 after the sweep and nothing in the sweep reads): with zero seeds the factorisation, its feed-forward
+    // terms and the block-0 rows are those of every column, so the point is factored once and each column is one forward pass
+    // started from R_RC row 0 = -e_j.  Output SP.out: jac [B][NS][n], column j in x's layout (its X_0 rows are e_j); status and
+    // NaN outputs as in sensitivity().
+    // ---------------------------------------------------------------------------------------
+    NMPC_PASS void sensitivity_x0(const NmpcSensParams &SP)
+    {
+        NMPC_LOCALS
+        const long long n = (long long)NS * S + (long long)NC * N;
+        double *jac = SP.out + inst * (NS * n);
+        auto xidx = [=](int k) -> long long { return isx ? (long long)k * NS + l : (long long)NS * S + (long long)k * NC + (l - NS); };
+        const int berr = P.bound_err ? *P.bound_err : 0;
+        const bool ok = sens_factor<false>(SP, berr == 0);
+        const double nan = (double)NAN;
+        for (int j = 0; j < NS; j++) {
+            if (ok) {
+                if (isx) row(R_RC, 0)[l] = -(l == j ? 1.0 : 0.0);
+                StepInfo si;
+                forward(0.0, 1.0, R_DZ, R_DS, R_YTC, R_YTD, si);
+            }
+            double *out = jac + j * n;
             for (int k = 0; k <= N; k++)
                 if (zvalid(k)) out[xidx(k)] = ok ? row(R_DZ, k)[l] : nan;
         }

@@ -330,23 +330,25 @@ class Problem:
         return o
 
     # ---- parametric sensitivities of returned solutions (nmpc_solution_vjp / nmpc_solution_jvp) ---------------------------
-    def _sensitivity(self, fn, out, p, lbx, ubx, lbg, ubg, seed, seed_cols, out_cols):
+    def _sensitivity(self, fn, out, p, lbx, ubx, lbg, ubg, seed, seed_cols, out_shape):
+        """seed None: the seedless call (nmpc_solution_x0_jacobian)."""
         torch = self._torch()
         x, lam_x, lam_g = out["x"], out["lam_x"], out["lam_g"]
         B, dev = x.shape[0], x.device
-        for t in (x, lam_x, lam_g, p, lbx, ubx, lbg, ubg, seed):
+        for t in (x, lam_x, lam_g, p, lbx, ubx, lbg, ubg) + (() if seed is None else (seed,)):
             if not (t.is_cuda and t.dtype == torch.float64 and t.is_contiguous() and t.device == dev):
                 raise ValueError("inputs must be contiguous float64 CUDA tensors on one device")
-        if tuple(seed.shape) != (B, seed_cols) or tuple(p.shape) != (B, self.np_):
+        if (seed is not None and tuple(seed.shape) != (B, seed_cols)) or tuple(p.shape) != (B, self.np_):
             raise ValueError("p must be [B, %d] and the seed [B, %d]" % (self.np_, seed_cols))
         batched = 1 if lbx.dim() == 2 else 0
         need = int(self.L.nmpc_sensitivity_workspace_bytes(self.h, B, batched))
         if getattr(self, "_sws", None) is None or self._sws.numel() < need or self._sws.device != dev:
             self._sws = torch.empty(max(need, 1), dtype=torch.uint8, device=dev)
-        res = torch.empty((B, out_cols), dtype=torch.float64, device=dev)
+        res = torch.empty((B,) + tuple(out_shape), dtype=torch.float64, device=dev)
         st = torch.empty(B, dtype=torch.int32, device=dev)
+        seed_arg = () if seed is None else (seed.data_ptr(),)
         check(fn(self.h, B, x.data_ptr(), lam_x.data_ptr(), lam_g.data_ptr(), p.data_ptr(), lbx.data_ptr(), ubx.data_ptr(),
-                 lbg.data_ptr(), ubg.data_ptr(), batched, seed.data_ptr(), res.data_ptr(), st.data_ptr(), self._sws.data_ptr(), need,
+                 lbg.data_ptr(), ubg.data_ptr(), batched, *seed_arg, res.data_ptr(), st.data_ptr(), self._sws.data_ptr(), need,
                  self._stream(dev)))
         return res, st
 
@@ -354,13 +356,40 @@ class Problem:
         """Reverse-mode derivative of the solution: p_bar [B, np] = x_bar' dx*/dp for x_bar [B, n], at the solutions `out` (the
         dict solve() returned: x, lam_x, lam_g) of the solve with this p and these bounds.  Returns (p_bar, sens_status):
         status 0 ok, 1 wrong inertia at the point (p_bar is NaN there), < 0 bounds rejected.  See nmpc_solution_vjp."""
-        return self._sensitivity(self.L.nmpc_solution_vjp, out, p, lbx, ubx, lbg, ubg, x_bar, self.n, self.np_)
+        return self._sensitivity(self.L.nmpc_solution_vjp, out, p, lbx, ubx, lbg, ubg, x_bar, self.n, (self.np_,))
 
     def solution_jvp(self, out, p, lbx, ubx, lbg, ubg, p_dot):
         """Forward-mode derivative of the solution: x_dot [B, n] = dx*/dp p_dot for p_dot [B, np]; (x_dot, sens_status) as in
         solution_vjp.  x + x_dot is the first-order prediction of the solution at p + p_dot (the sensitivity correction of an
         advanced-step controller)."""
-        return self._sensitivity(self.L.nmpc_solution_jvp, out, p, lbx, ubx, lbg, ubg, p_dot, self.np_, self.n)
+        return self._sensitivity(self.L.nmpc_solution_jvp, out, p, lbx, ubx, lbg, ubg, p_dot, self.np_, (self.n,))
+
+    # ---- advanced-step NMPC (nmpc_solution_x0_jacobian / nmpc_advanced_step) ------------------------------------------------
+    def solution_x0_jacobian(self, out, p, lbx, ubx, lbg, ubg):
+        """Jacobian of the solutions `out` (x, lam_x, lam_g of the solve with this p and these bounds) with respect to the
+        initial state x0bar = p[:, :3Nr]: (jac [B, 3Nr, n], sens_status).  jac[b, j] is solution_jvp's x_dot for p_dot = e_j;
+        one factorisation per instance.  The preparation phase of an advanced-step controller."""
+        return self._sensitivity(self.L.nmpc_solution_x0_jacobian, out, p, lbx, ubx, lbg, ubg, None, 0, (self.ns, self.n))
+
+    def advanced_step(self, out, jac, sens_status, p, x0bar_meas, lbx, ubx):
+        """Feedback phase of an advanced-step controller, one launch: x_corr [B, n] = x + jac' (x0bar_meas - p[:, :3Nr]) for the
+        measured states x0bar_meas [B, 3Nr], clamped into the variable bounds (never further out than x), X_0 = x0bar_meas;
+        instances with sens_status != 0 keep x.  See nmpc_advanced_step."""
+        torch = self._torch()
+        x = out["x"]
+        B, dev = x.shape[0], x.device
+        for t in (x, jac, p, x0bar_meas, lbx, ubx):
+            if not (t.is_cuda and t.dtype == torch.float64 and t.is_contiguous() and t.device == dev):
+                raise ValueError("inputs must be contiguous float64 CUDA tensors on one device")
+        if tuple(jac.shape) != (B, self.ns, self.n) or tuple(x0bar_meas.shape) != (B, self.ns) or tuple(p.shape) != (B, self.np_):
+            raise ValueError("jac must be [B, %d, %d], x0bar_meas [B, %d] and p [B, %d]" % (self.ns, self.n, self.ns, self.np_))
+        if not (sens_status.is_cuda and sens_status.dtype == torch.int32 and tuple(sens_status.shape) == (B,)):
+            raise ValueError("sens_status must be an int32 CUDA tensor [B]")
+        xc = torch.empty_like(x)
+        check(self.L.nmpc_advanced_step(self.h, B, x.data_ptr(), jac.data_ptr(), sens_status.contiguous().data_ptr(), p.data_ptr(),
+                                        x0bar_meas.data_ptr(), lbx.data_ptr(), ubx.data_ptr(), 1 if lbx.dim() == 2 else 0,
+                                        xc.data_ptr(), self._stream(dev)))
+        return xc
 
     def solve_differentiable(self, x0, p, lbx, ubx, lbg, ubg):
         """solve() as a torch.autograd function of p: returns x [B, n]; x.backward / torch.autograd.grad give the gradient with
@@ -440,7 +469,8 @@ def _solve_function():
     return _SOLVE_FUNCTION
 
 
-def closed_loop(prob, P, lbx, ubx, lbg, ubg, steps, tol=1e-1, dmin=None, obstacles=None, reference=None):
+def closed_loop(prob, P, lbx, ubx, lbg, ubg, steps, tol=1e-1, dmin=None, obstacles=None, reference=None, disturbance=None,
+                advanced_step=False):
     """Batched closed-loop driver, device resident (SURVEY.md 8f-1): the reference's loop body
     (centralized_six_robots_implementation.py:416-465 with the Euler plant of casadi_test.py:17-26) for B
     independent instances at once.  Per step: solve -> apply u_0 through the plant -> reference shift as the next
@@ -455,9 +485,23 @@ def closed_loop(prob, P, lbx, ubx, lbg, ubg, steps, tol=1e-1, dmin=None, obstacl
     no stop test (every instance is active at every step), and the result gains track_err [steps+1, B] = the largest xy distance
     over robots between the plant state and the reference state at the same time.
     Problem(tracking_obstacles=n_obs) requires both: step t solves with Z = reference rows t..t+N-1 and O = obstacle tables
-    t..t+N-1 (P then needs only x0bar), without a stop test, and the result carries both track_err and min_clearance."""
+    t..t+N-1 (P then needs only x0bar), without a stop test, and the result carries both track_err and min_clearance.
+    disturbance: CUDA float64 [steps, B, 3Nr], added to the plant's next state of the active instances at every step (process
+    noise or model mismatch; every family).
+    advanced_step=True (handles of nmpc_create / nmpc_create_tracking with 1..10 robots): advanced-step NMPC.  Step t solves at
+    the prediction xp_t = plant(x_{t-1}, u_{t-1}) (xp_0 = x_0), prepares the solution's Jacobian in x0bar
+    (Problem.solution_x0_jacobian), corrects the solution for the true state x_t = xp_t + w_{t-1} (Problem.advanced_step) and
+    applies U_0 of the corrected solution, whose shift is the next warm start; the stop test reads the true state.  The result
+    gains u_pred [steps, B, 2Nr] (U_0 before the correction) and sens_status [steps, B].  With a zero disturbance both loops
+    equal the default one bit for bit."""
     torch = prob._torch()
     B, ns, nc, N = P.shape[0], prob.ns, prob.nc, prob.N
+    if advanced_step and (isinstance(prob, SmallOcp) or prob.obstacles is not None or getattr(prob, "moving", False) or prob.Nr > 10):
+        raise ValueError("advanced_step=True needs a handle with parametric sensitivities: nmpc_create or nmpc_create_tracking, "
+                         "1..10 robots")
+    if disturbance is not None and (not (disturbance.is_cuda and disturbance.dtype == torch.float64)
+                                    or tuple(disturbance.shape) != (steps, B, ns)):
+        raise ValueError("disturbance must be a float64 CUDA tensor [steps, B, 3Nr] = [%d, %d, %d]" % (steps, B, ns))
     tracking = getattr(prob, "tracking", False)
     both = tracking and getattr(prob, "moving", False)      # Problem(tracking_obstacles=n_obs)
     if both and (reference is None or obstacles is None):
@@ -493,6 +537,10 @@ def closed_loop(prob, P, lbx, ubx, lbg, ubg, steps, tol=1e-1, dmin=None, obstacl
     act = torch.zeros((steps, B), dtype=torch.bool, device=P.device)
     traj[0] = p[:, :ns]
     out = {}
+    if advanced_step:
+        x_true = p[:, :ns].clone()          # p[:, :ns] holds the predicted state the solve is made for
+        u_pred = torch.zeros((steps, B, nc), dtype=torch.float64, device=P.device)
+        sst = torch.zeros((steps, B), dtype=torch.int32, device=P.device)
     for t in range(steps):
         if t == 0:
             prob.set_order(None)
@@ -506,19 +554,36 @@ def closed_loop(prob, P, lbx, ubx, lbg, ubg, steps, tol=1e-1, dmin=None, obstacl
                 p[:, ns:] = reference[t:t + N].permute(1, 0, 2).reshape(B, -1)
             active = torch.ones(B, dtype=torch.bool, device=P.device)
         else:
-            active = (p[:, :ns] - p[:, ns:2 * ns]).norm(dim=1) > tol
+            active = ((x_true if advanced_step else p[:, :ns]) - p[:, ns:2 * ns]).norm(dim=1) > tol
         act[t] = active
-        prob.solve(x0, p, lbx, ubx, lbg, ubg, want=(), out=out)
-        u0 = out["x"][:, ns * (N + 1):ns * (N + 1) + nc]
-        nxt = prob.plant(p[:, :ns].contiguous(), out["x"])
-        p[:, :ns] = torch.where(active[:, None], nxt, p[:, :ns])
+        u0s = slice(ns * (N + 1), ns * (N + 1) + nc)
+        if advanced_step:
+            prob.solve(x0, p, lbx, ubx, lbg, ubg, want=("lam_x", "lam_g"), out=out)
+            jac, sst[t] = prob.solution_x0_jacobian(out, p, lbx, ubx, lbg, ubg)
+            xa = prob.advanced_step(out, jac, sst[t], p, x_true, lbx, ubx)
+            u_pred[t] = torch.where(active[:, None], out["x"][:, u0s], torch.zeros_like(out["x"][:, u0s]))
+            nxt = prob.plant(x_true, xa)
+            p[:, :ns] = torch.where(active[:, None], nxt, x_true)
+            if disturbance is not None:
+                nxt = nxt + disturbance[t]
+            x_true = torch.where(active[:, None], nxt, x_true)
+        else:
+            prob.solve(x0, p, lbx, ubx, lbg, ubg, want=(), out=out)
+            xa = out["x"]
+            nxt = prob.plant(p[:, :ns].contiguous(), xa)
+            if disturbance is not None:
+                nxt = nxt + disturbance[t]
+            p[:, :ns] = torch.where(active[:, None], nxt, p[:, :ns])
+        u0 = xa[:, u0s]
         us[t] = torch.where(active[:, None], u0, torch.zeros_like(u0))
         st[t], its[t] = out["status"], out["iters"]
         prob.set_order(prob.order_from_iters(out["iters"]))      # longest solves first in the next step
-        x0 = prob.shift(out["x"])
-        traj[t + 1] = p[:, :ns]
+        x0 = prob.shift(xa)
+        traj[t + 1] = x_true if advanced_step else p[:, :ns]
     prob.set_order(None)
     res = dict(traj=traj, u=us, status=st, iters=its, active=act)
+    if advanced_step:
+        res.update(u_pred=u_pred, sens_status=sst)
     if prob.Nr > 1:
         pos = traj.reshape(steps + 1, B, prob.Nr, 3)[..., :2]
         d = (pos[:, :, :, None, :] - pos[:, :, None, :, :]).norm(dim=-1)
