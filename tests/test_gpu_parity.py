@@ -48,7 +48,7 @@ def test_eval_kernel_matches_oracle(pkg, torch_cuda, Nr, N, T):
 def test_shift_and_plant_kernels_exact(pkg, torch_cuda):
     torch = torch_cuda
     rng = np.random.default_rng(3)
-    for Nr, N in ((1, 25), (6, 20), (4, 3)):
+    for Nr, N in ((1, 25), (6, 20), (4, 3), (3, 1)):
         prob, orc = pkg.Problem(Nr, N, 0.3), Oracle(Nr, N, 0.3)
         w = rng.normal(size=(65, orc.n))
         sh = prob.shift(_t(torch, w)).cpu().numpy()
