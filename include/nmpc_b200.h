@@ -257,6 +257,28 @@ int nmpc_advanced_step(nmpc_handle *h, int B, const double *x, const double *jac
                        const double *x0bar_meas, const double *lbx, const double *ubx, int bounds_batched, double *x_corr,
                        void *stream);
 
+/* Distributed NMPC: S scenarios of R robots, each robot solved as its own one-robot instance (instance s R + r) against its
+ * teammates' predicted paths, which this call exchanges on the device.  For a one-robot handle of nmpc_create_moving_obstacles or
+ * nmpc_create_tracking_obstacles with K = n_obs, it writes into p [S R][nmpc_np] (row s R + a):
+ *   - x0bar = state[s][a] (state [S][R][3], current poses);
+ *   - the obstacle block O[N][K][3], at p + nmpc_np - 3 N K: O[k][o] = (x, y, clearance) of the o-th selected teammate's
+ *     prediction at stage k.  Robot j's prediction is its pose at k = 0 and X_{min(k+1, N)} of its plan for k = 1..N-1 (plan
+ *     [S R][n], the last solution in the handle's layout, X_k at 3k: the plan shifted by one period with the last stage
+ *     repeated, as nmpc_shift does); plan == NULL (no plan yet) holds the pose at every stage.  Robot a's candidates are the
+ *     other robots of its scenario, with key (d2, j), d2 = the smallest squared xy distance between the two predictions over
+ *     k < N; the K smallest keys are selected in lexicographic order (ties go to the lower index), o in key order.  With
+ *     R - 1 < K the remaining slots hold an inactive obstacle: the robot's own pose + (1e6, 0) at every stage, clearance 0;
+ * nothing else (xs, or Z on a tracking handle) is touched: goals and references are the caller's.  min_dist [S R] (may be NULL)
+ * gets the distance from each robot's pose to the nearest other robot of its scenario, over all R (+inf for R = 1).  Squares and
+ * sums round to nearest without FMA contraction, the square root is correctly rounded, positions and the clearance are copied.
+ * A row of robot a on stage 0 sits on the fixed X_0: a pair already closer than clearance + the obstacle rows' lbg margin makes
+ * the instance infeasible, which the solve reports per instance (returning the last iterate) as for any other instance.
+ * All pointers are DEVICE pointers; one launch (counted by nmpc_launch_count), asynchronous on stream, no allocation.  Other
+ * handles: NMPC_ENOTSUP.  S <= 0, R <= 0, S R >= 2^31, NULL state or p, a clearance that is negative or not finite, or a
+ * handle created on another device: NMPC_EINVAL. */
+int nmpc_neighbour_obstacles(nmpc_handle *h, int S, int R, const double *state, const double *plan, double clearance,
+                             double *p, double *min_dist, void *stream);
+
 /* Same call with HOST buffers (what a CasADi-style caller has): H2D of the inputs, solve, D2H of
  * the requested outputs, synchronous.  Staging buffers live in the handle and grow on demand. */
 int nmpc_solve_host(nmpc_handle *h, int B, const double *x0, const double *p,

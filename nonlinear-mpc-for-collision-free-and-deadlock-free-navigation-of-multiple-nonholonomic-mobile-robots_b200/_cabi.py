@@ -17,7 +17,8 @@ SYMBOLS = ["nmpc_default_opts", "nmpc_last_error", "nmpc_create", "nmpc_destroy"
            "nmpc_debug_block_profile", "nmpc_set_order", "nmpc_create_obstacles", "nmpc_create_ocp",
            "nmpc_default_tuning", "nmpc_create_tuned", "nmpc_probe_dmma", "nmpc_create_moving_obstacles",
            "nmpc_create_tracking", "nmpc_create_tracking_obstacles", "nmpc_solution_vjp", "nmpc_solution_jvp",
-           "nmpc_sensitivity_workspace_bytes", "nmpc_solution_x0_jacobian", "nmpc_advanced_step"]
+           "nmpc_sensitivity_workspace_bytes", "nmpc_solution_x0_jacobian", "nmpc_advanced_step",
+           "nmpc_neighbour_obstacles"]
 
 
 class Desc(C.Structure):
@@ -95,6 +96,7 @@ def lib():
     L.nmpc_solution_x0_jacobian.argtypes = [H, C.c_int] + [dp] * 8 + [C.c_int, dp, ip, vp, C.c_size_t, vp]
     L.nmpc_advanced_step.argtypes = [H, C.c_int, dp, dp, ip] + [dp] * 4 + [C.c_int, dp, vp]
     L.nmpc_sensitivity_workspace_bytes.restype = C.c_size_t
+    L.nmpc_neighbour_obstacles.argtypes = [H, C.c_int, C.c_int, dp, dp, C.c_double, dp, dp, vp]
     L.nmpc_probe_dmma.argtypes = [C.POINTER(C.c_double)]
     L.nmpc_launch_count.restype = C.c_longlong
     _LIB = L

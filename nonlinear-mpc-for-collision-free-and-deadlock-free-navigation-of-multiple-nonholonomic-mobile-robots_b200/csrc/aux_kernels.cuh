@@ -9,6 +9,8 @@
 //       plant_kernel  -- Euler plant (casadi_test.py:17-26)
 //       prep_bounds_kernel -- flat lbx/ubx/lbg/ubg (:349-352) -> relaxed stage-layout rows
 //       advanced_step_kernel -- first-order correction of a solution for the measured state (nmpc_advanced_step)
+//       neighbour_kernel -- distributed NMPC: each robot's K nearest teammates' predicted paths as its obstacle block
+//                        (nmpc_neighbour_obstacles)
 #pragma once
 #include "bounds_prep.cuh"
 #include "nmpc_internal.h"
@@ -338,5 +340,98 @@ __global__ void __launch_bounds__(256) advanced_step_kernel(int ns, int n, int n
         if (lb > -NMPC_INF) v = fmax(v, fmin(lb, xi));
         if (ub < NMPC_INF) v = fmin(v, fmax(ub, xi));
         xc[e] = v;
+    }
+}
+
+// Neighbour exchange of distributed NMPC (nmpc_neighbour_obstacles).  Robot j's prediction at stage k < N is its pose state[j] at
+// k = 0 and X_{min(k+1, N)} of its plan (plan [S R][n], X_k at 3k) for k >= 1: the plan shifted by one period with the last stage
+// repeated; plan == NULL holds the pose at every stage.  For robot a the key of a teammate j != a of its scenario is (d2, j),
+// d2 = min over k < N of the squared xy distance of the two predictions; the K smallest keys in lexicographic order (ties to the
+// lower index) give O[k][o] = (x, y, clearance) of the o-th one at stage k, and a slot left without a teammate (R - 1 < K) gets an
+// inactive obstacle: the own pose + (1e6, 0) with clearance 0.  x0bar = state; nothing else of p is written.  min_dist[a] is the
+// distance from a's pose to the nearest other robot of its scenario (+inf for R = 1).
+// One warp per robot, NB_WARPS robots of one scenario per CTA, (scenario, robot group) pairs strided over the grid.  Tiles of 32
+// candidates x N stages are staged in shared memory once per CTA for all its warps, stage-major ([N][32] double2, so lane c reads
+// its candidate's stage k without bank conflicts); each lane computes one candidate's key, and the warp keeps its 32 smallest keys
+// sorted across its lanes: a bitonic network on shuffles sorts the tile's 32 keys, min(kept[l], new[31 - l]) leaves the 32
+// smallest of the 64 as a bitonic sequence, and a 5-step bitonic merge sorts them again.  The arithmetic is __dsub_rn / __dmul_rn /
+// __dadd_rn (no FMA contraction), fmin and a correctly rounded sqrt, so a NumPy restatement matches bit for bit, and the result
+// depends neither on the tiling nor on the lane order (the keys are distinct but for the padding key, which is one value).
+#define NB_WARPS 8
+#define NB_NONE 0x7fffffff   // index of the padding key
+struct NbKey { double d; int j; };
+__device__ __forceinline__ bool nb_less(const NbKey &a, const NbKey &b) { return a.d < b.d || (a.d == b.d && a.j < b.j); }
+// compare-exchange with lane ^ m: the smaller of the two keys if keep_min, else the larger
+__device__ __forceinline__ NbKey nb_cx(const NbKey &k, int m, bool keep_min)
+{
+    const NbKey o = {__shfl_xor_sync(0xffffffffu, k.d, m), __shfl_xor_sync(0xffffffffu, k.j, m)};
+    return nb_less(o, k) == keep_min ? o : k;
+}
+
+__global__ void __launch_bounds__(NB_WARPS * 32) neighbour_kernel(int N, int K, int S, int R, int n, int np,
+                                                                  const double *__restrict__ state, const double *__restrict__ plan,
+                                                                  double clearance, double *__restrict__ p, double *__restrict__ min_dist)
+{
+    extern __shared__ double2 nb_sh[];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    double2 *tile = nb_sh, *own = nb_sh + (size_t)N * 32 + (size_t)warp * N;   // [N][32] candidates, [N] this warp's robot
+    const double inf = __longlong_as_double(0x7ff0000000000000LL);
+    const int groups = (R + NB_WARPS - 1) / NB_WARPS;
+    auto pred = [&](long long j, int k) {
+        const double *s = (k == 0 || !plan) ? state + 3 * j : plan + j * n + 3 * min(k + 1, N);
+        return make_double2(s[0], s[1]);
+    };
+    for (long long g = blockIdx.x; g < (long long)S * groups; g += gridDim.x) {
+        const long long base = (g / groups) * R;
+        const int a = (int)(g % groups) * NB_WARPS + warp;
+        const bool live = a < R;   // uniform over the warp
+        __syncwarp();
+        if (live)
+            for (int k = lane; k < N; k += 32) own[k] = pred(base + a, k);
+        NbKey kept = {inf, NB_NONE};
+        double d0 = inf;   // smallest squared distance between current poses seen by this lane
+        for (int j0 = 0; j0 < R; j0 += 32) {
+            __syncthreads();   // every warp is done with the previous tile
+            for (int e = threadIdx.x; e < 32 * N; e += blockDim.x)
+                if (j0 + (e & 31) < R) tile[e] = pred(base + j0 + (e & 31), e >> 5);
+            __syncthreads();
+            const int j = j0 + lane;
+            NbKey nk = {inf, NB_NONE};
+            if (live && j < R && j != a) {
+                double dm = inf;
+                for (int k = 0; k < N; k++) {
+                    const double2 q = tile[k * 32 + lane], o = own[k];
+                    const double dx = __dsub_rn(o.x, q.x), dy = __dsub_rn(o.y, q.y);
+                    const double d2 = __dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy));
+                    if (k == 0) d0 = fmin(d0, d2);
+                    dm = fmin(dm, d2);
+                }
+                nk = {dm, j};
+            }
+#pragma unroll
+            for (int size = 2; size <= 32; size <<= 1)
+#pragma unroll
+                for (int m = size >> 1; m > 0; m >>= 1) nk = nb_cx(nk, m, ((lane & m) == 0) == ((lane & size) == 0));
+            const NbKey r = {__shfl_sync(0xffffffffu, nk.d, 31 - lane), __shfl_sync(0xffffffffu, nk.j, 31 - lane)};
+            if (nb_less(r, kept)) kept = r;
+#pragma unroll
+            for (int m = 16; m > 0; m >>= 1) kept = nb_cx(kept, m, (lane & m) == 0);
+        }
+#pragma unroll
+        for (int m = 16; m > 0; m >>= 1) d0 = fmin(d0, __shfl_xor_sync(0xffffffffu, d0, m));
+        if (!live) continue;
+        const long long ia = base + a;
+        double *pa = p + ia * np, *O = pa + (np - 3 * N * K);
+        if (lane < 3) pa[lane] = state[3 * ia + lane];
+        if (lane == 0 && min_dist) min_dist[ia] = sqrt(d0);
+        const double2 me = own[0];
+        for (int e0 = 0; e0 < N * K; e0 += 32) {   // entry e = (k, o) = (e / K, e % K) of the block, three doubles each
+            const int e = e0 + lane, jo = __shfl_sync(0xffffffffu, kept.j, e % K);
+            if (e >= N * K) continue;
+            double2 q = make_double2(__dadd_rn(me.x, 1e6), me.y);
+            double c = 0.0;
+            if (jo != NB_NONE) { q = pred(base + jo, e / K); c = clearance; }
+            O[3 * e] = q.x; O[3 * e + 1] = q.y; O[3 * e + 2] = c;
+        }
     }
 }

@@ -785,6 +785,36 @@ extern "C" int nmpc_advanced_step(nmpc_handle *h, int B, const double *x, const 
     return 0;
 }
 
+// neighbour exchange of distributed NMPC: one launch of neighbour_kernel (aux_kernels.cuh), NB_WARPS robots of one scenario per
+// CTA, at most 8 CTAs per SM strided over the S * ceil(R / NB_WARPS) robot groups
+extern "C" int nmpc_neighbour_obstacles(nmpc_handle *h, int S, int R, const double *state, const double *plan, double clearance,
+                                        double *p, double *min_dist, void *stream)
+{
+    const char *fn = "nmpc_neighbour_obstacles";
+    if (!h) return fail(NMPC_EINVAL, "%s: NULL handle", fn);
+    if (h->family != 1 || !h->obs_in_p || h->d.Nr != 1)
+        return fail(NMPC_ENOTSUP, "%s: needs a one-robot handle of nmpc_create_moving_obstacles or nmpc_create_tracking_obstacles", fn);
+    if (!state || !p) return fail(NMPC_EINVAL, "%s: NULL argument", fn);
+    if (S <= 0 || R <= 0 || (long long)S * R > 0x7fffffffLL) return fail(NMPC_EINVAL, "%s: need S, R > 0 and S * R < 2^31", fn);
+    if (!(clearance >= 0.0 && clearance < NMPC_INF)) return fail(NMPC_EINVAL, "%s: the clearance must be finite and >= 0", fn);
+    int rc = sens_batch_device(h, S * R, fn);
+    if (rc) return rc;
+    const int N = h->d.N;
+    const size_t smem = (size_t)(32 + NB_WARPS) * N * sizeof(double2);
+    if (smem > 48 * 1024) {
+        cudaError_t e = cudaFuncSetAttribute(neighbour_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) return fail(NMPC_ENOTSUP, "%s: N = %d needs %zu B of shared memory: %s", fn, N, smem, cudaGetErrorString(e));
+    }
+    const long long groups = (long long)S * ((R + NB_WARPS - 1) / NB_WARPS);
+    const int grid = (int)std::min<long long>(groups, (long long)h->sm_count * 8);
+    neighbour_kernel<<<grid, NB_WARPS * 32, smem, (cudaStream_t)stream>>>(N, h->nobs, S, R, h->n, h->np, state, plan, clearance, p,
+                                                                         min_dist);
+    h->launches++;
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return fail(NMPC_ECUDA, "%s: launch failed: %s", fn, cudaGetErrorString(e));
+    return 0;
+}
+
 static size_t al(size_t v) { return (v + 255) & ~(size_t)255; }
 
 extern "C" int nmpc_solve_host(nmpc_handle *h, int B, const double *x0, const double *p, const double *lbx, const double *ubx,

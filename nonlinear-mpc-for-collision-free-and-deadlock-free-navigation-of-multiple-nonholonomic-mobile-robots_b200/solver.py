@@ -391,6 +391,32 @@ class Problem:
                                         xc.data_ptr(), self._stream(dev)))
         return xc
 
+    # ---- distributed NMPC (nmpc_neighbour_obstacles) --------------------------------------------------------------------------
+    def neighbour_obstacles(self, state, plan=None, *, clearance, p=None):
+        """Neighbour exchange of distributed NMPC on a one-robot Problem(moving_obstacles=K) or Problem(tracking_obstacles=K), one
+        launch: for the poses state [S, R, 3] of S scenarios of R robots and their last solutions plan [S R, n] (None: no plan
+        yet, every prediction holds the pose), writes x0bar = the robot's pose and the obstacle block O = the predicted paths of
+        its K nearest teammates (clearance each; inactive far points if R - 1 < K) into p [S R, np], instance s R + r.  The other
+        entries of p (xs, or Z) are left as they are: p=None allocates zeros for the caller to fill.  Returns (p, min_dist [S, R]),
+        min_dist the distance from each robot to the nearest other robot of its scenario.  See nmpc_neighbour_obstacles."""
+        torch = self._torch()
+        if not getattr(self, "moving", False) or self.Nr != 1:
+            raise ValueError("neighbour_obstacles needs a one-robot Problem(moving_obstacles=K) or Problem(tracking_obstacles=K)")
+        if not (state.is_cuda and state.dtype == torch.float64 and state.is_contiguous()) or state.dim() != 3 or state.shape[2] != 3:
+            raise ValueError("state must be a contiguous float64 CUDA tensor [S, R, 3]")
+        S, R = int(state.shape[0]), int(state.shape[1])
+        dev = state.device
+        for name, t, shape in (("plan", plan, (S * R, self.n)), ("p", p, (S * R, self.np_))):
+            if t is not None and (not (t.is_cuda and t.dtype == torch.float64 and t.is_contiguous() and t.device == dev)
+                                  or tuple(t.shape) != shape):
+                raise ValueError("%s must be a contiguous float64 CUDA tensor [S R, %d] on the device of state" % (name, shape[1]))
+        if p is None:
+            p = torch.zeros((S * R, self.np_), dtype=torch.float64, device=dev)
+        md = torch.empty((S, R), dtype=torch.float64, device=dev)
+        check(self.L.nmpc_neighbour_obstacles(self.h, S, R, state.data_ptr(), None if plan is None else plan.data_ptr(),
+                                              float(clearance), p.data_ptr(), md.data_ptr(), self._stream(dev)))
+        return p, md
+
     def solve_differentiable(self, x0, p, lbx, ubx, lbg, ubg):
         """solve() as a torch.autograd function of p: returns x [B, n]; x.backward / torch.autograd.grad give the gradient with
         respect to p through nmpc_solution_vjp at the returned solutions.  x0 and the bounds get no gradient (x* does not depend
@@ -598,6 +624,83 @@ def closed_loop(prob, P, lbx, ubx, lbg, ubg, steps, tol=1e-1, dmin=None, obstacl
         pos = traj.reshape(steps + 1, B, prob.Nr, 3)[..., :2]
         ref = reference[:steps + 1, :, :ns].reshape(steps + 1, B, prob.Nr, 3)[..., :2]
         res["track_err"] = (pos - ref).norm(dim=-1).amax(dim=2)
+    return res
+
+
+def distributed_loop(prob, state0, goals_or_reference, lbx, ubx, lbg, ubg, steps, clearance, tol=1e-1, disturbance=None):
+    """Distributed NMPC for S scenarios of R robots, device resident: every robot solves its own one-robot problem against the
+    predicted paths of its K nearest teammates (prob: Problem(1, N, T, moving_obstacles=K) or Problem(1, N, T,
+    tracking_obstacles=K); lbx..ubg that handle's bounds, e.g. bounds_obstacles(margin, ...), whose obstacle-row margin adds to
+    `clearance`, the centre distance the rows keep).  Per step: exchange (Problem.neighbour_obstacles: x0bar and the obstacle
+    block of every robot from the poses and the last solutions) -> one batched solve of the S R instances (instance s R + r;
+    warm start by the shift of the last solution, longest-first order from the last iteration counts, as in closed_loop) ->
+    Euler plant -> stop test.
+    goals_or_reference: the moving-obstacle handle takes goals [S, R, 3], written into xs once, and a robot within `tol` of its
+    goal stops; it stays an obstacle at its pose (its plan is replaced by its held pose before the exchange).  The
+    tracking-obstacle handle takes reference [steps + N, S, R, 5], rows [xr_t; ur_t] over time, of which step t solves with rows
+    t..t+N-1 as Z, with no stop test.  disturbance: CUDA float64 [steps, S, R, 3], added to the next state of the active robots.
+    Returns CUDA tensors traj [steps+1, S, R, 3], u [steps, S, R, 2], status, iters, active [steps, S, R] and min_dist
+    [steps+1, S], the smallest distance between two robots of a scenario at each time (from the exchange's audit); with a
+    reference also track_err [steps+1, S, R], the xy distance between each robot and its reference state."""
+    torch = prob._torch()
+    if not getattr(prob, "moving", False) or prob.Nr != 1:
+        raise ValueError("distributed_loop needs a one-robot Problem(moving_obstacles=K) or Problem(tracking_obstacles=K)")
+    if not (state0.is_cuda and state0.dtype == torch.float64) or state0.dim() != 3 or state0.shape[2] != 3:
+        raise ValueError("state0 must be a float64 CUDA tensor [S, R, 3]")
+    S, R, N, dev = int(state0.shape[0]), int(state0.shape[1]), prob.N, state0.device
+    B, tracking = S * R, prob.tracking
+    g = goals_or_reference
+    if not (g.is_cuda and g.dtype == torch.float64) or tuple(g.shape) != ((steps + N, S, R, 5) if tracking else (S, R, 3)):
+        raise ValueError("a Problem(tracking_obstacles=K) takes a float64 CUDA reference [steps + N, S, R, 5], a "
+                         "Problem(moving_obstacles=K) float64 CUDA goals [S, R, 3]")
+    if disturbance is not None and (not (disturbance.is_cuda and disturbance.dtype == torch.float64)
+                                    or tuple(disturbance.shape) != (steps, S, R, 3)):
+        raise ValueError("disturbance must be a float64 CUDA tensor [steps, S, R, 3] = [%d, %d, %d, 3]" % (steps, S, R))
+    f64 = dict(dtype=torch.float64, device=dev)
+    p = torch.zeros((B, prob.np_), **f64)
+    if not tracking:
+        goals = g.reshape(B, 3)
+        p[:, 3:6] = goals
+    state = state0.reshape(B, 3).clone()
+    hold = lambda x: torch.cat([x.repeat(1, N + 1), torch.zeros((B, 2 * N), **f64)], dim=1)     # Problem.cold_start
+    traj = torch.empty((steps + 1, S, R, 3), **f64)
+    us = torch.zeros((steps, S, R, 2), **f64)
+    st = torch.zeros((steps, S, R), dtype=torch.int32, device=dev)
+    its = torch.zeros((steps, S, R), dtype=torch.int32, device=dev)
+    act = torch.zeros((steps, S, R), dtype=torch.bool, device=dev)
+    md = torch.empty((steps + 1, S), **f64)
+    traj[0] = state0
+    plan, x0, out = None, hold(state), {}
+    u0s = slice(3 * (N + 1), 3 * (N + 1) + 2)
+    prob.set_order(None)
+    for t in range(steps):
+        if tracking:
+            p[:, 3:3 + 5 * N] = g[t:t + N].permute(1, 2, 0, 3).reshape(B, 5 * N)
+            active = torch.ones(B, dtype=torch.bool, device=dev)
+        else:
+            active = (state - goals).norm(dim=1) > tol
+        act[t] = active.reshape(S, R)
+        if plan is not None:
+            plan = torch.where(active[:, None], plan, hold(state))
+        _, d = prob.neighbour_obstacles(state.reshape(S, R, 3), plan, clearance=clearance, p=p)
+        md[t] = d.amin(dim=1)
+        prob.solve(x0, p, lbx, ubx, lbg, ubg, want=(), out=out)
+        xa = out["x"]
+        nxt = prob.plant(state, xa)
+        if disturbance is not None:
+            nxt = nxt + disturbance[t].reshape(B, 3)
+        state = torch.where(active[:, None], nxt, state)
+        us[t] = torch.where(active[:, None], xa[:, u0s], torch.zeros_like(xa[:, u0s])).reshape(S, R, 2)
+        st[t], its[t] = out["status"].reshape(S, R), out["iters"].reshape(S, R)
+        prob.set_order(prob.order_from_iters(out["iters"]))      # longest solves first in the next step
+        x0 = prob.shift(xa)
+        plan = xa.clone()
+        traj[t + 1] = state.reshape(S, R, 3)
+    prob.set_order(None)
+    md[steps] = prob.neighbour_obstacles(state.reshape(S, R, 3), None, clearance=clearance, p=p)[1].amin(dim=1)
+    res = dict(traj=traj, u=us, status=st, iters=its, active=act, min_dist=md)
+    if tracking:
+        res["track_err"] = (traj[..., :2] - g[:steps + 1, ..., :2]).norm(dim=-1)
     return res
 
 
